@@ -26,6 +26,13 @@ N > 1 adds, outside the timed region: `parity` (a 2 M-point strip build + exchan
 the full parity bar against the oracle on rank 0; the run fails on any unexplained mismatch)
 and `target_cfg3` (the north-star case: ONE 50 M-point cloud at 0.1 m cells, strong-scaled
 over the N strips, both input conventions).
+
+--dump-outputs DIR (N = 1): after the run, the voxel, slope and column tables of the last timed
+step, one DIR/<table>_<field>.npy per field (float fields float32, integer fields float64, both
+exact), DIR/<table>_rows.npy (the table rows written) and DIR/counts.npy.  Tables longer than
+DUMP_ROWS rows are written as a seeded sample of rows that depends only on the table's length:
+two runs whose tables have the same length get the same rows (counts.npy tells when they do
+not).  The input cloud is seeded, so two builds of the project can be compared output for output.
 """
 import argparse
 import json
@@ -49,6 +56,7 @@ REF_STEP_POINTS = 1_000_000      # --impl reference: points per timed step (boun
 CPU_BASELINE_POINTS = 4_000_000  # cpu_baseline leg of the default run
 TARGET_POINTS = int(os.environ.get("GNDT_BENCH_TARGET_POINTS", "50000000"))  # north-star cloud (N > 1); 0 disables
 WORKLOAD = "cfg2 multi-level bridge/underpass scene, 10M points per GPU, 0.2 m cells, z 0.1 m, slope_interval 0.08, demand slope (BASELINE configs[1])"
+DUMP_ROWS, DUMP_SEED = 200_000, 20260100  # --dump-outputs: rows per table (at most 55 MB in all)
 
 
 def measured_peak():
@@ -153,6 +161,26 @@ def make_cloud(rank):
         # box of every strip but the first over the whole map, costing those strips a partition pass)
         cloud[:, 0] += np.float32(SCENE_W * rank)
     return cloud
+
+
+def dump_outputs(out_dir, m):
+    """The result tables of the build held by TwoDmap `m` -> out_dir/<table>_<field>.npy."""
+    from grid_ndt_b200._abi import Counts
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"counts": np.array([m.counts()[k] for k, _ in Counts._fields_], np.float64)}
+    for table in ("voxels", "slopes", "columns"):
+        t = getattr(m, table)
+        rows = np.arange(len(t))
+        if len(t) > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(DUMP_SEED).choice(len(t), DUMP_ROWS, replace=False))
+        arrays[f"{table}_rows"] = rows.astype(np.float64)
+        for field in t.dtype.names:
+            if field != "reserved":
+                a = t[field][rows]
+                arrays[f"{table}_{field}"] = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sum(a.nbytes for a in arrays.values())
 
 
 def run_reference(args):
@@ -293,7 +321,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="N > 1: skip the parity and target_cfg3 legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="N = 1: write the result tables of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs writes the tables of a single-GPU build of our path: run it with --impl ours and one process")
     args.warmup = max(args.warmup, 3)
     # stdout carries exactly ONE line, the JSON: everything else any library writes to fd 1
     # (NCCL's version banner, for one) is sent to stderr for the whole run
@@ -403,6 +436,7 @@ def main():
         # throughput: two builds in flight on two streams (a second build fills the SMs left idle
         # by the partial last wave of every kernel and by the tiny kernels of the first)
         flight = CloudPipeline(GRID_LEN, Z_LEN, INTERVAL, "slope", depth=2, device=local)
+        last = {}  # the builder of the last step run_steps submitted (flight is not used after the timed region)
 
         def step(src):
             m.chatterCallback(src, "slope")
@@ -414,7 +448,8 @@ def main():
                     n_launch += flight.release().launch_count()
                 flight.submit(src)
             while flight.pending:
-                n_launch += flight.release().launch_count()
+                last["map"] = flight.release()
+                n_launch += last["map"].launch_count()
             flight.join()
             return n_launch
 
@@ -639,6 +674,9 @@ def main():
     if rank == 0:
         args.json_out.write(json.dumps(line) + "\n")
         args.json_out.flush()
+    if args.dump_outputs:
+        nbytes = dump_outputs(args.dump_outputs, last["map"])
+        print(f"outputs of the last timed step: {nbytes / 1e6:.1f} MB in {args.dump_outputs}", file=sys.stderr)
     if world > 1:
         dist.destroy_process_group()
     return 0
