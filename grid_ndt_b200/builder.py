@@ -308,10 +308,11 @@ class TwoDmap:
         return bool(en.value), int(n.value)
 
     def key_layout(self) -> dict:
-        """Live partition passes and key-field widths of the last build (introspection)."""
+        """Sort-key layout of the last build (introspection): live partition passes, bits of the
+        column id field, the column id's y radix (ny) and bits of the z field."""
         out = (C.c_int * 4)()
         _check(self._h, lib().gndt_key_layout(self._h, out))
-        return {"passes": out[0], "bits_x": out[1], "bits_y": out[2], "bits_z": out[3]}
+        return {"passes": out[0], "bits_col": out[1], "ny": out[2], "bits_z": out[3]}
 
     def launch_count(self) -> int:
         n = C.c_uint64()

@@ -398,7 +398,7 @@ __global__ void __launch_bounds__(128) fixup_kernel(Ctl *ctl, VoxMoments *mom, c
         if (lane + o < 32) merge_moments(mine, other);
       }
       if (lane == 0) merge_moments(acc, mine);
-      if (n_inc < 32) break;  // chain ended inside this chunk (warp-uniform)
+      if (n_inc < 32 || ends_here) break;  // chain ended in this chunk, lane 31 included: later leads are other voxels' (warp-uniform)
     }
     if (lane == 0) {
       VoxMoments *v = mom + carry[t].tail_slot;

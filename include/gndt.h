@@ -414,7 +414,8 @@ int gndt_morton_string(int32_t sx, int32_t sy, char *buf);
 int gndt_cell_center(const float origin[3], float grid_len, float z_len, int32_t sx, int32_t sy,
                      int32_t sz, float center[3]);
 /* Introspection: the sort-key layout the last build / update derived from the cloud's bounds:
- * out[0] = live partition passes (of the 6 launched), out[1..3] = bits of the x, y, z fields. */
+ * out[0] = live partition passes (of the 6 launched), out[1] = bits of the column id field
+ * ((cx - cx_min) * ny + (cy - cy_min)), out[2] = ny, out[3] = bits of the z field. */
 int gndt_key_layout(gndt_handle *h, int out[4]);
 /* Integer-keyed replacements for the planner's string lookups `map_cell.find(morton_xy)` /
  * `map_slope.find(morton_z)` (include/map2D.h:269-272,396-398; include/GlobalPlan.h:58-61) and

@@ -280,6 +280,7 @@ def run_case(cloud, params, demand="slope", device=None, check_reach=True):
     m.setInterval(params.slope_interval)
     m.params.min_points = params.min_points
     m.params.normalize_cov = params.normalize_cov
+    m.params.rough_max, m.params.angle_max_deg, m.params.reach_height = params.rough_max, params.angle_max_deg, params.reach_height
     m.params.tile_lo, m.params.tile_hi = params.tile_lo, params.tile_hi
     if params.origin_is_first_point:
         m.chatterCallback(cloud, demand)
