@@ -371,7 +371,9 @@ int sync_counts(gndt_handle *h) {
       return GNDT_ERR_CAPACITY;
     }
     std::swap(h->mom, h->mom_alt);
+    // the cloud-index counter follows n_input: a remove gives its points' indices back
     if (sign > 0) h->total_points += h->pending_points;
+    else h->total_points -= h->pending_points;
     u32 nc = 0;
     GNDT_CUDA(h, cudaMemcpy(&nc, h->changed_count_dev, 4, cudaMemcpyDeviceToHost));
     h->n_changed = nc;

@@ -60,6 +60,9 @@ finalize_label_kernel(Ctl *ctl, const VoxMoments *mom, gndt_voxel *table, gndt_s
   if (ctl->err) return;  // e.g. capacity exceeded: the moments table is incomplete
   const u32 V = ctl->n_voxels;
   const u32 n_blocks = (V + kLabelThreads - 1) / kLabelThreads;
+  const float o[3] = {ctl->origin[0], ctl->origin[1], ctl->origin[2]};
+  // absolute mean z of a record (the moments hold it relative to the cell centre, gndt_reduce.cuh)
+  auto mean_z = [&](const VoxMoments &r) { return (float)(r.m[2] + anchor_axis((u32)r.key & 0xFFFFu, o[2], P.z_len)); };
   if (tid == 0) mbar_init(&S.mbar, 1);
   for (u32 it = 0;; ++it) {
     __syncthreads();  // everyone is done with in[] / out[] of the previous block
@@ -87,7 +90,7 @@ finalize_label_kernel(Ctl *ctl, const VoxMoments *mom, gndt_voxel *table, gndt_s
       const VoxMoments &me = S.in[tid + 1];
       key = me.key; count = me.count; first = me.first;
       fitted = (int)count >= P.min_points;
-      mz = (float)me.m[2];
+      mz = mean_z(me);
       const bool has_lo = (v > 0) && (S.in[tid].key >> 16) == (key >> 16);
       const bool has_hi = (v + 1 < V) && (S.in[tid + 2].key >> 16) == (key >> 16);
       head = !has_lo;
@@ -98,12 +101,12 @@ finalize_label_kernel(Ctl *ctl, const VoxMoments *mom, gndt_voxel *table, gndt_s
         if (has_hi && (S.in[tid + 2].key & 0xFFFFu) == (key & 0xFFFFu) + 1) {
           const VoxMoments &hi = S.in[tid + 2];
           const bool seen = (int)hi.count >= P.min_points && (!ordered || hi.first < first);
-          up = fabsf(__fsub_rn(seen ? (float)hi.m[2] : 0.f, mz)) > P.slope_interval;
+          up = fabsf(__fsub_rn(seen ? mean_z(hi) : 0.f, mz)) > P.slope_interval;
         }
         if (ordered && has_lo && (S.in[tid].key & 0xFFFFu) + 1 == (key & 0xFFFFu)) {
           const VoxMoments &lo = S.in[tid];
           const bool seen = (int)lo.count >= P.min_points && lo.first < first;
-          down = fabsf(__fsub_rn(seen ? (float)lo.m[2] : 0.f, mz)) > P.slope_interval;
+          down = fabsf(__fsub_rn(seen ? mean_z(lo) : 0.f, mz)) > P.slope_interval;
         }
         if (up) flags |= GNDT_F_UP;
         if (down) flags |= GNDT_F_DOWN;
@@ -141,7 +144,9 @@ finalize_label_kernel(Ctl *ctl, const VoxMoments *mom, gndt_voxel *table, gndt_s
       u[3] = count; u[4] = first;
       if (fitted) {
         const VoxMoments &me = S.in[tid + 1];
-        f[5] = (float)me.m[0]; f[6] = (float)me.m[1]; f[7] = mz;
+        f[5] = (float)(me.m[0] + anchor_axis((u32)(key >> 32), o[0], P.grid_len));
+        f[6] = (float)(me.m[1] + anchor_axis((u32)(key >> 16) & 0xFFFFu, o[1], P.grid_len));
+        f[7] = mz;
         double a[6];
 #pragma unroll
         for (int k = 0; k < 6; ++k) {

@@ -41,10 +41,23 @@ struct __align__(16) VoxMoments {
   u64 key;      // voxel_key(cx,cy,cz)
   u32 count;
   u32 first;    // cloud index of the first point
-  double m[3];
+  double m[3];  // mean relative to the cell centre (cell_anchor)
   double s[6];
   u64 pad;
 };
+
+// Centre of a voxel's cell in binary64, from its key, the origin and the cell lengths.  Means are
+// kept relative to it: every partial of one voxel shares the anchor, so merges need no change, and
+// the inverse merge (unmerge_moments) cancels means of at most a cell's size instead of absolute
+// coordinates, whose rounding it would amplify by (points before) / (points after).
+__device__ __forceinline__ double anchor_axis(u32 biased, float o, float len) {
+  return __fma_rn((double)((int)biased - kIdxBias) + 0.5, (double)len, (double)o);
+}
+__device__ __forceinline__ void cell_anchor(u64 key, const float o[3], float grid_len, float z_len, double a[3]) {
+  a[0] = anchor_axis((u32)(key >> 32), o[0], grid_len);
+  a[1] = anchor_axis((u32)(key >> 16) & 0xFFFFu, o[1], grid_len);
+  a[2] = anchor_axis((u32)key & 0xFFFFu, o[2], z_len);
+}
 
 constexpr u32 kCarryHasLead = 1u, kCarryLeadContinues = 2u, kCarryHasTail = 4u;
 struct TileCarry {
@@ -67,13 +80,14 @@ __device__ __forceinline__ void merge_moments(Moments &a, const Moments &b) {
   a.n = n;
 }
 
-// Raw shifted sums (about the run's first point p0) -> (n, mean, centred scatter).
-__device__ __forceinline__ void close_moments(Moments &mo, double n, const float4 &p0, const double sd[3],
-                                              const double sq[6]) {
+// Raw shifted sums (about the run's first point p0) -> (n, mean relative to the cell centre
+// `anc`, centred scatter).
+__device__ __forceinline__ void close_moments(Moments &mo, double n, const float4 &p0, const double anc[3],
+                                              const double sd[3], const double sq[6]) {
   const double inv = 1.0 / n;
   const double m0 = sd[0] * inv, m1 = sd[1] * inv, m2 = sd[2] * inv;
   mo.n = n;
-  mo.m[0] = (double)p0.x + m0; mo.m[1] = (double)p0.y + m1; mo.m[2] = (double)p0.z + m2;
+  mo.m[0] = ((double)p0.x - anc[0]) + m0; mo.m[1] = ((double)p0.y - anc[1]) + m1; mo.m[2] = ((double)p0.z - anc[2]) + m2;
   mo.s[0] = sq[0] - sd[0] * m0; mo.s[1] = sq[1] - sd[0] * m1; mo.s[2] = sq[2] - sd[0] * m2;
   mo.s[3] = sq[3] - sd[1] * m1; mo.s[4] = sq[4] - sd[1] * m2; mo.s[5] = sq[5] - sd[2] * m2;
 }
@@ -276,13 +290,16 @@ reduce_kernel(Ctl *ctl, const float4 *buf_a, const float4 *buf_b, VoxMoments *mo
 
   // ---- one thread per run: shifted one-pass sums from shared memory (first round kept in
   //      registers so that the look-back below overlaps with nothing but finished work)
-  auto run_moments = [&](int j, Moments &mo) -> bool {
+  auto run_moments = [&](int j, Moments &mo, u64 &key) -> bool {
     const int s = S.run_start[j], e = S.run_start[j + 1];
     if (e - s > kLongRun) {
       S.long_list[atomicAdd(&S.n_long, 1u)] = (unsigned short)j;
       return false;
     }
     const float4 p0 = pts[s];
+    key = point_key<FAST>(p0, o, P);
+    double anc[3];
+    cell_anchor(key, o, P.grid_len, P.z_len, anc);
     double sd[3] = {0, 0, 0}, sq[6] = {0, 0, 0, 0, 0, 0};
     for (int i = s + 1; i < e; ++i) {
       const float4 p = pts[i];
@@ -290,11 +307,12 @@ reduce_kernel(Ctl *ctl, const float4 *buf_a, const float4 *buf_b, VoxMoments *mo
       sd[0] += dx; sd[1] += dy; sd[2] += dz;
       sq[0] += dx * dx; sq[1] += dx * dy; sq[2] += dx * dz; sq[3] += dy * dy; sq[4] += dy * dz; sq[5] += dz * dz;
     }
-    close_moments(mo, (double)(e - s), p0, sd, sq);
+    close_moments(mo, (double)(e - s), p0, anc, sd, sq);
     return true;
   };
   Moments mo0;
-  const bool have0 = (tid < n_runs) && run_moments(tid, mo0);
+  u64 key0;
+  const bool have0 = (tid < n_runs) && run_moments(tid, mo0, key0);
 
   if (warp == kRedThreads / 32 - 1) {  // the last warp has the fewest runs of its own: it resolves the voxel base
     const u64 vb = warp_lookback_grouped(tile_state, tile_groups, tile, 0u, heads, &ctl->err);
@@ -305,7 +323,7 @@ reduce_kernel(Ctl *ctl, const float4 *buf_a, const float4 *buf_b, VoxMoments *mo
   if (tid == 0 && base + cnt == M) ctl->n_voxels = vox_base + heads;
   TileCarry *my_carry = carry + tile;
 
-  auto emit = [&](int j, const Moments &mo) {
+  auto emit = [&](int j, const Moments &mo, u64 key) {
     const int s = S.run_start[j];
     const bool cont = (j == 0) && !first_is_head;
     const bool open_end = (j == n_runs - 1) && !last_complete;
@@ -316,16 +334,17 @@ reduce_kernel(Ctl *ctl, const float4 *buf_a, const float4 *buf_b, VoxMoments *mo
       return;
     }
     if (slot >= P.max_voxels) { atomicOr(&ctl->err, kErrCapacity); return; }
-    store_moments(mom + slot, point_key<FAST>(pts[s], o, P), __float_as_uint(pts[s].w), mo);
+    store_moments(mom + slot, key, __float_as_uint(pts[s].w), mo);
     if (open_end) {
       my_carry->tail_slot = slot;
       atomicOr(&my_carry->flags, kCarryHasTail);
     }
   };
-  if (have0) emit(tid, mo0);
+  if (have0) emit(tid, mo0, key0);
   for (int j = tid + kRedThreads; j < n_runs; j += kRedThreads) {
     Moments mo;
-    if (run_moments(j, mo)) emit(j, mo);
+    u64 key;
+    if (run_moments(j, mo, key)) emit(j, mo, key);
   }
   __syncthreads();
 
@@ -346,9 +365,12 @@ reduce_kernel(Ctl *ctl, const float4 *buf_a, const float4 *buf_b, VoxMoments *mo
 #pragma unroll
     for (int k = 0; k < 9; ++k) acc[k] = warp_sum(acc[k]);
     if (lane == 0) {
+      const u64 key = point_key<FAST>(p0, o, P);
+      double anc[3];
+      cell_anchor(key, o, P.grid_len, P.z_len, anc);
       Moments mo;
-      close_moments(mo, (double)(e - s), p0, acc, acc + 3);
-      emit(j, mo);
+      close_moments(mo, (double)(e - s), p0, anc, acc, acc + 3);
+      emit(j, mo, key);
     }
   }
 }

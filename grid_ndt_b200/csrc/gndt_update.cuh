@@ -68,13 +68,29 @@ __device__ __forceinline__ void load_moments(const VoxMoments &v, Moments &m) {
 }
 
 // Inverse of merge_moments: a = c (+) b  ->  a becomes c.  Needs a.n > b.n.
+// Means are relative to the cell centre (gndt_reduce.cuh), so the mean cancellation below loses
+// at most the rounding of a cell-sized value.  The scatter c.s = a.s - b.s - d d^T w still cancels
+// two large sums when a few points survive a large mass: an entry within a few rounding units of
+// that cancellation is noise and is set to 0, so that survivors whose batch scatter is exactly 0
+// (identical points) or rank 1 (collinear points) get it back.  The bound of entry (i, j) is
+// eps * sqrt(B_i B_j), B_i = |a.s_ii| + |b.s_ii| + d_i^2 w: a PSD matrix's off-diagonal entry is
+// bounded by the geometric mean of its diagonal ones, and so is its error.
+constexpr double kUnmergeTol = 8.0 * 2.220446049250313e-16;
 __device__ __forceinline__ void unmerge_moments(Moments &a, const Moments &b) {
   const double n = a.n - b.n;
   const double c0 = (a.n * a.m[0] - b.n * b.m[0]) / n, c1 = (a.n * a.m[1] - b.n * b.m[1]) / n, c2 = (a.n * a.m[2] - b.n * b.m[2]) / n;
-  const double d0 = b.m[0] - c0, d1 = b.m[1] - c1, d2 = b.m[2] - c2;
+  const double d[3] = {b.m[0] - c0, b.m[1] - c1, b.m[2] - c2};
   const double w = n * b.n / a.n;
-  a.s[0] -= b.s[0] + d0 * d0 * w; a.s[1] -= b.s[1] + d0 * d1 * w; a.s[2] -= b.s[2] + d0 * d2 * w;
-  a.s[3] -= b.s[3] + d1 * d1 * w; a.s[4] -= b.s[4] + d1 * d2 * w; a.s[5] -= b.s[5] + d2 * d2 * w;
+  double bound[3];
+  const int diag[3] = {0, 3, 5};
+#pragma unroll
+  for (int i = 0; i < 3; ++i) bound[i] = sqrt(fabs(a.s[diag[i]]) + fabs(b.s[diag[i]]) + d[i] * d[i] * w);
+  const int ri[6] = {0, 0, 0, 1, 1, 2}, rj[6] = {0, 1, 2, 1, 2, 2};
+#pragma unroll
+  for (int k = 0; k < 6; ++k) {
+    const double s = a.s[k] - (b.s[k] + d[ri[k]] * d[rj[k]] * w);
+    a.s[k] = fabs(s) <= kUnmergeTol * bound[ri[k]] * bound[rj[k]] ? 0.0 : s;
+  }
   a.m[0] = c0; a.m[1] = c1; a.m[2] = c2;
   a.n = n;
 }

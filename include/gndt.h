@@ -223,10 +223,16 @@ int gndt_update(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, 
  * backwards on the binary64 moments; voxels that lose all their points disappear).
  * Replaces: delCallback + uniformDelDivision + del2DMap (src/receiver.cpp:95-134,214-248;
  * include/map2D.h:826-915), commented out at every call site in the reference.  Contract:
- * build(A) + update(B) + remove(B) equals build(A) (first_index of a surviving voxel keeps
- * the value it had, which is the same thing whenever B was fused after A).  Every point of
- * the scan must have been fused before: otherwise the call fails with GNDT_ERR_STATE at the
- * next result query and the map is left unchanged.
+ * build(A) + update(B) + remove(B) equals build(A).  A remove gives its points' cloud indices
+ * back (n_input and the index of the next update's first point both drop by n), so:
+ *   - removing the most recent scan(s) restores the index space exactly: a later update(C)
+ *     equals build(A ++ C), first_index and morton_list order included;
+ *   - removing an older scan leaves first_index where it was for the voxels later scans
+ *     touched first, and a later update may reuse those indices: renumbering them exactly
+ *     would need per-point state the map does not keep.  Everything else (cells, counts,
+ *     moments, labels under GNDT_DEMAND_TRUE) equals the batch build without that scan.
+ * Every point of the scan must have been fused before: otherwise the call fails with
+ * GNDT_ERR_STATE at the next result query and the map is left unchanged.
  */
 int gndt_remove(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem,
                 void *stream);
