@@ -139,3 +139,43 @@ class PointCloud2(C.Structure):
     _fields_ = [("data", C.c_void_p), ("width", C.c_uint32), ("height", C.c_uint32), ("point_step", C.c_uint32),
                 ("x_offset", C.c_uint32), ("y_offset", C.c_uint32), ("z_offset", C.c_uint32),
                 ("is_bigendian", C.c_uint8), ("host_pinned", C.c_uint8), ("reserved", C.c_uint8 * 2)]
+
+
+NDT_CONVERGED, NDT_STALLED, NDT_MAX_ITER, NDT_NO_MATCH = 0, 1, 2, 3
+NDT_TERMINATION = ("converged", "stalled", "max_iter", "no_match")
+
+
+class NdtParams(C.Structure):
+    """gndt_ndt_params (include/gndt.h): settings of one gndt_register call."""
+
+    _fields_ = [("outlier_ratio", C.c_float), ("min_voxel_points", C.c_int32), ("max_iterations", C.c_int32),
+                ("reserved", C.c_int32), ("translation_epsilon", C.c_double), ("rotation_epsilon", C.c_double)]
+
+
+def default_ndt_params(**kw) -> NdtParams:
+    """gndt_default_ndt_params with any field overridden by keyword."""
+    p = NdtParams(0.55, 6, 100, 0, 1e-4, 1e-4)
+    for k, v in kw.items():
+        if k not in dict(NdtParams._fields_):
+            raise TypeError(f"unknown NDT parameter {k!r}")
+        setattr(p, k, v)
+    return p
+
+
+class Registration(C.Structure):
+    """gndt_registration (include/gndt.h): result of gndt_register."""
+
+    _fields_ = [("pose", C.c_double * 16), ("center", C.c_double * 3), ("score", C.c_double), ("gradient", C.c_double * 6),
+                ("hessian", C.c_double * 36), ("n_points", C.c_uint64), ("n_matched", C.c_uint64), ("n_pairs", C.c_uint64),
+                ("iterations", C.c_uint32), ("termination", C.c_int32)]
+
+    def as_dict(self):
+        return {
+            "pose": np.array(self.pose[:], np.float64).reshape(4, 4),
+            "center": np.array(self.center[:], np.float64),
+            "score": float(self.score),
+            "gradient": np.array(self.gradient[:], np.float64),
+            "hessian": np.array(self.hessian[:], np.float64).reshape(6, 6),
+            "n_points": int(self.n_points), "n_matched": int(self.n_matched), "n_pairs": int(self.n_pairs),
+            "iterations": int(self.iterations), "termination": int(self.termination),
+        }

@@ -5,14 +5,14 @@ import os
 import subprocess
 import sys
 
-from ._abi import Counts, Params, PointCloud2, XchgInfo, XchgView
+from ._abi import Counts, NdtParams, Params, PointCloud2, Registration, XchgInfo, XchgView
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(HERE)
 LIB_PATH = os.environ.get("GNDT_LIB") or os.path.join(HERE, "libgndt.so")  # GNDT_LIB: tuning variants only
 SOURCES = [os.path.join(HERE, "csrc", f) for f in (
     "gndt_api.cu", "gndt_device.cuh", "gndt_sort.cuh", "gndt_reduce.cuh", "gndt_label.cuh", "gndt_update.cuh",
-    "gndt_exchange.cuh", "gndt_graph.cuh", "gndt_scan.cuh")]
+    "gndt_exchange.cuh", "gndt_graph.cuh", "gndt_scan.cuh", "gndt_ndt.cuh")]
 HEADER = os.path.join(REPO, "include", "gndt.h")
 LOOKUP_HEADER = os.path.join(REPO, "include", "gndt_lookup.h")
 
@@ -96,6 +96,8 @@ SYMBOLS = {
     "gndt_cell_center": (_i, [C.POINTER(C.c_float), C.c_float, C.c_float, C.c_int32, C.c_int32, C.c_int32,
                               C.POINTER(C.c_float)]),
     "gndt_origin": (_i, [_vp, C.POINTER(C.c_float)]),
+    "gndt_default_ndt_params": (None, [C.POINTER(NdtParams)]),
+    "gndt_register": (_i, [_vp, _vp, _sz, _sz, _i, C.POINTER(C.c_double), C.POINTER(NdtParams), C.POINTER(Registration), _vp]),
     "gndt_key_layout": (_i, [_vp, C.POINTER(C.c_int)]),
     "gndt_find_column": (C.c_int64, [_vp, _sz, C.c_int32, C.c_int32]),
     "gndt_find_slope": (C.c_int64, [_vp, _sz, _vp, C.c_int32, C.c_int32, C.c_int32]),

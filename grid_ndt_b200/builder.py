@@ -204,6 +204,24 @@ class TwoDmap:
         self._views.clear()
         return True
 
+    def register(self, scan, guess=None, stream: Optional[int] = None, **ndt) -> dict:
+        """NDT registration of a scan against the resident map (gndt_register): the pose
+        map <- scan that best fits it, from `guess` (4x4, identity when None).  Keywords set
+        gndt_ndt_params fields (outlier_ratio, min_voxel_points, max_iterations,
+        translation_epsilon, rotation_epsilon).  Returns the gndt_registration fields as a dict;
+        pose is a 4x4 float64 array, termination one of _abi.NDT_*.  The map is not changed."""
+        ptr, n, stride, mem, st, keep = self._marshal(scan)
+        if stream is not None:
+            st = stream
+        T = np.eye(4) if guess is None else np.ascontiguousarray(guess, dtype=np.float64)
+        if T.shape != (4, 4):
+            raise GndtError(-1, "guess must be a 4x4 matrix")
+        np_ = _abi.default_ndt_params(**ndt)
+        out = _abi.Registration()
+        _check(self._h, lib().gndt_register(self._h, ptr, n, stride, mem, T.ctypes.data_as(C.POINTER(C.c_double)),
+                                            C.byref(np_), C.byref(out), st))
+        return out.as_dict()
+
     @property
     def changed_columns(self) -> np.ndarray:
         """Indices (into `columns`) of the cells the last change2DMap / del2DMap touched, in

@@ -22,6 +22,7 @@
 #include "gndt_update.cuh"
 #include "gndt_exchange.cuh"
 #include "gndt_graph.cuh"
+#include "gndt_ndt.cuh"
 #include <unistd.h>
 
 using namespace gndt;
@@ -92,6 +93,10 @@ struct gndt_handle {
   Buffer g_work, g_off, g_tgt;
   size_t g_slopes = 0, g_targets = 0;
   bool g_valid = false;
+  // NDT registration (gndt_register): Gaussians of the resident map, scan upload, per-block partials
+  Buffer ndt_vox, ndt_pts, ndt_part;
+  double *ndt_host = nullptr;  // pinned read-back of one pass
+  bool ndt_ready = false;      // ndt_vox describes the resident map (cleared by build / update / remove)
   // peer-mapped strip exchange (gndt_xchg_*)
   Buffer xbuf;
   XLayout xl = {};
@@ -530,9 +535,11 @@ int gndt_destroy(gndt_handle *h) {
   if (h->x_ev_counts) cudaEventDestroy(h->x_ev_counts);
   if (h->x_ev_copy) cudaEventDestroy(h->x_ev_copy);
   if (h->x_counts_host) cudaFreeHost(h->x_counts_host);
+  if (h->ndt_host) cudaFreeHost(h->ndt_host);
   if (h->ring) { cudaFreeHost(h->ring); for (int i = 0; i < 4; ++i) if (h->ring_ev[i]) cudaEventDestroy(h->ring_ev[i]); }
   Buffer *bufs[] = {&h->in_stage, &h->buf_a, &h->buf_b, &h->zero, &h->mom, &h->mom_alt, &h->table, &h->slopes,
-                    &h->columns, &h->vfirst, &h->slope_col, &h->mom_scan, &h->upd_work, &h->msg_points, &h->small, &h->lookback, &h->f_zero, &h->xbuf, &h->g_work, &h->g_off, &h->g_tgt};
+                    &h->columns, &h->vfirst, &h->slope_col, &h->mom_scan, &h->upd_work, &h->msg_points, &h->small, &h->lookback, &h->f_zero, &h->xbuf, &h->g_work, &h->g_off, &h->g_tgt,
+                    &h->ndt_vox, &h->ndt_pts, &h->ndt_part};
   for (Buffer *b : bufs) if (b->p) cudaFree(b->p);
   for (int i = 0; i < EV_COUNT; ++i) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
   delete h;
@@ -552,6 +559,7 @@ int gndt_set_params(gndt_handle *h, const gndt_params *params) {
 static int build_device(gndt_handle *h, const float *d_in, size_t n, size_t stride_bytes, cudaStream_t st) {
   const size_t start = h->params.origin_is_first_point ? 1 : 0;
   const DevParams dp = make_dev(h, h->params, h->cap_voxels);
+  h->ndt_ready = false;
   GNDT_CUDA(h, cudaEventRecord(h->ev[EV_START], st));
   int rc = front_end(h, st, d_in, n, stride_bytes / 4, start, dp, (VoxMoments *)h->mom.p);
   if (rc != GNDT_OK) return rc;
@@ -697,6 +705,7 @@ static int fuse_scan(gndt_handle *h, const void *xyz, size_t n, size_t stride_by
   h->counts_valid = false;
   h->launches = 0;
   h->n_changed_valid = false;
+  h->ndt_ready = false;  // recomputed by the next gndt_register whatever the verdict
 
   // capacity: every scan point could open a new voxel
   size_t cap_vox = h->cap_voxels;
@@ -1569,6 +1578,238 @@ int gndt_origin(gndt_handle *h, float origin[3]) {
   int rc = sync_counts(h);
   if (rc != GNDT_OK) return rc;
   for (int i = 0; i < 3; ++i) origin[i] = h->host_ctl.origin[i];
+  return GNDT_OK;
+}
+
+// ---- NDT scan-to-map registration -------------------------------------------------------
+
+void gndt_default_ndt_params(gndt_ndt_params *p) {
+  if (!p) return;
+  memset(p, 0, sizeof(*p));
+  p->outlier_ratio = 0.55f;
+  p->min_voxel_points = 6;
+  p->max_iterations = 100;
+  p->translation_epsilon = 1e-4;
+  p->rotation_epsilon = 1e-4;
+}
+
+namespace {
+
+struct NdtEval {  // one pass at one pose
+  double score, g[6], H[36], c[3];
+  uint64_t n_points, n_matched, n_pairs;
+};
+
+// Exp(phi) of so(3) (Rodrigues), row-major
+void so3_exp(const double phi[3], double E[9]) {
+  const double th2 = phi[0] * phi[0] + phi[1] * phi[1] + phi[2] * phi[2], th = std::sqrt(th2);
+  const double a = th2 < 1e-24 ? 1.0 - th2 / 6.0 : std::sin(th) / th;
+  const double b = th2 < 1e-24 ? 0.5 - th2 / 24.0 : (1.0 - std::cos(th)) / th2;
+  const double K[9] = {0.0, -phi[2], phi[1], phi[2], 0.0, -phi[0], -phi[1], phi[0], 0.0};
+  for (int i = 0; i < 3; ++i)
+    for (int j = 0; j < 3; ++j) {
+      double kk = 0.0;
+      for (int m = 0; m < 3; ++m) kk += K[3 * i + m] * K[3 * m + j];
+      E[3 * i + j] = (i == j ? 1.0 : 0.0) + a * K[3 * i + j] + b * kk;
+    }
+}
+
+// Cholesky solve of the 6x6 system A x = b; false if A is not positive definite
+bool chol6(const double A_in[36], const double b[6], double x[6]) {
+  double L[36] = {};
+  for (int i = 0; i < 6; ++i)
+    for (int j = 0; j <= i; ++j) {
+      double s = A_in[6 * i + j];
+      for (int k = 0; k < j; ++k) s -= L[6 * i + k] * L[6 * j + k];
+      if (i == j) {
+        if (!(s > 0.0) || !std::isfinite(s)) return false;
+        L[6 * i + i] = std::sqrt(s);
+      } else {
+        L[6 * i + j] = s / L[6 * j + j];
+      }
+    }
+  double y[6];
+  for (int i = 0; i < 6; ++i) {
+    double s = b[i];
+    for (int k = 0; k < i; ++k) s -= L[6 * i + k] * y[k];
+    y[i] = s / L[6 * i + i];
+  }
+  for (int i = 5; i >= 0; --i) {
+    double s = y[i];
+    for (int k = i + 1; k < 6; ++k) s -= L[6 * k + i] * x[k];
+    x[i] = s / L[6 * i + i];
+  }
+  return true;
+}
+
+int ndt_check_args(gndt_handle *h, const double *T, const gndt_ndt_params *np) {
+  for (int i = 0; i < 16; ++i)
+    if (!std::isfinite(T[i])) { h->err = "gndt_register: the guess is not finite"; return GNDT_ERR_INVALID_ARG; }
+  if (T[12] != 0.0 || T[13] != 0.0 || T[14] != 0.0 || T[15] != 1.0) { h->err = "gndt_register: the guess's bottom row is not 0 0 0 1"; return GNDT_ERR_INVALID_ARG; }
+  for (int i = 0; i < 3; ++i)
+    for (int j = 0; j < 3; ++j) {
+      const double rtr = T[i] * T[j] + T[4 + i] * T[4 + j] + T[8 + i] * T[8 + j];  // (R^T R)_ij
+      if (!(std::fabs(rtr - (i == j ? 1.0 : 0.0)) <= 1e-6)) { h->err = "gndt_register: the guess's rotation is not orthonormal"; return GNDT_ERR_INVALID_ARG; }
+    }
+  if (!(np->outlier_ratio > 0.f && np->outlier_ratio < 1.f) || np->min_voxel_points < 3 || np->max_iterations < 0 || np->reserved != 0 ||
+      !(np->translation_epsilon >= 0.0) || !(np->rotation_epsilon >= 0.0) || !std::isfinite(np->translation_epsilon) ||
+      !std::isfinite(np->rotation_epsilon)) {
+    h->err = "gndt_register: ndt parameter out of range";
+    return GNDT_ERR_INVALID_ARG;
+  }
+  return GNDT_OK;
+}
+
+}  // namespace
+
+int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, const double guess[16],
+                  const gndt_ndt_params *np, gndt_registration *out, void *stream) {
+  if (!h) return GNDT_ERR_INVALID_ARG;
+  if (!guess || !np || !out) { h->err = "gndt_register: guess, np and out must not be NULL"; return GNDT_ERR_INVALID_ARG; }
+  int rc = check_cloud_args(h, xyz, n, stride_bytes, mem, "gndt_register");
+  if (rc != GNDT_OK) return rc;
+  if ((rc = ndt_check_args(h, guess, np)) != GNDT_OK) return rc;
+  GNDT_CUDA(h, cudaSetDevice(h->device));
+  if ((rc = sync_counts(h)) != GNDT_OK) return rc;  // resolves a pending update / remove
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const gndt_params &rp = h->res_params;
+  const u32 n_vox = h->host_ctl.n_voxels, n_cols = h->host_ctl.n_columns;
+
+  // the resident map's Gaussians, once per map state
+  if (!h->ndt_ready) {
+    if ((rc = ensure(h, h->ndt_vox, std::max<size_t>(n_vox, 1) * sizeof(NdtVoxel))) != GNDT_OK) return rc;
+    ndt_prepare_kernel<<<grid_for(h, n_vox, 256, 8), 256, 0, st>>>(h->ctl, (const gndt_voxel *)h->table.p, (NdtVoxel *)h->ndt_vox.p,
+                                                                   rp.normalize_cov);
+  }
+  const float *d_in = static_cast<const float *>(xyz);
+  if (mem == GNDT_MEM_HOST) {
+    if ((rc = ensure(h, h->ndt_pts, n * stride_bytes)) != GNDT_OK) return rc;
+    GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_pts.p, xyz, n * stride_bytes, cudaMemcpyHostToDevice, st));
+    d_in = static_cast<const float *>(h->ndt_pts.p);
+  }
+  const int blocks = grid_for(h, n, kNdtThreads, 8);
+  if ((rc = ensure(h, h->ndt_part, ((size_t)blocks + 1) * kNdtWidth * sizeof(double))) != GNDT_OK) return rc;
+  if (!h->ndt_host) GNDT_CUDA(h, cudaHostAlloc(&h->ndt_host, kNdtWidth * sizeof(double), cudaHostAllocDefault));
+  double *part = static_cast<double *>(h->ndt_part.p), *dres = part + (size_t)blocks * kNdtWidth;
+  const size_t stride_f = stride_bytes / 4;
+
+  // centre: binary64 mean of the finite points, c = R pbar + t at every pose
+  ndt_mean_kernel<<<blocks, kNdtThreads, 0, st>>>(d_in, stride_f, n, part);
+  ndt_finish_kernel<<<1, 32, 0, st>>>(part, blocks, 4, dres);
+  GNDT_CUDA(h, cudaGetLastError());
+  GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_host, dres, 4 * sizeof(double), cudaMemcpyDeviceToHost, st));
+  GNDT_CUDA(h, cudaStreamSynchronize(st));
+  h->ndt_ready = true;
+  const uint64_t n_points = (uint64_t)h->ndt_host[3];
+  const double pbar[3] = {n_points ? h->ndt_host[0] / (double)n_points : 0.0, n_points ? h->ndt_host[1] / (double)n_points : 0.0,
+                          n_points ? h->ndt_host[2] / (double)n_points : 0.0};
+
+  NdtPose P = {};
+  {
+    const double p_o = np->outlier_ratio, V = (double)rp.grid_len * (double)rp.grid_len * (double)rp.z_len;
+    const double c1 = 10.0 * (1.0 - p_o), c2 = p_o / V, d3 = -std::log(c2);
+    P.d1 = -std::log(c1 + c2) - d3;
+    P.d2 = -2.0 * std::log((-std::log(c1 * std::exp(-0.5) + c2) - d3) / P.d1);
+  }
+  for (int i = 0; i < 3; ++i) P.origin[i] = h->host_ctl.origin[i];
+  P.grid_len = rp.grid_len;
+  P.z_len = rp.z_len;
+  P.min_points = (u32)np->min_voxel_points;
+
+  auto eval = [&](const double T[16], NdtEval &e) -> int {
+    for (int i = 0; i < 3; ++i) {
+      for (int j = 0; j < 3; ++j) P.r[3 * i + j] = T[4 * i + j];
+      P.t[i] = T[4 * i + 3];
+      P.c[i] = T[4 * i] * pbar[0] + T[4 * i + 1] * pbar[1] + T[4 * i + 2] * pbar[2] + T[4 * i + 3];
+    }
+    ndt_pass_kernel<<<blocks, kNdtThreads, 0, st>>>(d_in, stride_f, n, (const NdtVoxel *)h->ndt_vox.p, (const gndt_column *)h->columns.p,
+                                                    n_cols, P, part);
+    ndt_finish_kernel<<<1, 32, 0, st>>>(part, blocks, kNdtWidth, dres);
+    GNDT_CUDA(h, cudaGetLastError());
+    GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_host, dres, kNdtWidth * sizeof(double), cudaMemcpyDeviceToHost, st));
+    GNDT_CUDA(h, cudaStreamSynchronize(st));
+    const double *r = h->ndt_host;
+    e.score = r[0];
+    for (int k = 0; k < 6; ++k) e.g[k] = r[1 + k];
+    for (int k = 0, idx = 7; k < 6; ++k)
+      for (int l = k; l < 6; ++l, ++idx) e.H[6 * k + l] = e.H[6 * l + k] = r[idx];
+    for (int i = 0; i < 3; ++i) e.c[i] = P.c[i];
+    e.n_points = (uint64_t)r[28];
+    e.n_matched = (uint64_t)r[29];
+    e.n_pairs = (uint64_t)r[30];
+    return GNDT_OK;
+  };
+
+  double T[16];
+  memcpy(T, guess, sizeof(T));
+  NdtEval cur;
+  if ((rc = eval(T, cur)) != GNDT_OK) return rc;
+  int term = GNDT_NDT_MAX_ITER;
+  uint32_t iters = 0;
+  if (cur.n_pairs == 0) {
+    term = GNDT_NDT_NO_MATCH;
+    cur.score = 0.0;
+    memset(cur.g, 0, sizeof(cur.g));
+    memset(cur.H, 0, sizeof(cur.H));
+  } else {
+    // Levenberg-Marquardt on -S: (-H + lambda diag(max(-H_ii, tiny))) delta = g
+    constexpr double kLambda0 = 1e-3, kLambdaMin = 1e-12, kLambdaMax = 1e12;
+    double lambda = kLambda0;
+    while (iters < (uint32_t)np->max_iterations) {
+      double hmax = 0.0;
+      for (int i = 0; i < 6; ++i) hmax = std::max(hmax, std::fabs(cur.H[7 * i]));
+      const double tiny = std::max(1e-6 * hmax, 1e-300);
+      double A[36], delta[6];
+      for (int i = 0; i < 36; ++i) A[i] = -cur.H[i];
+      for (int i = 0; i < 6; ++i) A[7 * i] += lambda * std::max(-cur.H[7 * i], tiny);
+      if (!chol6(A, cur.g, delta)) {
+        lambda *= 10.0;
+        if (lambda > kLambdaMax) { term = GNDT_NDT_STALLED; break; }
+        continue;
+      }
+      // converged: the (nearly undamped) step to the optimum of the local model is below both
+      // epsilons.  Tested before the pass because there S need not rise any more: candidate sets
+      // change between poses, and on the tails of thin Gaussians the Hessian is indefinite, lambda
+      // grows and steps shrink far from the optimum, so a short damped step says nothing
+      const double dr = std::sqrt(delta[0] * delta[0] + delta[1] * delta[1] + delta[2] * delta[2]);
+      const double dp = std::sqrt(delta[3] * delta[3] + delta[4] * delta[4] + delta[5] * delta[5]);
+      if (lambda < 1.0 && dr < np->translation_epsilon && dp < np->rotation_epsilon) { term = GNDT_NDT_CONVERGED; break; }
+      // candidate: T' = (E, c + rho - E c) o T, E = Exp(phi)
+      double E[9], Tn[16];
+      so3_exp(delta + 3, E);
+      memcpy(Tn, T, sizeof(Tn));
+      for (int i = 0; i < 3; ++i) {
+        double tt = cur.c[i] + delta[i];
+        for (int j = 0; j < 3; ++j) {
+          Tn[4 * i + j] = E[3 * i] * T[j] + E[3 * i + 1] * T[4 + j] + E[3 * i + 2] * T[8 + j];
+          tt += E[3 * i + j] * (T[4 * j + 3] - cur.c[j]);
+        }
+        Tn[4 * i + 3] = tt;
+      }
+      NdtEval cand;
+      if ((rc = eval(Tn, cand)) != GNDT_OK) return rc;
+      ++iters;
+      if (cand.score > cur.score) {
+        memcpy(T, Tn, sizeof(T));
+        cur = cand;
+        lambda = std::max(lambda / 10.0, kLambdaMin);
+      } else {
+        lambda *= 10.0;
+        if (lambda > kLambdaMax) { term = GNDT_NDT_STALLED; break; }
+      }
+    }
+  }
+  memset(out, 0, sizeof(*out));
+  memcpy(out->pose, T, sizeof(T));
+  memcpy(out->center, cur.c, sizeof(cur.c));
+  out->score = cur.score;
+  memcpy(out->gradient, cur.g, sizeof(cur.g));
+  memcpy(out->hessian, cur.H, sizeof(cur.H));
+  out->n_points = n_points;
+  out->n_matched = cur.n_matched;
+  out->n_pairs = cur.n_pairs;
+  out->iterations = iters;
+  out->termination = term;
   return GNDT_OK;
 }
 

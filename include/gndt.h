@@ -402,6 +402,81 @@ int gndt_launch_count(gndt_handle *h, uint64_t *n_launches);
  * operands were compared.  GNDT_EXACT_DIV=1 in the environment forces the plain division. */
 int gndt_fast_div_status(gndt_handle *h, int *enabled, uint64_t *values_checked);
 
+/*
+ * NDT scan-to-map registration (Biber & Strasser 2003; Magnusson 2009, ch. 6): the rigid pose
+ * T (map <- scan) that maximises the NDT score of a scan against the normal distributions the
+ * resident map keeps per voxel.  The usual streaming loop is register, transform, gndt_update.
+ *
+ * Contract of gndt_register:
+ *   - Blocking: returns when the result is in *out.  Scans as for gndt_update (stride, host or
+ *     device memory, same argument checks); every point is used, there is no strip filter.
+ *   - A gndt_update / gndt_remove still awaiting its verdict is resolved first; if it failed,
+ *     its status (GNDT_ERR_CAPACITY / GNDT_ERR_STATE) is returned and the next call registers
+ *     against the unchanged map.
+ *   - GNDT_ERR_STATE without a successful build.  GNDT_ERR_INVALID_ARG when guess, np or out is
+ *     NULL, the guess is not finite, its bottom row is not exactly 0 0 0 1, max|R^T R - I| > 1e-6,
+ *     or a parameter is out of range.
+ *   - Nothing of the map changes: voxel / slope / column tables, counts, changed columns, key
+ *     layout, stage times and gndt_launch_count stay as they were.  The call uses its own
+ *     scratch and registers against the map with the parameters and origin it was built with
+ *     (later gndt_set_params values do not apply).
+ *
+ * Objective.  For a finite scan point p (binary32) and pose (R, t): x' = R p + t in binary64,
+ * each component ((R_i0 p0 + R_i1 p1) + R_i2 p2) + t_i with every operation rounded on its own
+ * (no FMA).  The candidates of x' are the voxels of x' rounded to binary32 (cell as in binning,
+ * resident origin and cell lengths; none when the index is out of range) whose column is the
+ * point's own or one of its 4 edge neighbours (cx +-1 or cy +-1) and whose |cz_v - cz| <= 1, at
+ * most 15, that are GNDT_F_FITTED, have count >= min_voxel_points and a usable Gaussian: mu =
+ * mean, Sigma = scatter / (n - 1) (normalize_cov == 0) or scatter * n / (n - 1), eigenvalues
+ * raised to >= 0.01 lambda_max (unusable if lambda_max <= 0), C = Sigma'^-1.  With V = grid_len^2
+ * z_len, c1 = 10 (1 - p_o), c2 = p_o / V, d3 = -ln c2, d1 = -ln(c1 + c2) - d3,
+ * d2 = -2 ln((-ln(c1 e^-1/2 + c2) - d3) / d1), d = x' - mu, every (point, voxel) pair adds
+ * -d1 exp(-d2 d^T C d / 2) to the score S.  Gradient and Hessian are those of S over the
+ * increment xi = (rho, phi) that maps x' to Exp(phi)(x' - c) + c + rho, at xi = 0, candidates
+ * frozen; c = R pbar + t, pbar the binary64 mean of the finite points.  An accepted step
+ * updates T <- (Exp(phi), c + rho - Exp(phi) c) o T.
+ *
+ * Solver: Levenberg-Marquardt on -S on the host, one pass over the scan on the device per
+ * pose: (-H + lambda diag(max(-H_ii, 1e-6 max|H_ii|))) delta = g, lambda from 1e-3, / 10 on an
+ * accepted step, * 10 on a rejected one or a failed Cholesky, STALLED above 1e12.  A step is
+ * accepted only if S strictly rises; out->pose is the last accepted pose (the guess
+ * when none was) and score / gradient / hessian / center / counts are those of that pose, so a
+ * max_iterations = 0 call at out->pose reproduces them bit for bit.  Results are bitwise
+ * repeatable for the same inputs on the same device.
+ */
+typedef struct gndt_ndt_params {
+  float outlier_ratio;        /* Magnusson's p_o in (0, 1); default 0.55 (PCL's default)          */
+  int32_t min_voxel_points;   /* voxels with fewer points are not used; default 6, must be >= 3   */
+  int32_t max_iterations;     /* derivative passes after the first; 0 = evaluate the guess only   */
+  int32_t reserved;           /* must be 0                                                        */
+  double translation_epsilon; /* converged when the solved step moves less than this (m) ...      */
+  double rotation_epsilon;    /* ... and rotates less than this (rad); |rho| and |phi| of the
+                                 step; defaults 1e-4 m and 1e-4 rad, both finite and >= 0        */
+} gndt_ndt_params;
+void gndt_default_ndt_params(gndt_ndt_params *p);
+
+enum { GNDT_NDT_CONVERGED = 0, GNDT_NDT_STALLED = 1, GNDT_NDT_MAX_ITER = 2, GNDT_NDT_NO_MATCH = 3 };
+
+typedef struct gndt_registration {
+  double pose[16];           /* row-major 4x4 map <- scan; the guess when nothing was accepted     */
+  double center[3];          /* c of the objective at `pose`: R pbar + t                           */
+  double score;              /* S, gradient and Hessian at `pose`                                  */
+  double gradient[6];        /* order: rho_x, rho_y, rho_z, phi_x, phi_y, phi_z                     */
+  double hessian[36];        /* row-major; -H^-1 is the usual pose covariance estimate              */
+  uint64_t n_points;         /* finite points of the scan                                          */
+  uint64_t n_matched;        /* points with at least one candidate voxel at `pose`                 */
+  uint64_t n_pairs;          /* (point, voxel) pairs at `pose`                                     */
+  uint32_t iterations;       /* derivative passes run after the first                              */
+  int32_t termination;       /* GNDT_NDT_*: CONVERGED = the solved step at `pose` is below both
+                                epsilons with damping lambda < 1 (lambda starts at 1e-3),
+                                STALLED = no improving step before the damping limit, MAX_ITER,
+                                NO_MATCH = no pair at the guess (pose = guess, S, g, H = 0)       */
+} gndt_registration;
+
+int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem,
+                  const double guess[16], const gndt_ndt_params *np, gndt_registration *out,
+                  void *stream);
+
 /* ---- host-side key helpers (pure C, no device) ------------------------------------- */
 
 /* TwoDmap::transMortonXYZ (include/map2D.h:950-976) for one position: signed non-zero
