@@ -9,7 +9,7 @@ from ._abi import Counts, NdtParams, Params, PointCloud2, Registration, XchgInfo
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(HERE)
-LIB_PATH = os.environ.get("GNDT_LIB") or os.path.join(HERE, "libgndt.so")  # GNDT_LIB: tuning variants only
+LIB_PATH = os.environ.get("GNDT_LIB") or os.path.join(HERE, "libgndt.so")  # GNDT_LIB: another build, for A/B runs
 SOURCES = [os.path.join(HERE, "csrc", f) for f in (
     "gndt_api.cu", "gndt_device.cuh", "gndt_sort.cuh", "gndt_reduce.cuh", "gndt_label.cuh", "gndt_update.cuh",
     "gndt_exchange.cuh", "gndt_graph.cuh", "gndt_scan.cuh", "gndt_ndt.cuh")]

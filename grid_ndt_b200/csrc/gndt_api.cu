@@ -44,6 +44,17 @@ struct DivCheck {  // result of the exhaustive hoisted-division check for one ce
   int ok = 0;
 };
 
+// Device words that outlive a build (h->small)
+struct SmallWords {
+  Totals tot;           // over every cloud fused into the map (totals_kernel); read back by sync_counts
+  u32 n_new;            // new voxels of the pending update (update_prepare_kernel -> merge)
+  struct {
+    int have[2];        // which halo rows arrived (xchg_halo_wait_kernel -> xchg_halo_edges_kernel)
+    u32 done_counter;   // push CTAs finished; the last one resets it
+  } x;                  // strip exchange, zeroed by gndt_xchg_create
+};
+static_assert(sizeof(Totals) == 32 && sizeof(SmallWords) == 48, "SmallWords layout");
+
 }  // namespace
 
 struct gndt_handle {
@@ -68,7 +79,7 @@ struct gndt_handle {
   const u32 *changed_dev = nullptr, *changed_count_dev = nullptr;
   size_t n_changed = 0;
   bool n_changed_valid = false;
-  Buffer small;  // Totals + n_new word, never memset by a build
+  Buffer small;  // one SmallWords, never memset by a build
   size_t cap_points = 0, cap_voxels = 0;
   // carved out of `zero`
   Ctl *ctl = nullptr;
@@ -103,8 +114,6 @@ struct gndt_handle {
   XPeers xp = {};
   void *x_opened[kMaxRanks] = {};  // cudaIpcOpenMemHandle mappings to close
   int x_what = 0;
-  int x_spare_ctas = 0;            // CTA slots the partition passes leave to the exchange (GNDT_XCHG_SPARE; measured: no gain)
-  int x_push_ctas = 48;            // grid of the push kernel (GNDT_XCHG_CTAS), 256 threads each
   cudaStream_t x_stream = nullptr; // high-priority stream of the push: it takes the first slots that free up
   cudaEvent_t x_ev[2] = {};
   // copy-engine transport (gndt_xchg_stage / gndt_xchg_send)
@@ -124,7 +133,7 @@ struct gndt_handle {
   bool timed_h2d = false;
   bool stage_timing = false;  // per-stage events (they sit between kernels and defeat the programmatic overlap there)
   bool stages_valid = false;  // the last build / update recorded them
-  uint64_t launches = 0;
+  uint64_t launches = 0;      // gndt_launch_count: launch() adds one per kernel, a build / update / remove restarts it
   uint64_t total_points = 0;  // points handed to build + updates so far (host copy)
   int sm_count = 148;
   int sort_ctas_per_sm[2] = {1, 1};  // resident CTAs of the partition pass kernels: [0] first pass, [1] later passes
@@ -167,24 +176,65 @@ int ensure_keep(gndt_handle *h, Buffer &b, size_t bytes, size_t keep, cudaStream
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-// Launch with programmatic stream serialization (PDL): the kernel's CTAs may be scheduled while
-// its predecessor in the stream drains; every such kernel starts with pdl_wait(), so no memory
-// is touched before the predecessor has completed.  GNDT_NO_PDL=1 falls back to plain launches.
-bool use_pdl() {
-  static const bool on = [] { const char *e = getenv("GNDT_NO_PDL"); return !(e && e[0] == '1'); }();
-  return on;
-}
+// Sub-allocations of one buffer, each on a 256-byte boundary: take() returns the offset, `bytes`
+// is what the buffer needs.
+struct Layout {
+  size_t bytes = 0;
+  size_t take(size_t n) { const size_t o = bytes; bytes = align_up(bytes + n, 256); return o; }
+};
+template <typename T> T *at(const Buffer &b, size_t off) { return reinterpret_cast<T *>(static_cast<char *>(b.p) + off); }
+
+// Scratch of one exclusive_scan_kernel over up to n items: ScanCtl | state | groups, zeroed together.
+struct ScanScratch {
+  size_t ctl, state, groups;
+  ScanScratch(Layout &L, size_t n) {
+    const LookbackScratch s = lookback_scratch((n + kScanTile - 1) / kScanTile);
+    ctl = L.take(sizeof(ScanCtl));
+    state = L.take(s.words * sizeof(u64));
+    groups = L.take(s.groups * sizeof(GroupState));
+  }
+};
+
+// Every kernel of this file is launched here, and counted once for gndt_launch_count.  With `pdl`
+// the launch allows programmatic stream serialization: the kernel's CTAs may be scheduled while its
+// predecessor in the stream drains.  Only kernels that start with pdl_wait() may be launched so;
+// they touch no memory before the predecessor has completed.
 template <typename... KArgs, typename... Args>
-void launch(gndt_handle *h, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args &&...args) {
+void launch(gndt_handle *h, bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+            Args &&...args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = use_pdl() ? 1 : 0;
+  cfg.numAttrs = pdl ? 1 : 0;
   cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);  // errors surface at the cudaGetLastError of the caller
   h->launches += 1;
+}
+
+// gndt_launch_count covers the map's build / update / remove and the calls on it that follow.  The
+// hoisted-division check (create, set_params) and gndt_register promise to leave it unchanged
+// (gndt.h): they hold one of these, which puts the count back when they return.
+struct KeepLaunchCount {
+  gndt_handle *h;
+  uint64_t n;
+  explicit KeepLaunchCount(gndt_handle *h_) : h(h_), n(h_->launches) {}
+  ~KeepLaunchCount() { h->launches = n; }
+};
+
+// The cloud as the kernels read it: a host cloud is copied into `stage` on `st` (`h2d0`, when given,
+// is recorded just before the copy), a device cloud is read where it is.
+int upload(gndt_handle *h, Buffer &stage, const void *xyz, size_t bytes, int mem, cudaStream_t st, cudaEvent_t h2d0,
+           const float **d_in) {
+  *d_in = static_cast<const float *>(xyz);
+  if (mem != GNDT_MEM_HOST) return GNDT_OK;
+  const int rc = ensure(h, stage, bytes);
+  if (rc != GNDT_OK) return rc;
+  if (h2d0) GNDT_CUDA(h, cudaEventRecord(h2d0, st));
+  GNDT_CUDA(h, cudaMemcpyAsync(stage.p, xyz, bytes, cudaMemcpyHostToDevice, st));
+  *d_in = static_cast<const float *>(stage.p);
+  return GNDT_OK;
 }
 
 // Largest non-negative float a with (int)ceil(a / len) <= GNDT_MAX_INDEX, by bisection over
@@ -256,9 +306,12 @@ int verify_fast_div(gndt_handle *h, float len, DivCheck &out) {
   const float top = 2.f * max_abs_offset(len);
   memcpy(&lo, &len, 4);
   memcpy(&hi, &top, 4);
-  divcheck_kernel<<<h->sm_count * 8, 256>>>(len, lo, hi, (float *)scratch, (unsigned long long *)((char *)scratch + 8));
+  KeepLaunchCount keep(h);
+  launch(h, false, divcheck_kernel, h->sm_count * 8, 256, 0, nullptr, len, lo, hi, (float *)scratch,
+         (unsigned long long *)((char *)scratch + 8));
   unsigned long long host[2] = {0, 0};
-  cudaError_t e = cudaMemcpy(host, scratch, 16, cudaMemcpyDeviceToHost);
+  cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) e = cudaMemcpy(host, scratch, 16, cudaMemcpyDeviceToHost);
   cudaFree(scratch);
   if (e != cudaSuccess) { h->err = std::string("divcheck: ") + cudaGetErrorString(e); return GNDT_ERR_CUDA; }
   memcpy(&out.rinv, &host[0], 4);
@@ -286,10 +339,8 @@ int validate_params(const gndt_params *p) {
 
 // Workspace for n points and cap_vox voxels; carves the zero-initialised region.
 // `keep_mom` bytes of the resident moments survive a regrow (streaming update).
-int reserve(gndt_handle *h, size_t n, size_t cap_vox, bool host_input, size_t stride_bytes, size_t keep_mom,
-            cudaStream_t st) {
+int reserve(gndt_handle *h, size_t n, size_t cap_vox, size_t keep_mom, cudaStream_t st) {
   int rc;
-  if (host_input && (rc = ensure(h, h->in_stage, n * stride_bytes)) != GNDT_OK) return rc;
   if ((rc = ensure(h, h->buf_a, n * sizeof(float4))) != GNDT_OK) return rc;
   if ((rc = ensure(h, h->buf_b, n * sizeof(float4))) != GNDT_OK) return rc;
   if ((rc = ensure_keep(h, h->mom, cap_vox * sizeof(VoxMoments), keep_mom, st)) != GNDT_OK) return rc;
@@ -298,46 +349,46 @@ int reserve(gndt_handle *h, size_t n, size_t cap_vox, bool host_input, size_t st
   if ((rc = ensure(h, h->columns, cap_vox * sizeof(gndt_column))) != GNDT_OK) return rc;
   if ((rc = ensure(h, h->vfirst, cap_vox * sizeof(u32))) != GNDT_OK) return rc;
   if ((rc = ensure(h, h->slope_col, cap_vox * sizeof(u32))) != GNDT_OK) return rc;
-  if ((rc = ensure(h, h->small, 256)) != GNDT_OK) return rc;
+  if ((rc = ensure(h, h->small, sizeof(SmallWords))) != GNDT_OK) return rc;
   h->cap_points = n;
   h->cap_voxels = cap_vox;
   h->sort_tiles = (n + kSortTile - 1) / kSortTile;
   h->sort_groups = (h->sort_tiles + kSortGroup - 1) / kSortGroup;
   h->red_tiles = (n + kRedTile - 1) / kRedTile;
   h->label_blocks = (cap_vox + kLabelThreads - 1) / kLabelThreads;
-  size_t off = 0;
-  auto carve = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-  const size_t o_ctl = carve(sizeof(Ctl));
-  const size_t o_hist = carve((size_t)kMaxPasses * kMaxBins * sizeof(u32));
-  const size_t o_zh = carve(kZHistBins * sizeof(u32));
-  const size_t o_rs = carve(65536 * sizeof(u32));
-  const size_t o_re = carve(65536 * sizeof(u32));
-  const size_t o_ts = carve(h->red_tiles * sizeof(u64));
-  const size_t o_tg = carve((h->red_tiles / kScanGroup + 1) * sizeof(GroupState));
-  const size_t o_ca = carve(h->red_tiles * sizeof(TileCarry));
-  const size_t o_bs = carve(h->label_blocks * sizeof(u64));
-  const size_t o_bg = carve((h->label_blocks / kScanGroup + 1) * sizeof(GroupState));
-  if ((rc = ensure(h, h->zero, off)) != GNDT_OK) return rc;
-  char *z = static_cast<char *>(h->zero.p);
-  h->ctl = reinterpret_cast<Ctl *>(z + o_ctl);
-  h->hist = reinterpret_cast<u32 *>(z + o_hist);
-  h->zhist = reinterpret_cast<u32 *>(z + o_zh);
-  h->row_start = reinterpret_cast<u32 *>(z + o_rs);
-  h->row_end = reinterpret_cast<u32 *>(z + o_re);
-  {  // look-back regions (not part of the memset region)
-    const size_t lb_bytes = align_up(h->sort_tiles * kMaxBins * sizeof(u32) + 256, 256);
-    const size_t glb_bytes = align_up(h->sort_groups * kMaxBins * sizeof(u64) + 256, 256);
-    if ((rc = ensure(h, h->lookback, 2 * (lb_bytes + glb_bytes))) != GNDT_OK) return rc;
-    char *b = static_cast<char *>(h->lookback.p);
-    h->lb[0] = reinterpret_cast<u32 *>(b); h->lb[1] = reinterpret_cast<u32 *>(b + lb_bytes);
-    h->glb[0] = reinterpret_cast<u64 *>(b + 2 * lb_bytes); h->glb[1] = reinterpret_cast<u64 *>(b + 2 * lb_bytes + glb_bytes);
+  const LookbackScratch red = lookback_scratch(h->red_tiles), fin = lookback_scratch(h->label_blocks);
+  Layout Z;
+  const size_t o_ctl = Z.take(sizeof(Ctl));
+  const size_t o_hist = Z.take((size_t)kMaxPasses * kMaxBins * sizeof(u32));
+  const size_t o_zh = Z.take(kZHistBins * sizeof(u32));
+  const size_t o_rs = Z.take(65536 * sizeof(u32));
+  const size_t o_re = Z.take(65536 * sizeof(u32));
+  const size_t o_ts = Z.take(red.words * sizeof(u64));
+  const size_t o_tg = Z.take(red.groups * sizeof(GroupState));
+  const size_t o_ca = Z.take(h->red_tiles * sizeof(TileCarry));
+  const size_t o_bs = Z.take(fin.words * sizeof(u64));
+  const size_t o_bg = Z.take(fin.groups * sizeof(GroupState));
+  if ((rc = ensure(h, h->zero, Z.bytes)) != GNDT_OK) return rc;
+  h->ctl = at<Ctl>(h->zero, o_ctl);
+  h->hist = at<u32>(h->zero, o_hist);
+  h->zhist = at<u32>(h->zero, o_zh);
+  h->row_start = at<u32>(h->zero, o_rs);
+  h->row_end = at<u32>(h->zero, o_re);
+  h->tile_state = at<u64>(h->zero, o_ts);
+  h->tile_groups = at<GroupState>(h->zero, o_tg);
+  h->carry = at<TileCarry>(h->zero, o_ca);
+  h->blk_state = at<u64>(h->zero, o_bs);
+  h->blk_groups = at<GroupState>(h->zero, o_bg);
+  h->zero_bytes_used = Z.bytes;
+  // look-back words of the partition passes (not part of the memset region)
+  Layout B;
+  const size_t lb_bytes = h->sort_tiles * kMaxBins * sizeof(u32) + 256, glb_bytes = h->sort_groups * kMaxBins * sizeof(u64) + 256;
+  const size_t o_lb[2] = {B.take(lb_bytes), B.take(lb_bytes)}, o_glb[2] = {B.take(glb_bytes), B.take(glb_bytes)};
+  if ((rc = ensure(h, h->lookback, B.bytes)) != GNDT_OK) return rc;
+  for (int k = 0; k < 2; ++k) {
+    h->lb[k] = at<u32>(h->lookback, o_lb[k]);
+    h->glb[k] = at<u64>(h->lookback, o_glb[k]);
   }
-  h->tile_state = reinterpret_cast<u64 *>(z + o_ts);
-  h->tile_groups = reinterpret_cast<GroupState *>(z + o_tg);
-  h->carry = reinterpret_cast<TileCarry *>(z + o_ca);
-  h->blk_state = reinterpret_cast<u64 *>(z + o_bs);
-  h->blk_groups = reinterpret_cast<GroupState *>(z + o_bg);
-  h->zero_bytes_used = off;
   return GNDT_OK;
 }
 
@@ -397,9 +448,9 @@ int front_end(gndt_handle *h, cudaStream_t st, const float *d_in, size_t n, size
   // K1: bounds + exact z histogram (+ zeroes the first pass's look-back words), then the key layout
   const size_t tiles = (n + kSortTile - 1) / kSortTile, groups = (tiles + kSortGroup - 1) / kSortGroup;
   auto *bounds = dp.fast_div ? bounds_kernel<true> : bounds_kernel<false>;
-  launch(h, bounds, grid_for(h, n, 256 * 4, 8), 256, 0, st, h->ctl, h->zhist, d_in, stride_f, n, start, (void *)h->lb[0],
+  launch(h, true, bounds, grid_for(h, n, 256 * 4, 8), 256, 0, st, h->ctl, h->zhist, d_in, stride_f, n, start, (void *)h->lb[0],
          tiles * kFirstMaxBins * sizeof(u32), (void *)h->glb[0], groups * kFirstMaxBins * sizeof(u64), dp);
-  launch(h, plan_kernel, 1, kZHistBins, 0, st, h->ctl, (const u32 *)h->zhist, h->hist);
+  launch(h, true, plan_kernel, 1, kZHistBins, 0, st, h->ctl, (const u32 *)h->zhist, h->hist);
   if (h->stage_timing) GNDT_CUDA(h, cudaEventRecord(h->ev[EV_KEY], st));
   // K2: partition passes (pass p writes buffer A when p is even, B when odd).  Persistent CTAs:
   // a pass beyond the planned count costs one launch of CTAs that return at once.
@@ -407,26 +458,23 @@ int front_end(gndt_handle *h, cudaStream_t st, const float *d_in, size_t n, size
   // the division mode is a template argument (two instantiations), not a run-time select
   auto *first_pass = dp.fast_div ? sort_pass_kernel<true, true> : sort_pass_kernel<true, false>;
   auto *next_pass = dp.fast_div ? sort_pass_kernel<false, true> : sort_pass_kernel<false, false>;
-  // With a strip exchange attached, a few CTA slots stay free: the persistent passes would otherwise hold every
-  // SM for 60 % of a build and the exchange of the previous build (another stream) could not run beside them.
-  const size_t spare = h->x_created ? (size_t)h->x_spare_ctas : 0;
-  const int g0 = (int)std::min<size_t>(tiles, std::max<size_t>((size_t)h->sm_count * h->sort_ctas_per_sm[0], spare + 1) - spare);
-  const int g1 = (int)std::min<size_t>(tiles, std::max<size_t>((size_t)h->sm_count * h->sort_ctas_per_sm[1], spare + 1) - spare);
-  launch(h, first_pass, g0, kSortThreads, sizeof(SortSmem), st, h->ctl, 0, d_in, stride_f, n, start, (const float4 *)nullptr, A,
+  const int g0 = (int)std::min<size_t>(tiles, (size_t)h->sm_count * h->sort_ctas_per_sm[0]);
+  const int g1 = (int)std::min<size_t>(tiles, (size_t)h->sm_count * h->sort_ctas_per_sm[1]);
+  launch(h, true, first_pass, g0, kSortThreads, sizeof(SortSmem), st, h->ctl, 0, d_in, stride_f, n, start, (const float4 *)nullptr, A,
          h->lb[0], h->glb[0], h->lb[1], h->glb[1], h->hist, dp);
   for (int p = 1; p < kMaxPasses; ++p) {
     const float4 *src = (p & 1) ? A : B;
     float4 *dst = (p & 1) ? B : A;
-    launch(h, next_pass, g1, kSortThreads, sizeof(SortSmem), st, h->ctl, p, (const float *)nullptr, (size_t)4, n, (size_t)0, src, dst,
+    launch(h, true, next_pass, g1, kSortThreads, sizeof(SortSmem), st, h->ctl, p, (const float *)nullptr, (size_t)4, n, (size_t)0, src, dst,
            h->lb[p & 1], h->glb[p & 1], h->lb[(p + 1) & 1], h->glb[(p + 1) & 1], h->hist, dp);
   }
   if (h->stage_timing) GNDT_CUDA(h, cudaEventRecord(h->ev[EV_SORT], st));
   // K3: per-voxel moments
   const int rtiles = (int)((n + kRedTile - 1) / kRedTile);
   auto *reduce = dp.fast_div ? reduce_kernel<true> : reduce_kernel<false>;
-  launch(h, reduce, rtiles, kRedThreads, sizeof(RedSmem), st, h->ctl, (const float4 *)A, (const float4 *)B, out, h->carry,
+  launch(h, true, reduce, rtiles, kRedThreads, sizeof(RedSmem), st, h->ctl, (const float4 *)A, (const float4 *)B, out, h->carry,
          h->tile_state, h->tile_groups, dp);
-  launch(h, fixup_kernel, grid_for(h, (size_t)rtiles * 32, 128, 16), 128, 0, st, h->ctl, out, (const TileCarry *)h->carry);
+  launch(h, true, fixup_kernel, grid_for(h, (size_t)rtiles * 32, 128, 16), 128, 0, st, h->ctl, out, (const TileCarry *)h->carry);
   if (h->stage_timing) GNDT_CUDA(h, cudaEventRecord(h->ev[EV_REDUCE], st));
   return GNDT_OK;
 }
@@ -444,14 +492,14 @@ __global__ void table_bounds_kernel(Ctl *ctl, const gndt_voxel *table, u32 n_fix
 // sorted raw moments -> voxel / slope / column tables + reachability bits
 int back_end(gndt_handle *h, cudaStream_t st, const DevParams &dp, const VoxMoments *mom, bool bounds_from_table) {
   const int g_lab = grid_for(h, h->cap_voxels, kLabelThreads, 8);
-  launch(h, finalize_label_kernel, g_lab, kFinThreads, sizeof(FinSmem), st, h->ctl, mom, (gndt_voxel *)h->table.p,
+  launch(h, true, finalize_label_kernel, g_lab, kFinThreads, sizeof(FinSmem), st, h->ctl, mom, (gndt_voxel *)h->table.p,
          (gndt_slope *)h->slopes.p, (gndt_column *)h->columns.p, (u32 *)h->vfirst.p, (u32 *)h->slope_col.p, h->blk_state, h->blk_groups,
          &h->ctl->ticket[7], dp);
-  if (bounds_from_table) launch(h, table_bounds_kernel, 1, 32, 0, st, h->ctl, (const gndt_voxel *)h->table.p, 0u);
-  launch(h, column_finish_kernel, g_lab, 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p, (const u32 *)h->vfirst.p, 0u,
+  if (bounds_from_table) launch(h, true, table_bounds_kernel, 1, 32, 0, st, h->ctl, (const gndt_voxel *)h->table.p, 0u);
+  launch(h, true, column_finish_kernel, g_lab, 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p, (const u32 *)h->vfirst.p, 0u,
          (gndt_column *)h->columns.p, h->row_start, h->row_end, 0, 0);
   if (h->stage_timing) GNDT_CUDA(h, cudaEventRecord(h->ev[EV_LABEL], st));
-  launch(h, edges_kernel, g_lab, 256, 0, st, h->ctl, (gndt_voxel *)h->table.p, (gndt_slope *)h->slopes.p,
+  launch(h, true, edges_kernel, g_lab, 256, 0, st, h->ctl, (gndt_voxel *)h->table.p, (gndt_slope *)h->slopes.p,
          (const gndt_column *)h->columns.p, (const u32 *)h->slope_col.p, (const u32 *)h->row_start, (const u32 *)h->row_end, 0, 0, 0, dp);
   GNDT_CUDA(h, cudaEventRecord(h->ev[EV_EDGES], st));
   return GNDT_OK;
@@ -516,7 +564,6 @@ int gndt_create(const gndt_params *params, int device, gndt_handle **out) {
                : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, sort_pass_kernel<false, true>, kSortThreads, sizeof(SortSmem));
     if (e != cudaSuccess || nb < 1) { g_create_error = "partition pass kernel does not fit on this device"; delete h; return GNDT_ERR_CUDA; }
     h->sort_ctas_per_sm[k] = nb;
-    if (const char *w = getenv("GNDT_SORT_WAVES")) h->sort_ctas_per_sm[k] = nb * std::max(1, atoi(w));  // tuning: > 1 = more, shorter-lived CTAs
   }
   int rc = verify_fast_div(h, h->params.grid_len, h->div[0]);
   if (rc == GNDT_OK) rc = verify_fast_div(h, h->params.z_len, h->div[1]);
@@ -563,7 +610,7 @@ static int build_device(gndt_handle *h, const float *d_in, size_t n, size_t stri
   GNDT_CUDA(h, cudaEventRecord(h->ev[EV_START], st));
   int rc = front_end(h, st, d_in, n, stride_bytes / 4, start, dp, (VoxMoments *)h->mom.p);
   if (rc != GNDT_OK) return rc;
-  launch(h, totals_kernel, 1, 32, 0, st, (Totals *)h->small.p, (const Ctl *)h->ctl, (u64)n, 1, 1);
+  launch(h, true, totals_kernel, 1, 32, 0, st, &static_cast<SmallWords *>(h->small.p)->tot, (const Ctl *)h->ctl, (u64)n, 1, 1);
   rc = back_end(h, st, dp, (const VoxMoments *)h->mom.p, false);
   if (rc != GNDT_OK) return rc;
   GNDT_CUDA(h, cudaGetLastError());
@@ -577,27 +624,26 @@ static int build_device(gndt_handle *h, const float *d_in, size_t n, size_t stri
   return GNDT_OK;
 }
 
-int gndt_build(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, void *stream) {
-  if (!h) return GNDT_ERR_INVALID_ARG;
-  int rc = check_cloud_args(h, xyz, n, stride_bytes, mem, "gndt_build");
-  if (rc != GNDT_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+// what a build does before its cloud is on the device: no map until it completes, the launch count
+// restarts, the workspace fits n points
+static int begin_build(gndt_handle *h, size_t n, cudaStream_t st) {
   GNDT_CUDA(h, cudaSetDevice(h->device));
   h->built = false;
   h->counts_valid = false;
   h->launches = 0;
   const size_t cap_vox = h->params.max_voxels ? (size_t)h->params.max_voxels : n;
-  rc = reserve(h, n, cap_vox, mem == GNDT_MEM_HOST, stride_bytes, 0, st);
-  if (rc != GNDT_OK) return rc;
+  return reserve(h, n, cap_vox, 0, st);
+}
 
-  const float *d_in = static_cast<const float *>(xyz);
-  h->timed_h2d = false;
-  if (mem == GNDT_MEM_HOST) {
-    GNDT_CUDA(h, cudaEventRecord(h->ev[EV_H2D0], st));
-    GNDT_CUDA(h, cudaMemcpyAsync(h->in_stage.p, xyz, n * stride_bytes, cudaMemcpyHostToDevice, st));
-    d_in = static_cast<const float *>(h->in_stage.p);
-    h->timed_h2d = true;
-  }
+int gndt_build(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, void *stream) {
+  if (!h) return GNDT_ERR_INVALID_ARG;
+  int rc = check_cloud_args(h, xyz, n, stride_bytes, mem, "gndt_build");
+  if (rc != GNDT_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((rc = begin_build(h, n, st)) != GNDT_OK) return rc;
+  const float *d_in;
+  h->timed_h2d = mem == GNDT_MEM_HOST;
+  if ((rc = upload(h, h->in_stage, xyz, n * stride_bytes, mem, st, h->ev[EV_H2D0], &d_in)) != GNDT_OK) return rc;
   return build_device(h, d_in, n, stride_bytes, st);
 }
 
@@ -658,12 +704,8 @@ int gndt_build_msg(gndt_handle *h, const gndt_pointcloud2 *msg, void *stream) {
   }
   if (n > GNDT_MAX_POINTS) { h->err = "gndt_build_msg: width * height exceeds GNDT_MAX_POINTS"; return GNDT_ERR_CAPACITY; }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  GNDT_CUDA(h, cudaSetDevice(h->device));
-  h->built = false;
-  h->counts_valid = false;
-  h->launches = 0;
-  const size_t cap_vox = h->params.max_voxels ? (size_t)h->params.max_voxels : n;
-  int rc = reserve(h, n, cap_vox, true, ps, 0, st);
+  int rc = begin_build(h, n, st);
+  if (rc == GNDT_OK) rc = ensure(h, h->in_stage, n * ps);
   if (rc != GNDT_OK) return rc;
   GNDT_CUDA(h, cudaEventRecord(h->ev[EV_H2D0], st));
   if (msg->host_pinned) GNDT_CUDA(h, cudaMemcpyAsync(h->in_stage.p, msg->data, n * ps, cudaMemcpyHostToDevice, st));
@@ -674,9 +716,8 @@ int gndt_build_msg(gndt_handle *h, const gndt_pointcloud2 *msg, void *stream) {
                       msg->z_offset == msg->x_offset + 8;
   if (direct) return build_device(h, reinterpret_cast<const float *>(static_cast<const char *>(h->in_stage.p) + msg->x_offset), n, ps, st);
   if ((rc = ensure(h, h->msg_points, n * sizeof(float4))) != GNDT_OK) return rc;
-  ingest_kernel<<<grid_for(h, n, 256, 8), 256, 0, st>>>(static_cast<const unsigned char *>(h->in_stage.p), n, ps, msg->x_offset, msg->y_offset,
-                                                        msg->z_offset, msg->is_bigendian ? 1 : 0, static_cast<float4 *>(h->msg_points.p));
-  h->launches += 1;
+  launch(h, false, ingest_kernel, grid_for(h, n, 256, 8), 256, 0, st, static_cast<const unsigned char *>(h->in_stage.p), n, ps,
+         msg->x_offset, msg->y_offset, msg->z_offset, msg->is_bigendian ? 1 : 0, static_cast<float4 *>(h->msg_points.p));
   return build_device(h, static_cast<const float *>(h->msg_points.p), n, sizeof(float4), st);
 }
 
@@ -711,38 +752,34 @@ static int fuse_scan(gndt_handle *h, const void *xyz, size_t n, size_t stride_by
   size_t cap_vox = h->cap_voxels;
   const size_t need = (size_t)n_res + (sign > 0 ? n : 0);
   if (h->params.max_voxels == 0 && need > cap_vox) cap_vox = need + need / 2;
-  rc = reserve(h, n > h->cap_points ? n : h->cap_points, cap_vox, mem == GNDT_MEM_HOST, stride_bytes,
-               (size_t)n_res * sizeof(VoxMoments), st);
+  rc = reserve(h, n > h->cap_points ? n : h->cap_points, cap_vox, (size_t)n_res * sizeof(VoxMoments), st);
   if (rc != GNDT_OK) return rc;
   if ((rc = ensure(h, h->mom_alt, cap_vox * sizeof(VoxMoments))) != GNDT_OK) return rc;
   if ((rc = ensure(h, h->mom_scan, n * sizeof(VoxMoments))) != GNDT_OK) return rc;
   // scratch: per scan voxel / point (n + 1 words each): is_new, new_pos, order, valid, order_pos, changed; keys (u64)
   //          per resident / merged voxel (cap_vox + 1 words each): inv, dead, dead_pos, touch_first
-  //          scan state for the largest of the two
-  const size_t wn = align_up((n + 1) * 4, 256), wv = align_up((cap_vox + 1) * 4, 256);
-  const size_t scan_tiles = (std::max(n, cap_vox) + kScanTile - 1) / kScanTile + 1;
-  const size_t w_state = align_up(scan_tiles * sizeof(u64), 256), w_groups = align_up((scan_tiles / kScanGroup + 2) * sizeof(GroupState), 256);
-  const size_t w_scan = 256 + w_state + w_groups;  // ScanCtl | state | groups: one per scan launched (3)
-  if ((rc = ensure(h, h->upd_work, 6 * wn + align_up(n * 8, 256) + 4 * wv + 3 * w_scan)) != GNDT_OK) return rc;
-  char *w = static_cast<char *>(h->upd_work.p);
-  u32 *is_new = (u32 *)w, *new_pos = (u32 *)(w + wn), *order = (u32 *)(w + 2 * wn), *valid = (u32 *)(w + 3 * wn),
-      *order_pos = (u32 *)(w + 4 * wn), *changed = (u32 *)(w + 5 * wn);
-  u64 *new_keys = (u64 *)(w + 6 * wn);
-  char *wv0 = w + 6 * wn + align_up(n * 8, 256);
-  u32 *inv = (u32 *)wv0, *dead = (u32 *)(wv0 + wv), *dead_pos = (u32 *)(wv0 + 2 * wv), *touch_first = (u32 *)(wv0 + 3 * wv);
-  char *ws = wv0 + 4 * wv;
-  auto scan_ctl = [&](int k) { return reinterpret_cast<ScanCtl *>(ws + k * w_scan); };
-  auto scan_state = [&](int k) { return reinterpret_cast<u64 *>(ws + k * w_scan + 256); };
-  auto scan_groups = [&](int k) { return reinterpret_cast<GroupState *>(ws + k * w_scan + 256 + w_state); };
+  //          one per exclusive scan launched (3), each sized for the larger of the two
+  Layout W;
+  const size_t wn = (n + 1) * 4, wv = (cap_vox + 1) * 4;
+  const size_t o_is_new = W.take(wn), o_new_pos = W.take(wn), o_order = W.take(wn), o_valid = W.take(wn), o_order_pos = W.take(wn),
+               o_changed = W.take(wn), o_new_keys = W.take(n * 8);
+  const size_t o_inv = W.take(wv), o_dead = W.take(wv), o_dead_pos = W.take(wv), o_touch_first = W.take(wv);
+  const size_t scan_items = std::max(n, cap_vox);
+  const ScanScratch sc[3] = {ScanScratch(W, scan_items), ScanScratch(W, scan_items), ScanScratch(W, scan_items)};
+  if ((rc = ensure(h, h->upd_work, W.bytes)) != GNDT_OK) return rc;
+  const Buffer &w = h->upd_work;
+  u32 *is_new = at<u32>(w, o_is_new), *new_pos = at<u32>(w, o_new_pos), *order = at<u32>(w, o_order), *valid = at<u32>(w, o_valid),
+      *order_pos = at<u32>(w, o_order_pos), *changed = at<u32>(w, o_changed);
+  u64 *new_keys = at<u64>(w, o_new_keys);
+  u32 *inv = at<u32>(w, o_inv), *dead = at<u32>(w, o_dead), *dead_pos = at<u32>(w, o_dead_pos), *touch_first = at<u32>(w, o_touch_first);
+  auto exclusive_scan = [&](int k, const u32 *in, u32 n_fixed, const u32 *n_dev, u32 *out, size_t items) {
+    launch(h, false, exclusive_scan_kernel, grid_for(h, (items + kScanTile - 1) / kScanTile, 1, 4), 256, 0, st, at<ScanCtl>(w, sc[k].ctl),
+           in, n_fixed, n_dev, out, at<u64>(w, sc[k].state), at<GroupState>(w, sc[k].groups));
+  };
 
-  const float *d_in = static_cast<const float *>(xyz);
-  h->timed_h2d = false;
-  if (mem == GNDT_MEM_HOST) {
-    GNDT_CUDA(h, cudaEventRecord(h->ev[EV_H2D0], st));
-    GNDT_CUDA(h, cudaMemcpyAsync(h->in_stage.p, xyz, n * stride_bytes, cudaMemcpyHostToDevice, st));
-    d_in = static_cast<const float *>(h->in_stage.p);
-    h->timed_h2d = true;
-  }
+  const float *d_in;
+  h->timed_h2d = mem == GNDT_MEM_HOST;
+  if ((rc = upload(h, h->in_stage, xyz, n * stride_bytes, mem, st, h->ev[EV_H2D0], &d_in)) != GNDT_OK) return rc;
   gndt_params p = h->params;  // every point of the scan is binned against the resident origin
   p.origin_is_first_point = 0;
   p.origin[0] = origin[0]; p.origin[1] = origin[1]; p.origin[2] = origin[2];
@@ -753,35 +790,33 @@ static int fuse_scan(gndt_handle *h, const void *xyz, size_t n, size_t stride_by
   VoxMoments *res = (VoxMoments *)h->mom.p, *scan = (VoxMoments *)h->mom_scan.p, *merged = (VoxMoments *)h->mom_alt.p;
   rc = front_end(h, st, d_in, n, stride_bytes / 4, 0, dp, scan);
   if (rc != GNDT_OK) return rc;
-  totals_kernel<<<1, 32, 0, st>>>((Totals *)h->small.p, h->ctl, (u64)n, 0, sign);
-  u32 *n_new = reinterpret_cast<u32 *>(static_cast<char *>(h->small.p) + 128);
+  SmallWords *small = static_cast<SmallWords *>(h->small.p);
+  launch(h, false, totals_kernel, 1, 32, 0, st, &small->tot, h->ctl, (u64)n, 0, sign);
   const int g_scan = grid_for(h, n, 256, 8), g_res = grid_for(h, std::max<size_t>(n_res, 1), 256, 8);
-  // zero: is_new .. valid (4 arrays), dead / dead_pos, scan states; 0xFF: inv, touch_first
-  GNDT_CUDA(h, cudaMemsetAsync(is_new, 0, 4 * wn, st));
-  GNDT_CUDA(h, cudaMemsetAsync(dead, 0, 2 * wv, st));
-  GNDT_CUDA(h, cudaMemsetAsync(ws, 0, 3 * w_scan, st));
+  // zero: is_new .. valid (4 arrays), dead / dead_pos, scan scratch; 0xFF: inv, touch_first
+  GNDT_CUDA(h, cudaMemsetAsync(is_new, 0, o_order_pos - o_is_new, st));
+  GNDT_CUDA(h, cudaMemsetAsync(dead, 0, o_touch_first - o_dead, st));
+  GNDT_CUDA(h, cudaMemsetAsync(at<char>(w, sc[0].ctl), 0, W.bytes - sc[0].ctl, st));
   GNDT_CUDA(h, cudaMemsetAsync(inv, 0xFF, wv, st));
   GNDT_CUDA(h, cudaMemsetAsync(touch_first, 0xFF, wv, st));
-  update_match_kernel<<<g_scan, 256, 0, st>>>(h->ctl, res, n_res, scan, sign, inv, is_new, dead);
-  const int g_tiles_n = grid_for(h, (n + kScanTile - 1) / kScanTile, 1, 4), g_tiles_v = grid_for(h, ((size_t)n_res + kScanTile - 1) / kScanTile, 1, 4);
-  exclusive_scan_kernel<<<g_tiles_n, 256, 0, st>>>(scan_ctl(0), is_new, 0u, &h->ctl->n_voxels, new_pos, scan_state(0), scan_groups(0));
-  if (sign < 0) exclusive_scan_kernel<<<g_tiles_v, 256, 0, st>>>(scan_ctl(1), dead, n_res, nullptr, dead_pos, scan_state(1), scan_groups(1));
-  update_new_keys_kernel<<<g_scan, 256, 0, st>>>(h->ctl, scan, is_new, new_pos, new_keys);
-  update_prepare_kernel<<<1, 32, 0, st>>>(h->ctl, n_res, new_pos, sign < 0 ? dead_pos : nullptr, (u32)cap_vox, n_new);
-  update_merge_resident_kernel<<<g_res, 256, 0, st>>>(h->ctl, res, n_res, scan, sign, inv, new_keys, n_new, dead, dead_pos, merged);
-  if (sign > 0) update_merge_new_kernel<<<g_scan, 256, 0, st>>>(h->ctl, res, n_res, scan, is_new, new_pos, merged);
-  h->launches += 6 + (sign < 0 ? 1 : 1);
+  launch(h, false, update_match_kernel, g_scan, 256, 0, st, h->ctl, res, n_res, scan, sign, inv, is_new, dead);
+  exclusive_scan(0, is_new, 0u, &h->ctl->n_voxels, new_pos, n);
+  if (sign < 0) exclusive_scan(1, dead, n_res, nullptr, dead_pos, n_res);
+  launch(h, false, update_new_keys_kernel, g_scan, 256, 0, st, h->ctl, scan, is_new, new_pos, new_keys);
+  launch(h, false, update_prepare_kernel, 1, 32, 0, st, h->ctl, n_res, new_pos, sign < 0 ? dead_pos : nullptr, (u32)cap_vox, &small->n_new);
+  launch(h, false, update_merge_resident_kernel, g_res, 256, 0, st, h->ctl, res, n_res, scan, sign, inv, new_keys, &small->n_new, dead,
+         dead_pos, merged);
+  if (sign > 0) launch(h, false, update_merge_new_kernel, g_scan, 256, 0, st, h->ctl, res, n_res, scan, is_new, new_pos, merged);
   rc = back_end(h, st, dp, merged, true);
   if (rc != GNDT_OK) return rc;
   // the cells this scan touched, in first-touched order (changeMorton_list)
-  changed_mark_kernel<<<g_scan, 256, 0, st>>>(h->ctl, scan, (const gndt_column *)h->columns.p, touch_first);
-  changed_order_kernel<<<grid_for(h, cap_vox, 256, 8), 256, 0, st>>>(h->ctl, touch_first, dp.idx_offset, (u32)n, order, valid);
-  exclusive_scan_kernel<<<g_tiles_n, 256, 0, st>>>(scan_ctl(2), valid, (u32)n, nullptr, order_pos, scan_state(2), scan_groups(2));
-  changed_compact_kernel<<<g_scan, 256, 0, st>>>(order, valid, order_pos, (u32)n, changed);
-  h->launches += 4;
+  launch(h, false, changed_mark_kernel, g_scan, 256, 0, st, h->ctl, scan, (const gndt_column *)h->columns.p, touch_first);
+  launch(h, false, changed_order_kernel, grid_for(h, cap_vox, 256, 8), 256, 0, st, h->ctl, touch_first, dp.idx_offset, (u32)n, order, valid);
+  exclusive_scan(2, valid, (u32)n, nullptr, order_pos, n);
+  launch(h, false, changed_compact_kernel, g_scan, 256, 0, st, order, valid, order_pos, (u32)n, changed);
   GNDT_CUDA(h, cudaGetLastError());
   h->changed_dev = changed;
-  h->changed_count_dev = &scan_ctl(2)->total;
+  h->changed_count_dev = &at<ScanCtl>(w, sc[2].ctl)->total;
   h->pending_fuse = sign;         // resolved by the next sync_counts: swap the moment tables, or roll back
   h->pending_points = n;
   h->stages_valid = h->stage_timing;
@@ -872,9 +907,8 @@ int gndt_halo_pack(gndt_handle *h, gndt_voxel *first_row_out, gndt_voxel *last_r
   if (!h->built) { h->err = "no map has been built on this handle"; return GNDT_ERR_STATE; }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   GNDT_CUDA(h, cudaSetDevice(h->device));
-  halo_pack_kernel<<<2, 256, 0, st>>>(h->ctl, (const gndt_voxel *)h->table.p, (const gndt_column *)h->columns.p, h->row_start,
-                                      h->row_end, first_row_out, last_row_out, (u32)cap_records);
-  h->launches += 1;
+  launch(h, false, halo_pack_kernel, 2, 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p, (const gndt_column *)h->columns.p,
+         h->row_start, h->row_end, first_row_out, last_row_out, (u32)cap_records);
   GNDT_CUDA(h, cudaGetLastError());
   return GNDT_OK;
 }
@@ -885,9 +919,8 @@ int gndt_halo_edges(gndt_handle *h, const gndt_voxel *from_prev, const gndt_voxe
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   GNDT_CUDA(h, cudaSetDevice(h->device));
   const DevParams dp = make_dev(h, h->params, h->cap_voxels);
-  halo_edges_kernel<<<grid_for(h, h->cap_voxels, 256, 8), 256, 0, st>>>(h->ctl, (gndt_voxel *)h->table.p, (gndt_slope *)h->slopes.p,
-                                                                        from_prev, from_next, dp);
-  h->launches += 1;
+  launch(h, false, halo_edges_kernel, grid_for(h, h->cap_voxels, 256, 8), 256, 0, st, h->ctl, (gndt_voxel *)h->table.p,
+         (gndt_slope *)h->slopes.p, from_prev, from_next, dp);
   h->counts_valid = false;
   GNDT_CUDA(h, cudaGetLastError());
   return GNDT_OK;
@@ -901,8 +934,7 @@ int gndt_apply_strip_offsets(gndt_handle *h, gndt_voxel *table, const uint64_t *
   for (int r = 0; r < n_strips; ++r) {
     const uint64_t cnt = offsets[r + 1] - offsets[r];
     if (!cnt || (col_offsets[r] == 0 && slope_offsets[r] == 0)) continue;
-    strip_offsets_kernel<<<grid_for(h, cnt, 256, 8), 256, 0, st>>>(table, offsets[r], cnt, col_offsets[r], slope_offsets[r]);
-    h->launches += 1;
+    launch(h, false, strip_offsets_kernel, grid_for(h, cnt, 256, 8), 256, 0, st, table, offsets[r], cnt, col_offsets[r], slope_offsets[r]);
   }
   GNDT_CUDA(h, cudaGetLastError());
   return GNDT_OK;
@@ -950,40 +982,37 @@ int gndt_build_edges(gndt_handle *h, const gndt_slope *slopes, size_t n_slopes, 
   }
   const int n_rows = cx_hi - cx_lo + 1;
   const u32 S = (u32)n_slopes, C = (u32)n_columns;
-  const size_t n_tiles = (n_slopes + kScanTile - 1) / kScanTile;
-  // work buffer: ctl | rows start/end | scan state | scan groups | slope_col | deg
-  size_t off = 0;
-  auto carve = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-  const size_t o_ctl = carve(sizeof(ScanCtl)), o_rs = carve((size_t)n_rows * 4), o_re = carve((size_t)n_rows * 4),
-               o_st = carve((n_tiles + 1) * sizeof(u64)), o_gr = carve((n_tiles / kScanGroup + 1) * sizeof(GroupState));
-  const size_t zero_bytes = off;
-  const size_t o_sc = carve((n_slopes + 1) * 4), o_dg = carve((n_slopes + 1) * 4);
-  if ((rc = ensure(h, h->g_work, off)) != GNDT_OK) return rc;
+  // work buffer: scan scratch | rows start/end (zeroed) | slope_col | deg
+  Layout W;
+  const ScanScratch sc(W, n_slopes);
+  const size_t o_rs = W.take((size_t)n_rows * 4), o_re = W.take((size_t)n_rows * 4);
+  const size_t zero_bytes = W.bytes;
+  const size_t o_sc = W.take((n_slopes + 1) * 4), o_dg = W.take((n_slopes + 1) * 4);
+  if ((rc = ensure(h, h->g_work, W.bytes)) != GNDT_OK) return rc;
   if ((rc = ensure(h, h->g_off, (n_slopes + 1) * 4)) != GNDT_OK) return rc;
-  char *w = static_cast<char *>(h->g_work.p);
-  ScanCtl *g = reinterpret_cast<ScanCtl *>(w + o_ctl);
-  u32 *rs = reinterpret_cast<u32 *>(w + o_rs), *re = reinterpret_cast<u32 *>(w + o_re);
-  u32 *slope_col = reinterpret_cast<u32 *>(w + o_sc), *deg = reinterpret_cast<u32 *>(w + o_dg);
-  GNDT_CUDA(h, cudaMemsetAsync(w, 0, zero_bytes, st));
+  const Buffer &w = h->g_work;
+  ScanCtl *g = at<ScanCtl>(w, sc.ctl);
+  u32 *rs = at<u32>(w, o_rs), *re = at<u32>(w, o_re), *slope_col = at<u32>(w, o_sc), *deg = at<u32>(w, o_dg);
+  GNDT_CUDA(h, cudaMemsetAsync(w.p, 0, zero_bytes, st));
   GNDT_CUDA(h, cudaMemsetAsync(h->g_off.p, 0, (n_slopes + 1) * 4, st));
   h->g_slopes = n_slopes;
   h->g_targets = 0;
   if (S && C) {
     const DevParams dp = make_dev(h, h->params, 0);
     const int grid_c = grid_for(h, C, 256, 8), grid_s = grid_for(h, S, 256, 8);
-    graph_prepare_kernel<<<grid_c, 256, 0, st>>>(columns, C, cx_lo, slope_col, rs, re);
-    graph_edges_kernel<false><<<grid_s, 256, 0, st>>>(slopes, S, columns, C, slope_col, rs, re, cx_lo, n_rows, deg, nullptr, nullptr, dp);
-    exclusive_scan_kernel<<<grid_for(h, n_tiles, 1, 4), 256, 0, st>>>(g, deg, S, nullptr, (u32 *)h->g_off.p,
-                                                                      reinterpret_cast<u64 *>(w + o_st), reinterpret_cast<GroupState *>(w + o_gr));
+    launch(h, false, graph_prepare_kernel, grid_c, 256, 0, st, columns, C, cx_lo, slope_col, rs, re);
+    launch(h, false, graph_edges_kernel<false>, grid_s, 256, 0, st, slopes, S, columns, C, slope_col, rs, re, cx_lo, n_rows, deg, nullptr,
+           nullptr, dp);
+    launch(h, false, exclusive_scan_kernel, grid_for(h, (n_slopes + kScanTile - 1) / kScanTile, 1, 4), 256, 0, st, g, deg, S, nullptr,
+           (u32 *)h->g_off.p, at<u64>(w, sc.state), at<GroupState>(w, sc.groups));
     ScanCtl hg;
     GNDT_CUDA(h, cudaMemcpyAsync(&hg, g, sizeof(hg), cudaMemcpyDeviceToHost, st));
     GNDT_CUDA(h, cudaStreamSynchronize(st));
     if (hg.err) { h->err = "graph scan watchdog"; return GNDT_ERR_INTERNAL; }
     h->g_targets = hg.total;
     if ((rc = ensure(h, h->g_tgt, std::max<size_t>(hg.total, 1) * 4)) != GNDT_OK) return rc;
-    graph_edges_kernel<true><<<grid_s, 256, 0, st>>>(slopes, S, columns, C, slope_col, rs, re, cx_lo, n_rows, nullptr,
-                                                     (const u32 *)h->g_off.p, (u32 *)h->g_tgt.p, dp);
-    h->launches += 4;
+    launch(h, false, graph_edges_kernel<true>, grid_s, 256, 0, st, slopes, S, columns, C, slope_col, rs, re, cx_lo, n_rows, nullptr,
+           (const u32 *)h->g_off.p, (u32 *)h->g_tgt.p, dp);
     GNDT_CUDA(h, cudaStreamSynchronize(st));
   }
   GNDT_CUDA(h, cudaGetLastError());
@@ -1012,6 +1041,7 @@ int gndt_copy_edges(gndt_handle *h, uint32_t *offsets, size_t cap_offsets, uint3
 // ---- peer-mapped strip exchange --------------------------------------------------------
 static_assert(sizeof(gndt_xchg_info) == 128, "gndt_xchg_info is 128 bytes");
 static_assert(sizeof(cudaIpcMemHandle_t) == 64, "ipc handle size");
+constexpr int kPushCtas = 48;  // grid of xchg_push_kernel
 
 int gndt_xchg_create(gndt_handle *h, int rank, int world, size_t cap_records, size_t cap_halo_records, int what,
                      gndt_xchg_info *mine) {
@@ -1021,22 +1051,21 @@ int gndt_xchg_create(gndt_handle *h, int rank, int world, size_t cap_records, si
   if (cap_records > 0xFFFFFFFEull) return GNDT_ERR_CAPACITY;
   GNDT_CUDA(h, cudaSetDevice(h->device));
   XLayout L = {};
-  size_t off = 0;
-  auto carve = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
-  L.mail = carve(sizeof(XMail));
-  L.halo[0] = carve((cap_halo_records + 1) * sizeof(gndt_voxel));
-  L.halo[1] = carve((cap_halo_records + 1) * sizeof(gndt_voxel));
-  L.voxels = carve((what & GNDT_X_VOXELS) ? cap_records * sizeof(gndt_voxel) : 0);
-  L.slopes = carve((what & GNDT_X_SLOPES) ? cap_records * sizeof(gndt_slope) : 0);
-  L.columns = carve((what & GNDT_X_COLUMNS) ? cap_records * sizeof(gndt_column) : 0);
-  L.total = off;
+  Layout B;
+  L.mail = B.take(sizeof(XMail));
+  L.halo[0] = B.take((cap_halo_records + 1) * sizeof(gndt_voxel));
+  L.halo[1] = B.take((cap_halo_records + 1) * sizeof(gndt_voxel));
+  L.voxels = B.take((what & GNDT_X_VOXELS) ? cap_records * sizeof(gndt_voxel) : 0);
+  L.slopes = B.take((what & GNDT_X_SLOPES) ? cap_records * sizeof(gndt_slope) : 0);
+  L.columns = B.take((what & GNDT_X_COLUMNS) ? cap_records * sizeof(gndt_column) : 0);
+  L.total = B.bytes;
   L.cap_records = cap_records;
   L.cap_halo = cap_halo_records;
   int rc;
   if ((rc = ensure(h, h->xbuf, L.total)) != GNDT_OK) return rc;
-  if ((rc = ensure(h, h->small, 256)) != GNDT_OK) return rc;
+  if ((rc = ensure(h, h->small, sizeof(SmallWords))) != GNDT_OK) return rc;
   GNDT_CUDA(h, cudaMemset(h->xbuf.p, 0, sizeof(XMail)));
-  GNDT_CUDA(h, cudaMemset(static_cast<char *>(h->small.p) + 160, 0, 64));
+  GNDT_CUDA(h, cudaMemset(&static_cast<SmallWords *>(h->small.p)->x, 0, sizeof(SmallWords::x)));
   h->xl = L;
   h->xp = XPeers{};
   h->xp.rank = rank;
@@ -1045,8 +1074,6 @@ int gndt_xchg_create(gndt_handle *h, int rank, int world, size_t cap_records, si
   h->x_epoch = 0;
   h->x_created = true;
   h->x_connected = false;
-  if (const char *e = getenv("GNDT_XCHG_SPARE")) h->x_spare_ctas = std::max(0, atoi(e));
-  if (const char *e = getenv("GNDT_XCHG_CTAS")) h->x_push_ctas = std::max(1, atoi(e));
   if (!h->x_stream) {
     int lo_p = 0, hi_p = 0;
     GNDT_CUDA(h, cudaDeviceGetStreamPriorityRange(&lo_p, &hi_p));
@@ -1108,23 +1135,19 @@ int gndt_xchg_connect(gndt_handle *h, const gndt_xchg_info *all, int world) {
 }
 
 // publish -> halo rows -> boundary reach bits (everything of an exchange that needs no bulk transfer)
-static int xchg_front(gndt_handle *h, cudaStream_t st, u32 epoch, bool halo) {
+static void xchg_front(gndt_handle *h, cudaStream_t st, u32 epoch) {
   const XPeers &X = h->xp;
   const XLayout &L = h->xl;
-  int *have = reinterpret_cast<int *>(static_cast<char *>(h->small.p) + 160);
+  int *have = static_cast<SmallWords *>(h->small.p)->x.have;
   const DevParams dp = make_dev(h, h->params, h->cap_voxels);
   unsigned char *mine = X.buf[X.rank];
-  xchg_publish_kernel<<<1, 32, 0, st>>>(h->ctl, X, L, epoch);
-  h->launches += 1;
-  if (!halo) return GNDT_OK;
-  xchg_halo_send_kernel<<<2, 256, 0, st>>>(h->ctl, (const gndt_voxel *)h->table.p, (const gndt_column *)h->columns.p, h->row_start,
-                                           h->row_end, X, L, epoch);
-  xchg_halo_wait_kernel<<<1, 32, 0, st>>>(h->ctl, X, L, epoch, have);
-  xchg_halo_edges_kernel<<<grid_for(h, h->cap_voxels, 256, 4), 256, 0, st>>>(
-      h->ctl, (gndt_voxel *)h->table.p, (gndt_slope *)h->slopes.p, reinterpret_cast<const gndt_voxel *>(mine + L.halo[0]),
-      reinterpret_cast<const gndt_voxel *>(mine + L.halo[1]), have, dp);
-  h->launches += 3;
-  return GNDT_OK;
+  launch(h, false, xchg_publish_kernel, 1, 32, 0, st, h->ctl, X, L, epoch);
+  launch(h, false, xchg_halo_send_kernel, 2, 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p, (const gndt_column *)h->columns.p,
+         h->row_start, h->row_end, X, L, epoch);
+  launch(h, false, xchg_halo_wait_kernel, 1, 32, 0, st, h->ctl, X, L, epoch, have);
+  launch(h, false, xchg_halo_edges_kernel, grid_for(h, h->cap_voxels, 256, 4), 256, 0, st, h->ctl, (gndt_voxel *)h->table.p,
+         (gndt_slope *)h->slopes.p, reinterpret_cast<const gndt_voxel *>(mine + L.halo[0]),
+         reinterpret_cast<const gndt_voxel *>(mine + L.halo[1]), have, dp);
 }
 
 static int xchg_check(gndt_handle *h, const char *who) {
@@ -1143,20 +1166,16 @@ int gndt_xchg_run(gndt_handle *h, void *stream) {
   const u32 epoch = ++h->x_epoch;
   const XPeers &X = h->xp;
   const XLayout &L = h->xl;
-  u32 *done_counter = reinterpret_cast<u32 *>(static_cast<char *>(h->small.p) + 192);
-  static const int skip = [] { const char *e = getenv("GNDT_XCHG_SKIP"); return e ? atoi(e) : 0; }();  // diagnosis only
-  if (skip & 4) return GNDT_OK;
-  xchg_front(h, st, epoch, !(skip & 1));
-  if (skip & 2) return GNDT_OK;
+  u32 *done_counter = &static_cast<SmallWords *>(h->small.p)->x.done_counter;
+  xchg_front(h, st, epoch);
   // the bulk transfer and the final wait run on the high-priority stream, fenced by events on both sides
   GNDT_CUDA(h, cudaEventRecord(h->x_ev[0], st));
   GNDT_CUDA(h, cudaStreamWaitEvent(h->x_stream, h->x_ev[0], 0));
-  xchg_push_kernel<<<h->x_push_ctas, kPushThreads, 0, h->x_stream>>>(h->ctl, (const gndt_voxel *)h->table.p, (const gndt_slope *)h->slopes.p,
-                                                            (const gndt_column *)h->columns.p, X, L, h->x_what, epoch, done_counter, 0);
-  xchg_wait_kernel<<<1, 32, 0, h->x_stream>>>(h->ctl, X, L, epoch);
+  launch(h, false, xchg_push_kernel, kPushCtas, kPushThreads, 0, h->x_stream, h->ctl, (const gndt_voxel *)h->table.p,
+         (const gndt_slope *)h->slopes.p, (const gndt_column *)h->columns.p, X, L, h->x_what, epoch, done_counter, 0);
+  launch(h, false, xchg_wait_kernel, 1, 32, 0, h->x_stream, h->ctl, X, L, epoch);
   GNDT_CUDA(h, cudaEventRecord(h->x_ev[1], h->x_stream));
   GNDT_CUDA(h, cudaStreamWaitEvent(st, h->x_ev[1], 0));
-  h->launches += 2;
   h->counts_valid = false;
   h->last_stream = st;
   GNDT_CUDA(h, cudaGetLastError());
@@ -1180,14 +1199,13 @@ int gndt_xchg_stage(gndt_handle *h, void *stream) {
   const u32 epoch = ++h->x_epoch;
   const XPeers &X = h->xp;
   const XLayout &L = h->xl;
-  u32 *done_counter = reinterpret_cast<u32 *>(static_cast<char *>(h->small.p) + 192);
-  xchg_front(h, st, epoch, true);  // its halo gate has seen every strip's counts of this epoch
-  xchg_push_kernel<<<h->x_push_ctas, kPushThreads, 0, st>>>(h->ctl, (const gndt_voxel *)h->table.p, (const gndt_slope *)h->slopes.p,
-                                                   (const gndt_column *)h->columns.p, X, L, h->x_what, epoch, done_counter, 1);
+  u32 *done_counter = &static_cast<SmallWords *>(h->small.p)->x.done_counter;
+  xchg_front(h, st, epoch);  // its halo gate has seen every strip's counts of this epoch
+  launch(h, false, xchg_push_kernel, kPushCtas, kPushThreads, 0, st, h->ctl, (const gndt_voxel *)h->table.p, (const gndt_slope *)h->slopes.p,
+         (const gndt_column *)h->columns.p, X, L, h->x_what, epoch, done_counter, 1);
   const XMail *mail = reinterpret_cast<const XMail *>(X.buf[X.rank] + L.mail);
   GNDT_CUDA(h, cudaMemcpyAsync(h->x_counts_host, mail->counts[epoch & 1], kMaxRanks * 4 * sizeof(u32), cudaMemcpyDeviceToHost, st));
   GNDT_CUDA(h, cudaEventRecord(h->x_ev_counts, st));
-  h->launches += 1;
   h->x_staged = true;
   h->counts_valid = false;
   h->last_stream = st;
@@ -1244,11 +1262,10 @@ int gndt_xchg_send(gndt_handle *h, void *stream) {
     GNDT_CUDA(h, cudaEventRecord(j ? h->x_ev_copy : h->x_ev[0], h->x_copy[j]));
     GNDT_CUDA(h, cudaStreamWaitEvent(h->x_stream, j ? h->x_ev_copy : h->x_ev[0], 0));
   }
-  xchg_done_kernel<<<1, 32, 0, h->x_stream>>>(X, L, epoch);
-  xchg_wait_kernel<<<1, 32, 0, h->x_stream>>>(h->ctl, X, L, epoch);
+  launch(h, false, xchg_done_kernel, 1, 32, 0, h->x_stream, X, L, epoch);
+  launch(h, false, xchg_wait_kernel, 1, 32, 0, h->x_stream, h->ctl, X, L, epoch);
   GNDT_CUDA(h, cudaEventRecord(h->x_ev[1], h->x_stream));
   GNDT_CUDA(h, cudaStreamWaitEvent(st, h->x_ev[1], 0));
-  h->launches += 2;
   h->counts_valid = false;
   h->last_stream = st;
   GNDT_CUDA(h, cudaGetLastError());
@@ -1433,19 +1450,15 @@ int gndt_plan_tiles(gndt_handle *h, const void *xyz, size_t n, size_t stride_byt
   if (!h || !xyz || !cuts || ntiles < 1 || n == 0 || stride_bytes < 12 || (stride_bytes & 3)) return GNDT_ERR_INVALID_ARG;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   GNDT_CUDA(h, cudaSetDevice(h->device));
-  int rc;
-  const float *d_in = static_cast<const float *>(xyz);
-  if (mem == GNDT_MEM_HOST) {
-    if ((rc = ensure(h, h->in_stage, n * stride_bytes)) != GNDT_OK) return rc;
-    GNDT_CUDA(h, cudaMemcpyAsync(h->in_stage.p, xyz, n * stride_bytes, cudaMemcpyHostToDevice, st));
-    d_in = static_cast<const float *>(h->in_stage.p);
-  }
+  const float *d_in;
+  int rc = upload(h, h->in_stage, xyz, n * stride_bytes, mem, st, nullptr, &d_in);
+  if (rc != GNDT_OK) return rc;
   if ((rc = ensure(h, h->f_zero, 65536 * sizeof(u32) + 1024)) != GNDT_OK) return rc;
   GNDT_CUDA(h, cudaMemsetAsync(h->f_zero.p, 0, 65536 * sizeof(u32), st));
   const DevParams dp = make_dev(h, h->params, 0);
-  cx_hist_kernel<<<grid_for(h, n, 256 * 8, 8), 256, 0, st>>>((u32 *)h->f_zero.p, d_in, stride_bytes / 4, n,
-                                                             h->params.origin_is_first_point ? 1 : 0, dp);
-  h->launches += 1;
+  launch(h, false, cx_hist_kernel, grid_for(h, n, 256 * 8, 8), 256, 0, st, (u32 *)h->f_zero.p, d_in, stride_bytes / 4, n,
+         h->params.origin_is_first_point ? 1 : 0, dp);
+  GNDT_CUDA(h, cudaGetLastError());
   u32 *hist = (u32 *)malloc(65536 * sizeof(u32));
   cudaError_t e = cudaMemcpyAsync(hist, h->f_zero.p, 65536 * sizeof(u32), cudaMemcpyDeviceToHost, st);
   if (e == cudaSuccess) e = cudaStreamSynchronize(st);
@@ -1671,6 +1684,7 @@ int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes
   if ((rc = ndt_check_args(h, guess, np)) != GNDT_OK) return rc;
   GNDT_CUDA(h, cudaSetDevice(h->device));
   if ((rc = sync_counts(h)) != GNDT_OK) return rc;  // resolves a pending update / remove
+  KeepLaunchCount keep(h);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const gndt_params &rp = h->res_params;
   const u32 n_vox = h->host_ctl.n_voxels, n_cols = h->host_ctl.n_columns;
@@ -1678,15 +1692,11 @@ int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes
   // the resident map's Gaussians, once per map state
   if (!h->ndt_ready) {
     if ((rc = ensure(h, h->ndt_vox, std::max<size_t>(n_vox, 1) * sizeof(NdtVoxel))) != GNDT_OK) return rc;
-    ndt_prepare_kernel<<<grid_for(h, n_vox, 256, 8), 256, 0, st>>>(h->ctl, (const gndt_voxel *)h->table.p, (NdtVoxel *)h->ndt_vox.p,
-                                                                   rp.normalize_cov);
+    launch(h, false, ndt_prepare_kernel, grid_for(h, n_vox, 256, 8), 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p,
+           (NdtVoxel *)h->ndt_vox.p, rp.normalize_cov);
   }
-  const float *d_in = static_cast<const float *>(xyz);
-  if (mem == GNDT_MEM_HOST) {
-    if ((rc = ensure(h, h->ndt_pts, n * stride_bytes)) != GNDT_OK) return rc;
-    GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_pts.p, xyz, n * stride_bytes, cudaMemcpyHostToDevice, st));
-    d_in = static_cast<const float *>(h->ndt_pts.p);
-  }
+  const float *d_in;
+  if ((rc = upload(h, h->ndt_pts, xyz, n * stride_bytes, mem, st, nullptr, &d_in)) != GNDT_OK) return rc;
   const int blocks = grid_for(h, n, kNdtThreads, 8);
   if ((rc = ensure(h, h->ndt_part, ((size_t)blocks + 1) * kNdtWidth * sizeof(double))) != GNDT_OK) return rc;
   if (!h->ndt_host) GNDT_CUDA(h, cudaHostAlloc(&h->ndt_host, kNdtWidth * sizeof(double), cudaHostAllocDefault));
@@ -1694,8 +1704,8 @@ int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes
   const size_t stride_f = stride_bytes / 4;
 
   // centre: binary64 mean of the finite points, c = R pbar + t at every pose
-  ndt_mean_kernel<<<blocks, kNdtThreads, 0, st>>>(d_in, stride_f, n, part);
-  ndt_finish_kernel<<<1, 32, 0, st>>>(part, blocks, 4, dres);
+  launch(h, false, ndt_mean_kernel, blocks, kNdtThreads, 0, st, d_in, stride_f, n, part);
+  launch(h, false, ndt_finish_kernel, 1, 32, 0, st, part, blocks, 4, dres);
   GNDT_CUDA(h, cudaGetLastError());
   GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_host, dres, 4 * sizeof(double), cudaMemcpyDeviceToHost, st));
   GNDT_CUDA(h, cudaStreamSynchronize(st));
@@ -1722,9 +1732,9 @@ int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes
       P.t[i] = T[4 * i + 3];
       P.c[i] = T[4 * i] * pbar[0] + T[4 * i + 1] * pbar[1] + T[4 * i + 2] * pbar[2] + T[4 * i + 3];
     }
-    ndt_pass_kernel<<<blocks, kNdtThreads, 0, st>>>(d_in, stride_f, n, (const NdtVoxel *)h->ndt_vox.p, (const gndt_column *)h->columns.p,
-                                                    n_cols, P, part);
-    ndt_finish_kernel<<<1, 32, 0, st>>>(part, blocks, kNdtWidth, dres);
+    launch(h, false, ndt_pass_kernel, blocks, kNdtThreads, 0, st, d_in, stride_f, n, (const NdtVoxel *)h->ndt_vox.p,
+           (const gndt_column *)h->columns.p, n_cols, P, part);
+    launch(h, false, ndt_finish_kernel, 1, 32, 0, st, part, blocks, kNdtWidth, dres);
     GNDT_CUDA(h, cudaGetLastError());
     GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_host, dres, kNdtWidth * sizeof(double), cudaMemcpyDeviceToHost, st));
     GNDT_CUDA(h, cudaStreamSynchronize(st));

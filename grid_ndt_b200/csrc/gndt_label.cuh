@@ -41,13 +41,11 @@ struct __align__(128) FinSmem {
   u32 tile, total;
 };
 
-#ifndef GNDT_FIN_MINBLOCKS
-#define GNDT_FIN_MINBLOCKS 3
-#endif
 // 256 voxel threads + one helper warp: the helper publishes the block's (columns, slopes)
 // counts and resolves their prefix (two L2 round trips) WHILE the voxel warps do the eigen work.
 constexpr int kFinThreads = kLabelThreads + 32;
-__global__ void __launch_bounds__(kFinThreads, GNDT_FIN_MINBLOCKS)
+constexpr int kFinMinBlocks = 3;  // resident finalize CTAs per SM (__launch_bounds__)
+__global__ void __launch_bounds__(kFinThreads, kFinMinBlocks)
 finalize_label_kernel(Ctl *ctl, const VoxMoments *mom, gndt_voxel *table, gndt_slope *slopes,
                       gndt_column *columns, u32 *vfirst, u32 *slope_col, u64 *blk_state, GroupState *blk_groups, u32 *counters,
                       DevParams P) {

@@ -17,16 +17,11 @@
 
 namespace gndt {
 
-#ifndef GNDT_RED_MINBLOCKS
-#define GNDT_RED_MINBLOCKS 5
-#endif
-#ifndef GNDT_RED_LONGRUN
-#define GNDT_RED_LONGRUN 64
-#endif
 constexpr int kRedThreads = 256;
+constexpr int kRedMinBlocks = 5;                   // resident reduce CTAs per SM (__launch_bounds__)
 constexpr int kRedItems = 8;
 constexpr int kRedTile = kRedThreads * kRedItems;  // 2048 points
-constexpr int kLongRun = GNDT_RED_LONGRUN;          // longer runs are reduced by a whole warp each
+constexpr int kLongRun = 64;                        // longer runs are reduced by a whole warp each
 constexpr int kMaxLong = kRedTile / kLongRun;
 
 struct Moments {
@@ -210,7 +205,7 @@ __device__ __forceinline__ void store_moments(VoxMoments *dst, u64 key, u32 firs
 // K3: one CTA per tile of 2048 sorted points -> raw moments of every voxel whose run starts
 // in the tile; partial runs at the tile edges go to the carry array.
 template <bool FAST>
-__global__ void __launch_bounds__(kRedThreads, GNDT_RED_MINBLOCKS)
+__global__ void __launch_bounds__(kRedThreads, kRedMinBlocks)
 reduce_kernel(Ctl *ctl, const float4 *buf_a, const float4 *buf_b, VoxMoments *mom, TileCarry *carry,
               u64 *tile_state, GroupState *tile_groups, DevParams P) {
   pdl_wait();

@@ -14,8 +14,8 @@ constexpr int kScanItems = 4;
 constexpr int kScanTile = 256 * kScanItems;
 
 // out[i] = sum of in[0..i), out[n] = total (also ScanCtl::total).  n = *n_dev when n_dev != NULL.
-// `state` needs ceil(n / kScanTile) + 1 words, `groups` ceil(that / kScanGroup) + 1 entries, `g`,
-// `state` and `groups` zeroed before the launch.
+// `state` and `groups` are lookback_scratch(ceil(n / kScanTile)); `g`, `state` and `groups` are
+// zeroed before the launch.
 __global__ void __launch_bounds__(256)
 exclusive_scan_kernel(ScanCtl *g, const u32 *in, u32 n_fixed, const u32 *n_dev, u32 *out, u64 *state, GroupState *groups) {
   __shared__ u32 warp_sums[32];

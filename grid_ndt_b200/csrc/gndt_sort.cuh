@@ -27,27 +27,16 @@
 
 namespace gndt {
 
-#ifndef GNDT_SORT_THREADS
-#define GNDT_SORT_THREADS 512
-#endif
-#ifndef GNDT_SORT_ITEMS
-#define GNDT_SORT_ITEMS 8
-#endif
-#ifndef GNDT_SORT_MINBLOCKS
-#define GNDT_SORT_MINBLOCKS 2
-#endif
-constexpr int kSortThreads = GNDT_SORT_THREADS;
-constexpr int kSortItems = GNDT_SORT_ITEMS;
+constexpr int kSortThreads = 512;
+constexpr int kSortItems = 8;
+constexpr int kSortMinBlocks = 2;                     // resident partition CTAs per SM (__launch_bounds__)
 constexpr int kSortTile = kSortThreads * kSortItems;  // points per tile
 constexpr int kSortWarps = kSortThreads / 32;
 constexpr int kFirstMaxBits = 8;                      // first digit: fixed look-back stride, zeroed by the bounds pass
 constexpr int kFirstMaxBins = 1 << kFirstMaxBits;
 constexpr int kDigitsPerThread = (kMaxBins + kSortThreads - 1) / kSortThreads;
 static_assert(kSortThreads % 32 == 0 && kSortTile < 65536 && 32 * kSortItems < 65536, "tile shape");
-#ifndef GNDT_SORT_GROUP
-#define GNDT_SORT_GROUP 16
-#endif
-constexpr int kSortGroup = GNDT_SORT_GROUP;  // tiles per look-back group
+constexpr int kSortGroup = 16;               // tiles per look-back group
 constexpr int kGroupSumBits = 26;            // group word: arrivals << 26 | sum of the tiles' digit counts
 static_assert(kSortGroup >= 1 && kSortGroup < 64 && (long long)kSortGroup * kSortTile < (1ll << kGroupSumBits), "group word");
 
@@ -288,7 +277,7 @@ __device__ __forceinline__ u64 block_exclusive_scan64(u64 v, u64 *warp_sums) {
 // pass, zeroed here by the whole grid (their size depends on that pass's digit width).
 // ---------------------------------------------------------------------------------------
 template <bool FIRST, bool FAST>
-__global__ void __launch_bounds__(kSortThreads, GNDT_SORT_MINBLOCKS)
+__global__ void __launch_bounds__(kSortThreads, kSortMinBlocks)
 sort_pass_kernel(Ctl *ctl, int pass, const float *in_raw, size_t stride_f, size_t n_in, size_t start,
                  const float4 *src, float4 *dst, u32 *lb, u64 *glb, u32 *lb_next, u64 *glb_next, u32 *hist_all,
                  DevParams P) {

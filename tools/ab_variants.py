@@ -19,7 +19,7 @@ for _ in range(builds):
     s = m.stage_ms(); tot.append(s["total"])
     best = s if best is None else {k: min(best[k], s[k]) for k in s}
 c = m.counts()
-print(json.dumps({"lib": os.path.basename(os.environ.get("GNDT_LIB", "default")) + os.environ.get("GNDT_SORT_WAVES", ""), "stage_ms": {k: round(v, 4) for k, v in best.items() if k != "h2d"},
+print(json.dumps({"lib": os.path.basename(os.environ.get("GNDT_LIB", "default")), "stage_ms": {k: round(v, 4) for k, v in best.items() if k != "h2d"},
                   "median_total": round(sorted(tot)[len(tot) // 2], 4), "layout": m.key_layout(), "voxels": c["n_voxels"], "launches": m.launch_count()}))
 ''' % ROOT
 

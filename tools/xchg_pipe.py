@@ -1,5 +1,5 @@
-"""Diagnosis: pipelined throughput of TiledTwoDmap (depth 3) with parts of the exchange switched off (GNDT_XCHG_SKIP:
-1 halo, 2 push + wait, 4 everything).  Run under torchrun; one setting per process."""
+"""Diagnosis: pipelined throughput of TiledTwoDmap (DEPTH builds in flight, default 3) with the exchange transport
+TRANSPORT ("sm" or "ce").  Run under torchrun; one setting per process."""
 import json, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, torch.distributed as dist
@@ -26,5 +26,5 @@ e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=Tr
 e0.record(); run(30); e1.record(); torch.cuda.synchronize()
 t = torch.tensor([e0.elapsed_time(e1) / 30], device=dev); dist.all_reduce(t, op=dist.ReduceOp.MAX)
 bm = torch.zeros(world, device=dev); bm[rank] = float(np.mean(build_ms[-30:])); dist.all_reduce(bm)
-if rank == 0: print(json.dumps({"world": world, "depth": depth, "transport": tm.transport, "skip": os.environ.get("GNDT_XCHG_SKIP", "0"), "ms_per_step": round(float(t.item()), 4), "build_ms_per_rank": [round(float(x), 3) for x in bm.tolist()]}), flush=True)
+if rank == 0: print(json.dumps({"world": world, "depth": depth, "transport": tm.transport, "ms_per_step": round(float(t.item()), 4), "build_ms_per_rank": [round(float(x), 3) for x in bm.tolist()]}), flush=True)
 dist.barrier(); dist.destroy_process_group()

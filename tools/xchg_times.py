@@ -1,6 +1,5 @@
 """Where the strip exchange spends its time (run under torchrun, N >= 2): strip build alone, build + exchange one
-at a time, the exchange alone (events around gndt_xchg_run), per push grid size (GNDT_XCHG_CTAS is read at first use,
-so each setting runs in a fresh process: call this script once per setting)."""
+at a time, the exchange alone (events around gndt_xchg_run)."""
 import ctypes as C, json, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, torch.distributed as dist
@@ -32,7 +31,7 @@ def build_xchg():
     tm.build(cloud, "slope", origin=origin, cuts=None, filter_points=False)
 def xchg_only():
     _check(m._h, L.gndt_xchg_run(m._h, torch.cuda.current_stream().cuda_stream))
-res = {"world": world, "ctas": os.environ.get("GNDT_XCHG_CTAS", "sm_count"), "gather": gather,
+res = {"world": world, "gather": gather,
        "build_ms": timed(build_only), "build_xchg_ms": timed(build_xchg)}
 build_only(); torch.cuda.synchronize(); dist.barrier()
 res["xchg_only_ms"] = timed(xchg_only)
