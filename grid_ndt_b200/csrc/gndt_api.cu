@@ -49,7 +49,7 @@ struct SmallWords {
   Totals tot;           // over every cloud fused into the map (totals_kernel); read back by sync_counts
   u32 n_new;            // new voxels of the pending update (update_prepare_kernel -> merge)
   struct {
-    int have[2];        // which halo rows arrived (xchg_halo_wait_kernel -> xchg_halo_edges_kernel)
+    int have[2];        // which halo rows arrived (xchg_halo_wait_kernel -> halo_edges_kernel)
     u32 done_counter;   // push CTAs finished; the last one resets it
   } x;                  // strip exchange, zeroed by gndt_xchg_create
 };
@@ -479,10 +479,10 @@ int front_end(gndt_handle *h, cudaStream_t st, const float *d_in, size_t n, size
   return GNDT_OK;
 }
 
-__global__ void table_bounds_kernel(Ctl *ctl, const gndt_voxel *table, u32 n_fixed) {
+__global__ void table_bounds_kernel(Ctl *ctl, const gndt_voxel *table) {
   pdl_wait();
   pdl_trigger();
-  const u32 n = n_fixed ? n_fixed : ctl->n_voxels;
+  const u32 n = ctl->n_voxels;
   if (threadIdx.x == 0 && n && !ctl->err) {
     ctl->cx_min = contiguous_index(table[0].sx);
     ctl->cx_max = contiguous_index(table[n - 1].sx);
@@ -495,12 +495,12 @@ int back_end(gndt_handle *h, cudaStream_t st, const DevParams &dp, const VoxMome
   launch(h, true, finalize_label_kernel, g_lab, kFinThreads, sizeof(FinSmem), st, h->ctl, mom, (gndt_voxel *)h->table.p,
          (gndt_slope *)h->slopes.p, (gndt_column *)h->columns.p, (u32 *)h->vfirst.p, (u32 *)h->slope_col.p, h->blk_state, h->blk_groups,
          &h->ctl->ticket[7], dp);
-  if (bounds_from_table) launch(h, true, table_bounds_kernel, 1, 32, 0, st, h->ctl, (const gndt_voxel *)h->table.p, 0u);
-  launch(h, true, column_finish_kernel, g_lab, 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p, (const u32 *)h->vfirst.p, 0u,
-         (gndt_column *)h->columns.p, h->row_start, h->row_end, 0, 0);
+  if (bounds_from_table) launch(h, true, table_bounds_kernel, 1, 32, 0, st, h->ctl, (const gndt_voxel *)h->table.p);
+  launch(h, true, column_finish_kernel, g_lab, 256, 0, st, h->ctl, (const u32 *)h->vfirst.p, (gndt_column *)h->columns.p,
+         h->row_start, h->row_end);
   if (h->stage_timing) GNDT_CUDA(h, cudaEventRecord(h->ev[EV_LABEL], st));
   launch(h, true, edges_kernel, g_lab, 256, 0, st, h->ctl, (gndt_voxel *)h->table.p, (gndt_slope *)h->slopes.p,
-         (const gndt_column *)h->columns.p, (const u32 *)h->slope_col.p, (const u32 *)h->row_start, (const u32 *)h->row_end, 0, 0, 0, dp);
+         (const gndt_column *)h->columns.p, (const u32 *)h->slope_col.p, (const u32 *)h->row_start, (const u32 *)h->row_end, dp);
   GNDT_CUDA(h, cudaEventRecord(h->ev[EV_EDGES], st));
   return GNDT_OK;
 }
@@ -907,8 +907,8 @@ int gndt_halo_pack(gndt_handle *h, gndt_voxel *first_row_out, gndt_voxel *last_r
   if (!h->built) { h->err = "no map has been built on this handle"; return GNDT_ERR_STATE; }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   GNDT_CUDA(h, cudaSetDevice(h->device));
-  launch(h, false, halo_pack_kernel, 2, 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p, (const gndt_column *)h->columns.p,
-         h->row_start, h->row_end, first_row_out, last_row_out, (u32)cap_records);
+  launch(h, false, halo_pack_kernel, 2, 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p, first_row_out, last_row_out,
+         (u32)cap_records);
   GNDT_CUDA(h, cudaGetLastError());
   return GNDT_OK;
 }
@@ -920,7 +920,7 @@ int gndt_halo_edges(gndt_handle *h, const gndt_voxel *from_prev, const gndt_voxe
   GNDT_CUDA(h, cudaSetDevice(h->device));
   const DevParams dp = make_dev(h, h->params, h->cap_voxels);
   launch(h, false, halo_edges_kernel, grid_for(h, h->cap_voxels, 256, 8), 256, 0, st, h->ctl, (gndt_voxel *)h->table.p,
-         (gndt_slope *)h->slopes.p, from_prev, from_next, dp);
+         (gndt_slope *)h->slopes.p, from_prev, from_next, nullptr, dp);
   h->counts_valid = false;
   GNDT_CUDA(h, cudaGetLastError());
   return GNDT_OK;
@@ -1142,10 +1142,9 @@ static void xchg_front(gndt_handle *h, cudaStream_t st, u32 epoch) {
   const DevParams dp = make_dev(h, h->params, h->cap_voxels);
   unsigned char *mine = X.buf[X.rank];
   launch(h, false, xchg_publish_kernel, 1, 32, 0, st, h->ctl, X, L, epoch);
-  launch(h, false, xchg_halo_send_kernel, 2, 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p, (const gndt_column *)h->columns.p,
-         h->row_start, h->row_end, X, L, epoch);
+  launch(h, false, xchg_halo_send_kernel, 2, 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p, X, L, epoch);
   launch(h, false, xchg_halo_wait_kernel, 1, 32, 0, st, h->ctl, X, L, epoch, have);
-  launch(h, false, xchg_halo_edges_kernel, grid_for(h, h->cap_voxels, 256, 4), 256, 0, st, h->ctl, (gndt_voxel *)h->table.p,
+  launch(h, false, halo_edges_kernel, grid_for(h, h->cap_voxels, 256, 4), 256, 0, st, h->ctl, (gndt_voxel *)h->table.p,
          (gndt_slope *)h->slopes.p, reinterpret_cast<const gndt_voxel *>(mine + L.halo[0]),
          reinterpret_cast<const gndt_voxel *>(mine + L.halo[1]), have, dp);
 }

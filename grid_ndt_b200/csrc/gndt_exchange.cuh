@@ -1,5 +1,4 @@
-// gndt_exchange.cuh — multi-GPU x strips: thin halo + gather of the finished tables through
-// peer-mapped memory (NVLink / NVSwitch), no NCCL, no host round trip.
+// gndt_exchange.cuh — multi-GPU x strips: thin halo + gather of the finished tables.
 //
 // SURVEY §8(e): every quantity up to the surface labels depends on one x-y column only, so the
 // strips are built without communication.  What crosses GPUs is (1) the first / last x row of a
@@ -7,17 +6,22 @@
 // neighbours, reference include/map2D.h:219-253, that live on another GPU), and (2) the
 // finished tables, so that every GPU (and the host planner behind it) holds the whole map.
 //
-// Every rank owns one exchange buffer that its peers map (cudaIpc between processes, plain peer
-// access inside one process): a mailbox, two halo rows, and the gathered tables.  All traffic is
-// PUSHED by the producer with ordinary stores to the peer's buffer, followed by a system-scope
-// fence and an epoch flag in the peer's mailbox; consumers spin on flags in their OWN memory.
-// Strip sizes never visit the host: ranks publish their counts to every mailbox and every rank
-// derives the offsets of all strips on the device.
+// The halo row format, its packer, the boundary-edge kernel and the index rule of a gathered voxel
+// record serve two transports: the caller's own (gndt_halo_pack / gndt_halo_edges /
+// gndt_apply_strip_offsets, e.g. over NCCL) and the library's, through peer-mapped memory
+// (NVLink / NVSwitch), no NCCL, no host round trip (gndt_xchg_*).
+//
+// In the library's transport every rank owns one exchange buffer that its peers map (cudaIpc
+// between processes, plain peer access inside one process): a mailbox, two halo rows, and the
+// gathered tables.  All traffic is PUSHED by the producer with ordinary stores to the peer's
+// buffer, followed by a system-scope fence and an epoch flag in the peer's mailbox; consumers spin
+// on flags in their OWN memory.  Strip sizes never visit the host: ranks publish their counts to
+// every mailbox and every rank derives the offsets of all strips on the device.
 //
 //   publish   counts of this strip -> every mailbox
 //   halo_send first row -> nearest non-empty lower strip, last row -> nearest non-empty upper strip
 //             (empty strips are skipped: their neighbours exchange rows with each other)
-//   halo_edges (gndt_label.cuh) once both rows have arrived
+//   halo_edges once both rows have arrived
 //   push      this strip's voxel / slope / column records, strip-local indices made global on the
 //             fly, into every rank's gathered tables at the strip's offset; then a `done` flag
 //   wait      until every strip has arrived here
@@ -26,6 +30,109 @@
 #include "gndt_label.cuh"
 
 namespace gndt {
+
+// ---- the halo, shared by both transports --------------------------------------------------
+
+struct HaloHeader {  // occupies the first 96-byte slot of a halo buffer
+  u32 count;         // records that follow (0 when the strip is empty or the row did not fit)
+  int cx;            // contiguous x index of the packed row
+  u32 overflow;      // row larger than the buffer: the receiver raises GNDT_ERR_CAPACITY
+  u32 pad[21];
+};
+static_assert(sizeof(HaloHeader) == sizeof(gndt_voxel), "header uses one record slot");
+
+// Pack the strip's first (last = false) or last x row into `out`: header + up to cap records.
+// Called by every thread of one CTA, which copies cooperatively.
+__device__ __forceinline__ void pack_halo_row(const Ctl *ctl, const gndt_voxel *table, bool last, gndt_voxel *out, u32 cap) {
+  const u32 V = ctl->n_voxels;
+  u32 lo = 0, hi = 0;
+  int cx = 0;
+  if (V && ctl->n_columns && !ctl->err) {
+    lo = last ? ctl->last_row_begin : 0u;
+    hi = last ? V : ctl->first_row_end;
+    cx = last ? ctl->cx_max : ctl->cx_min;
+  }
+  const u32 n = hi - lo;
+  const bool fits = n <= cap;
+  HaloHeader *hdr = reinterpret_cast<HaloHeader *>(out);
+  if (threadIdx.x == 0) { hdr->count = fits ? n : 0; hdr->cx = cx; hdr->overflow = fits ? 0u : 1u; }
+  if (!fits) return;
+  const float4 *src = reinterpret_cast<const float4 *>(table + lo);
+  float4 *dst = reinterpret_cast<float4 *>(out + 1);
+  for (u32 i = threadIdx.x; i < n * 6; i += blockDim.x) dst[i] = src[i];
+}
+
+// Block 0 packs the first x row into `first_out`, block 1 the last x row into `last_out`.
+__global__ void __launch_bounds__(256)
+halo_pack_kernel(const Ctl *ctl, const gndt_voxel *table, gndt_voxel *first_out, gndt_voxel *last_out, u32 cap) {
+  const bool last = blockIdx.x == 1;
+  pack_halo_row(ctl, table, last, last ? last_out : first_out, cap);
+}
+
+// Does the halo row hold, in the column with contiguous y index `cy`, a Slope reachable from
+// (normal n, n_len = normal_length(n), mean z)?  Halo records are voxels sorted by (cy, cz).
+__device__ __forceinline__ bool halo_reachable(const gndt_voxel *halo, u32 n_halo, int cy, const float n[3], double n_len,
+                                               float mz, const DevParams &P) {
+  u32 lo = 0, hi = n_halo;
+  while (lo < hi) {
+    const u32 mid = (lo + hi) >> 1;
+    if (contiguous_index(halo[mid].sy) < cy) lo = mid + 1; else hi = mid;
+  }
+  for (u32 v = lo; v < n_halo && contiguous_index(halo[v].sy) == cy; ++v) {
+    const gndt_voxel &t = halo[v];
+    if ((t.flags & GNDT_F_SLOPE) && reachable(t.normal, t.rough, t.mean[2], t.flags, n, n_len, mz, P)) return true;
+  }
+  return false;
+}
+
+// Fix the forward/back reachability of this strip's boundary rows against the neighbours'
+// halo rows: `from_prev` = last row of the strip below in x, `from_next` = first row of the
+// strip above.  A row is ignored when its pointer is NULL (an end of the map) or when
+// have[0] / have[1] is 0 (no neighbour sent it); have = NULL means the rows given are present.
+__global__ void __launch_bounds__(256)
+halo_edges_kernel(Ctl *ctl, gndt_voxel *table, gndt_slope *slopes, const gndt_voxel *from_prev, const gndt_voxel *from_next,
+                  const int *have, DevParams P) {
+  const u32 S = ctl->n_slopes;
+  const int cx_lo = ctl->cx_min, cx_hi = ctl->cx_max;
+  const HaloHeader *hp = (!have || have[0]) ? reinterpret_cast<const HaloHeader *>(from_prev) : nullptr;
+  const HaloHeader *hn = (!have || have[1]) ? reinterpret_cast<const HaloHeader *>(from_next) : nullptr;
+  if ((hp && hp->overflow) || (hn && hn->overflow)) { if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(&ctl->err, kErrCapacity); return; }
+  const bool use_prev = hp && hp->count && hp->cx == cx_lo - 1;  // adjacent x rows only
+  const bool use_next = hn && hn->count && hn->cx == cx_hi + 1;
+  if (!use_prev && !use_next) return;
+  for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < S; i += gridDim.x * blockDim.x) {
+    const int cx = contiguous_index(slopes[i].sx);
+    if (cx != cx_lo && cx != cx_hi) continue;
+    const gndt_slope me = slopes[i];
+    const int cy = contiguous_index(me.sy);
+    const float n[3] = {me.normal[0], me.normal[1], me.normal[2]};
+    const double n_len = normal_length(n);
+    u32 bits = 0;
+    if (use_prev && cx == cx_lo && halo_reachable(from_prev + 1, hp->count, cy, n, n_len, me.mean[2], P)) bits |= GNDT_F_REACH_B;
+    if (use_next && cx == cx_hi && halo_reachable(from_next + 1, hn->count, cy, n, n_len, me.mean[2], P)) bits |= GNDT_F_REACH_F;
+    if (bits) {
+      slopes[i].flags = me.flags | bits;
+      table[me.voxel].flags |= bits;
+    }
+  }
+}
+
+// The strip-local `column` / `slope` indices of a gathered voxel record made global: the strip's
+// columns and Slopes before it are added; a voxel without a Slope keeps slope = 0xFFFFFFFF.
+__device__ __forceinline__ void globalize_voxel_indices(u32 &column, u32 &slope, u32 cols_before, u32 slopes_before) {
+  column += cols_before;
+  if (slope != 0xFFFFFFFFu) slope += slopes_before;
+}
+
+// After the caller's all-gather: globalize the records [begin, begin+count) of one strip.
+__global__ void strip_offsets_kernel(gndt_voxel *table, u64 begin, u64 count, u32 col_off, u32 slope_off) {
+  for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (u64)gridDim.x * blockDim.x) {
+    gndt_voxel *r = table + begin + i;
+    globalize_voxel_indices(r->column, r->slope, col_off, slope_off);
+  }
+}
+
+// ---- the library's transport through peer-mapped memory ------------------------------------
 
 constexpr int kMaxRanks = 16;
 constexpr u32 kXWaitLimitNs = 4000000000u;  // a peer that never shows up trips the watchdog after 4 s
@@ -99,11 +206,9 @@ __device__ __forceinline__ int nearest_nonempty(const XMail *mine, u32 epoch, in
   return -1;
 }
 
-// X2: block 0 sends the first x row down, block 1 the last x row up.  Same row format as
-// halo_pack_kernel (header slot + records).
+// X2: block 0 sends the first x row down, block 1 the last x row up.
 __global__ void __launch_bounds__(256)
-xchg_halo_send_kernel(Ctl *ctl, const gndt_voxel *table, const gndt_column *columns, const u32 *row_start, const u32 *row_end,
-                      XPeers X, XLayout L, u32 epoch) {
+xchg_halo_send_kernel(Ctl *ctl, const gndt_voxel *table, XPeers X, XLayout L, u32 epoch) {
   __shared__ int s_target;
   const bool last = blockIdx.x == 1;
   const XMail *mine = reinterpret_cast<const XMail *>(X.buf[X.rank] + L.mail);
@@ -118,32 +223,7 @@ xchg_halo_send_kernel(Ctl *ctl, const gndt_voxel *table, const gndt_column *colu
   if (target < 0) return;
   // my first row is the target's "from the upper neighbour" row (slot 1), my last row its "from the lower" (slot 0)
   const int slot = last ? 0 : 1;
-  gndt_voxel *out = reinterpret_cast<gndt_voxel *>(X.buf[target] + L.halo[slot]);
-  HaloHeader *hdr = reinterpret_cast<HaloHeader *>(out);
-  const u32 V = ctl->n_voxels, C = ctl->n_columns;
-  u32 lo = 0, hi = 0;
-  int cx = 0;
-  {
-    const int n_rows = ctl->cx_max - ctl->cx_min + 1;
-    if (!last) {
-      const u32 c_end = row_end[0];
-      lo = 0;
-      hi = (c_end < C) ? columns[c_end].voxel_begin : V;
-      cx = ctl->cx_min;
-    } else {
-      lo = columns[row_start[n_rows - 1]].voxel_begin;
-      hi = V;
-      cx = ctl->cx_max;
-    }
-  }
-  const u32 n = hi - lo;
-  const bool fits = n <= (u32)L.cap_halo;
-  if (threadIdx.x == 0) { hdr->count = fits ? n : 0; hdr->cx = cx; hdr->overflow = fits ? 0u : 1u; }
-  if (fits) {
-    const float4 *src = reinterpret_cast<const float4 *>(table + lo);
-    float4 *dst = reinterpret_cast<float4 *>(out + 1);
-    for (u32 i = threadIdx.x; i < n * 6; i += blockDim.x) dst[i] = src[i];
-  }
+  pack_halo_row(ctl, table, last, reinterpret_cast<gndt_voxel *>(X.buf[target] + L.halo[slot]), (u32)L.cap_halo);
   __threadfence_system();
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -152,8 +232,8 @@ xchg_halo_send_kernel(Ctl *ctl, const gndt_voxel *table, const gndt_column *colu
   }
 }
 
-// X3: wait for the neighbours' rows, then finish the forward / back reach bits of this strip's
-// boundary rows (halo_edges_kernel does the work; this is its gate, one thread).
+// X3: wait for the neighbours' rows and tell halo_edges_kernel, which runs next, which of them
+// arrived (one thread).
 __global__ void xchg_halo_wait_kernel(Ctl *ctl, XPeers X, XLayout L, u32 epoch, int *have /* [2] */) {
   if (threadIdx.x || blockIdx.x) return;
   const XMail *mine = reinterpret_cast<const XMail *>(X.buf[X.rank] + L.mail);
@@ -166,34 +246,6 @@ __global__ void xchg_halo_wait_kernel(Ctl *ctl, XPeers X, XLayout L, u32 epoch, 
   if (!ok) atomicOr(&ctl->err, kErrWatchdog);
   have[0] = prev >= 0 ? 1 : 0;
   have[1] = next >= 0 ? 1 : 0;
-}
-
-// halo_edges with the row pointers gated by `have` (a row that no neighbour sent is ignored).
-__global__ void __launch_bounds__(256)
-xchg_halo_edges_kernel(Ctl *ctl, gndt_voxel *table, gndt_slope *slopes, const gndt_voxel *from_prev, const gndt_voxel *from_next,
-                       const int *have, DevParams P) {
-  const u32 S = ctl->n_slopes;
-  const int cx_lo = ctl->cx_min, cx_hi = ctl->cx_max;
-  const HaloHeader *hp = have[0] ? reinterpret_cast<const HaloHeader *>(from_prev) : nullptr;
-  const HaloHeader *hn = have[1] ? reinterpret_cast<const HaloHeader *>(from_next) : nullptr;
-  if ((hp && hp->overflow) || (hn && hn->overflow)) { if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(&ctl->err, kErrCapacity); return; }
-  const bool use_prev = hp && hp->count && hp->cx == cx_lo - 1;  // adjacent x rows only
-  const bool use_next = hn && hn->count && hn->cx == cx_hi + 1;
-  if (!use_prev && !use_next) return;
-  for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < S; i += gridDim.x * blockDim.x) {
-    const int cx = contiguous_index(slopes[i].sx);
-    if (cx != cx_lo && cx != cx_hi) continue;
-    const gndt_slope me = slopes[i];
-    const int cy = contiguous_index(me.sy);
-    const float n[3] = {me.normal[0], me.normal[1], me.normal[2]};
-    u32 bits = 0;
-    if (use_prev && cx == cx_lo && halo_reachable(from_prev + 1, hp->count, cy, n, me.mean[2], P)) bits |= GNDT_F_REACH_B;
-    if (use_next && cx == cx_hi && halo_reachable(from_next + 1, hn->count, cy, n, me.mean[2], P)) bits |= GNDT_F_REACH_F;
-    if (bits) {
-      slopes[i].flags = me.flags | bits;
-      table[me.voxel].flags |= bits;
-    }
-  }
 }
 
 // X4: push this strip into every rank's gathered tables.  16-byte chunks, each loaded ONCE and
@@ -222,7 +274,7 @@ __device__ __forceinline__ void push_table(const uint4 *src, size_t n_chunks, si
       const size_t i = i0 + u * stride;
       if (i >= n_chunks) break;
       const u32 part = (u32)(i % kPer);
-      if (KIND == 0) { if (part == 5) { v[u].z += off[1]; if (v[u].w != 0xFFFFFFFFu) v[u].w += off[2]; } }
+      if (KIND == 0) { if (part == 5) globalize_voxel_indices(v[u].z, v[u].w, off[1], off[2]); }
       else if (KIND == 1) { if (part == 2) v[u].w += off[0]; }
       else { if (part == 0) v[u].w += off[0]; else v[u].y += off[2]; }
       for (int p = p_lo; p < p_hi; ++p) reinterpret_cast<uint4 *>(X.buf[p] + dst_off_bytes)[first_chunk + i] = v[u];

@@ -10,8 +10,8 @@
 // themselves, several layers per neighbour cell.  List order = the reference's: left, right,
 // forward, back cell; inside a cell ascending z (std::map<int, Slope*> order).
 // Predicate = countReachable with comand 2.5 / 4 and the checkList variant (:284-287,306-315):
-// !up && rough <= rough_max && countAngle <= angle_max && |dz| <= reach_height.  (The 3-D
-// comparison variant countReachable3D, :323-338, has no `up` test and is not reproduced.)
+// `reachable` of gndt_label.cuh, which also decides the reach bits.  (The 3-D comparison
+// variant countReachable3D, :323-338, has no `up` test and is not reproduced.)
 //
 // Works from a (slopes, columns) table pair alone — a single GPU's or the gathered tables of
 // a multi-GPU map — and builds its own x-row directory.
@@ -71,11 +71,7 @@ graph_edges_kernel(const gndt_slope *slopes, u32 S, const gndt_column *columns, 
       const gndt_column c = columns[nb[d]];
       for (u32 s = c.slope_begin; s < c.slope_begin + c.slope_count; ++s) {
         const gndt_slope &t = slopes[s];
-        if (t.flags & GNDT_F_UP) continue;
-        if (!(t.rough <= P.rough_max)) continue;
-        const float tn[3] = {t.normal[0], t.normal[1], t.normal[2]};
-        if (!(count_angle(tn, n, n_len) <= P.angle_max_deg)) continue;
-        if (!(fabsf(__fsub_rn(t.mean[2], me.mean[2])) <= P.reach_height)) continue;
+        if (!reachable(t.normal, t.rough, t.mean[2], t.flags, n, n_len, me.mean[2], P)) continue;
         if (FILL) targets[base + k] = s;
         ++k;
       }

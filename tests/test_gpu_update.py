@@ -168,9 +168,19 @@ def test_remove_undoes_update():
 
 
 def test_failed_update_and_remove_leave_the_map_unchanged():
-    """ADVICE r1: a capacity overflow used to leave the resident map half-fused."""
-    _gpu()
-    from grid_ndt_b200 import GndtError, TwoDmap
+    """ADVICE r1: a capacity overflow used to leave the resident map half-fused.  The halo rows
+    of the map are checked too: a failed call must not change what gndt_halo_pack sends."""
+    torch = _gpu()
+    from grid_ndt_b200 import GndtError, TwoDmap, lib
+    from grid_ndt_b200.builder import _check
+    cap = 65536
+
+    def halo():  # first and last x row of m, packed into fresh zeroed buffers
+        bufs = torch.zeros(2, (cap + 1) * _abi.VOXEL_DTYPE.itemsize, dtype=torch.uint8, device="cuda")
+        _check(m._h, lib().gndt_halo_pack(m._h, bufs[0].data_ptr(), bufs[1].data_ptr(), cap, 0))
+        torch.cuda.synchronize()
+        return bufs.cpu().numpy().tobytes()
+
     cloud = synthetic.cfg2(500_000, scale=0.22)
     a, b = cloud[:300_000], cloud[300_000:]
     m = TwoDmap(0.2, 0.1)
@@ -183,16 +193,21 @@ def test_failed_update_and_remove_leave_the_map_unchanged():
     m.params.max_voxels = n0 + 10  # room for the map of A, not for A + B
     m.chatterCallback(a, "slope")
     before = (m.voxels.tobytes(), m.slopes.tobytes(), m.columns.tobytes(), m.counts())
+    halo_before = halo()
+    hdr = np.frombuffer(halo_before, np.uint32).reshape(2, -1)[:, :3]  # count, cx, overflow of each row
+    assert (hdr[:, 0] > 0).all() and (hdr[:, 2] == 0).all() and hdr[0, 0] + hdr[1, 0] < before[3]["n_voxels"]
     m.change2DMap(b)
     with pytest.raises(GndtError) as e:
         m.counts()
     assert e.value.status == _abi.GNDT_ERR_CAPACITY
     assert (m.voxels.tobytes(), m.slopes.tobytes(), m.columns.tobytes(), m.counts()) == before
+    assert halo() == halo_before
     m.del2DMap(b)  # never fused
     with pytest.raises(GndtError) as e:
         m.counts()
     assert e.value.status == _abi.GNDT_ERR_STATE
     assert (m.voxels.tobytes(), m.slopes.tobytes(), m.columns.tobytes(), m.counts()) == before
+    assert halo() == halo_before
     m.params.max_voxels = 0
     # changing the cell size under a resident map is refused (two key spaces cannot be fused)
     m.setLen(0.3)
