@@ -7,6 +7,7 @@
 // All stream-ordered with no host round trip; counts are read back only when asked for.
 #include <algorithm>
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -47,13 +48,15 @@ struct DivCheck {  // result of the exhaustive hoisted-division check for one ce
 // Device words that outlive a build (h->small)
 struct SmallWords {
   Totals tot;           // over every cloud fused into the map (totals_kernel); read back by sync_counts
+  u32 fuse_err;         // Ctl::err as the pending update / remove left it (its verdict); read back with tot
   u32 n_new;            // new voxels of the pending update (update_prepare_kernel -> merge)
   struct {
     int have[2];        // which halo rows arrived (xchg_halo_wait_kernel -> halo_edges_kernel)
     u32 done_counter;   // push CTAs finished; the last one resets it
   } x;                  // strip exchange, zeroed by gndt_xchg_create
 };
-static_assert(sizeof(Totals) == 32 && sizeof(SmallWords) == 48, "SmallWords layout");
+static_assert(sizeof(Totals) == 32 && sizeof(SmallWords) == 56, "SmallWords layout");
+static_assert(offsetof(SmallWords, fuse_err) == sizeof(Totals), "fuse_err is read back together with the totals");
 
 }  // namespace
 
@@ -119,8 +122,11 @@ struct gndt_handle {
   // copy-engine transport (gndt_xchg_stage / gndt_xchg_send)
   cudaStream_t x_copy[2] = {};     // the peer copies alternate between two streams (two engines busy)
   cudaEvent_t x_ev_counts = nullptr, x_ev_copy = nullptr;
-  u32 *x_counts_host = nullptr;    // pinned: every strip's {voxels, columns, slopes, epoch} of the staged epoch
+  u32 *x_counts_host = nullptr;    // pinned: every strip's {voxels, columns, slopes, epoch, failed, ...} of the staged epoch
   bool x_staged = false;
+  int x_send_rc = GNDT_OK;         // verdict of the last gndt_xchg_send, reported again by gndt_xchg_view_get
+  std::string x_send_err;
+  bool x_peer_failed = false;      // the last gndt_xchg_view_get failed because ANOTHER strip failed
   u32 x_epoch = 0;
   bool x_created = false, x_connected = false;
   // state
@@ -128,6 +134,7 @@ struct gndt_handle {
   bool counts_valid = false;
   Ctl host_ctl;
   Totals host_tot, saved_tot;
+  u32 host_fuse_err = 0;       // SmallWords::fuse_err, read back with host_tot
   cudaStream_t last_stream = nullptr;
   cudaEvent_t ev[EV_COUNT] = {};
   bool timed_h2d = false;
@@ -407,14 +414,17 @@ int sync_counts(gndt_handle *h) {
   // handles on other streams (a pipelined caller) keep running while this one is read back
   GNDT_CUDA(h, cudaMemcpyAsync(&h->host_ctl, h->ctl, sizeof(Ctl), cudaMemcpyDeviceToHost, h->last_stream));
   GNDT_CUDA(h, cudaMemcpyAsync(&h->host_tot, h->small.p, sizeof(Totals), cudaMemcpyDeviceToHost, h->last_stream));
+  if (h->pending_fuse)
+    GNDT_CUDA(h, cudaMemcpyAsync(&h->host_fuse_err, &static_cast<SmallWords *>(h->small.p)->fuse_err, sizeof(u32), cudaMemcpyDeviceToHost,
+                                 h->last_stream));
   GNDT_CUDA(h, cudaStreamSynchronize(h->last_stream));
-  if (h->pending_fuse) {  // verdict of the last gndt_update / gndt_remove
-    const int sign = h->pending_fuse;
+  if (h->pending_fuse) {  // verdict of the last gndt_update / gndt_remove, from ITS error bits: a halo or an
+    const int sign = h->pending_fuse;  // exchange enqueued behind it may have raised more since
     h->pending_fuse = 0;
-    if (h->host_ctl.err) {
+    if (h->host_fuse_err) {
       // failed on the device: the resident moments were never touched and the tables were not rewritten
       // (the back end returns at once when the error word is set); put the counters back
-      const u32 e = h->host_ctl.err;
+      const u32 e = h->host_fuse_err;
       h->host_ctl = h->saved_ctl;
       h->host_tot = h->saved_tot;
       GNDT_CUDA(h, cudaMemcpyAsync(h->ctl, &h->saved_ctl, sizeof(Ctl), cudaMemcpyHostToDevice, h->last_stream));
@@ -435,8 +445,12 @@ int sync_counts(gndt_handle *h) {
     h->n_changed = nc;
     h->n_changed_valid = true;
   }
-  if (h->host_ctl.err & kErrWatchdog) { h->err = "device watchdog tripped (look-back / TMA wait never resolved)"; return GNDT_ERR_INTERNAL; }
-  if (h->host_ctl.err & kErrCapacity) { h->err = "voxel table capacity (max_voxels) exceeded"; return GNDT_ERR_CAPACITY; }
+  // bits raised by the build (or after the update's verdict, by the halo and the exchange) stay until the next build
+  const u32 e = h->host_ctl.err;
+  if (e & kErrWatchdog) { h->err = "device watchdog tripped (look-back / TMA / exchange wait never resolved)"; return GNDT_ERR_INTERNAL; }
+  if (e & kErrCapacity) { h->err = "voxel table capacity (max_voxels) exceeded"; return GNDT_ERR_CAPACITY; }
+  if (e & kErrHaloCapacity) { h->err = "a neighbour strip's halo row exceeds cap_halo_records"; return GNDT_ERR_CAPACITY; }
+  if (e & kErrGatherCapacity) { h->err = "gathered map exceeds the exchange capacity (cap_records)"; return GNDT_ERR_CAPACITY; }
   h->counts_valid = true;
   return GNDT_OK;
 }
@@ -814,6 +828,8 @@ static int fuse_scan(gndt_handle *h, const void *xyz, size_t n, size_t stride_by
   launch(h, false, changed_order_kernel, grid_for(h, cap_vox, 256, 8), 256, 0, st, h->ctl, touch_first, dp.idx_offset, (u32)n, order, valid);
   exclusive_scan(2, valid, (u32)n, nullptr, order_pos, n);
   launch(h, false, changed_compact_kernel, g_scan, 256, 0, st, order, valid, order_pos, (u32)n, changed);
+  // the verdict: Ctl::err as this call leaves it, before anything enqueued behind it adds bits
+  GNDT_CUDA(h, cudaMemcpyAsync(&small->fuse_err, &h->ctl->err, sizeof(u32), cudaMemcpyDeviceToDevice, st));
   GNDT_CUDA(h, cudaGetLastError());
   h->changed_dev = changed;
   h->changed_count_dev = &at<ScanCtl>(w, sc[2].ctl)->total;
@@ -1050,6 +1066,17 @@ int gndt_xchg_create(gndt_handle *h, int rank, int world, size_t cap_records, si
     return GNDT_ERR_INVALID_ARG;
   if (cap_records > 0xFFFFFFFEull) return GNDT_ERR_CAPACITY;
   GNDT_CUDA(h, cudaSetDevice(h->device));
+  // Load every kernel of the exchange now.  Under lazy module loading (the CUDA 12 default) the first
+  // launch of a kernel loads it, and loading may wait for the kernels running on the device.  A rank's
+  // halo send spins until every rank has published, so a host thread that drives several ranks and
+  // enqueued rank 0's halo send would block loading rank 0's next kernel until the 4 s watchdog fired.
+  const void *xk[] = {(const void *)xchg_publish_kernel, (const void *)xchg_halo_send_kernel, (const void *)xchg_halo_wait_kernel,
+                      (const void *)halo_edges_kernel,   (const void *)xchg_push_kernel,      (const void *)xchg_done_kernel,
+                      (const void *)xchg_wait_kernel};
+  for (const void *k : xk) {
+    cudaFuncAttributes fa;
+    GNDT_CUDA(h, cudaFuncGetAttributes(&fa, k));
+  }
   XLayout L = {};
   Layout B;
   L.mail = B.take(sizeof(XMail));
@@ -1082,7 +1109,7 @@ int gndt_xchg_create(gndt_handle *h, int rank, int world, size_t cap_records, si
     for (int i = 0; i < 2; ++i) GNDT_CUDA(h, cudaStreamCreateWithFlags(&h->x_copy[i], cudaStreamNonBlocking));
     GNDT_CUDA(h, cudaEventCreateWithFlags(&h->x_ev_counts, cudaEventDisableTiming));
     GNDT_CUDA(h, cudaEventCreateWithFlags(&h->x_ev_copy, cudaEventDisableTiming));
-    GNDT_CUDA(h, cudaHostAlloc(reinterpret_cast<void **>(&h->x_counts_host), kMaxRanks * 4 * sizeof(u32), cudaHostAllocDefault));
+    GNDT_CUDA(h, cudaHostAlloc(reinterpret_cast<void **>(&h->x_counts_host), kMaxRanks * kXCountWords * sizeof(u32), cudaHostAllocDefault));
   }
   h->x_staged = false;
   memset(mine, 0, sizeof(*mine));
@@ -1166,6 +1193,7 @@ int gndt_xchg_run(gndt_handle *h, void *stream) {
   const XPeers &X = h->xp;
   const XLayout &L = h->xl;
   u32 *done_counter = &static_cast<SmallWords *>(h->small.p)->x.done_counter;
+  h->x_send_rc = GNDT_OK;
   xchg_front(h, st, epoch);
   // the bulk transfer and the final wait run on the high-priority stream, fenced by events on both sides
   GNDT_CUDA(h, cudaEventRecord(h->x_ev[0], st));
@@ -1185,7 +1213,7 @@ int gndt_xchg_run(gndt_handle *h, void *stream) {
 // SM-issued stores to peers slow the build that runs beside them on the SENDING GPU (measured:
 // profiles/xchg_overlap_r2.md); copy-engine transfers do not.  The engines need sizes and addresses
 // on the host, so the exchange is split: gndt_xchg_stage enqueues everything up to the strip sitting,
-// indices made global, in this rank's own gathered tables, plus a 256-byte read-back of every strip's
+// indices made global, in this rank's own gathered tables, plus a 512-byte read-back of every strip's
 // counts; gndt_xchg_send waits for that read-back (the one host round trip; the next builds are
 // already queued behind it) and enqueues the peer copies, the `done` flags and the final wait.
 int gndt_xchg_stage(gndt_handle *h, void *stream) {
@@ -1199,11 +1227,12 @@ int gndt_xchg_stage(gndt_handle *h, void *stream) {
   const XPeers &X = h->xp;
   const XLayout &L = h->xl;
   u32 *done_counter = &static_cast<SmallWords *>(h->small.p)->x.done_counter;
+  h->x_send_rc = GNDT_OK;
   xchg_front(h, st, epoch);  // its halo gate has seen every strip's counts of this epoch
   launch(h, false, xchg_push_kernel, kPushCtas, kPushThreads, 0, st, h->ctl, (const gndt_voxel *)h->table.p, (const gndt_slope *)h->slopes.p,
          (const gndt_column *)h->columns.p, X, L, h->x_what, epoch, done_counter, 1);
   const XMail *mail = reinterpret_cast<const XMail *>(X.buf[X.rank] + L.mail);
-  GNDT_CUDA(h, cudaMemcpyAsync(h->x_counts_host, mail->counts[epoch & 1], kMaxRanks * 4 * sizeof(u32), cudaMemcpyDeviceToHost, st));
+  GNDT_CUDA(h, cudaMemcpyAsync(h->x_counts_host, mail->counts[epoch & 1], kMaxRanks * kXCountWords * sizeof(u32), cudaMemcpyDeviceToHost, st));
   GNDT_CUDA(h, cudaEventRecord(h->x_ev_counts, st));
   h->x_staged = true;
   h->counts_valid = false;
@@ -1235,13 +1264,23 @@ int gndt_xchg_send(gndt_handle *h, void *stream) {
   const int W = X.world;
   uint64_t off[3] = {0, 0, 0}, total = 0;  // voxels, columns, slopes before this strip
   for (int r = 0; r < W; ++r) {
-    const u32 *c = h->x_counts_host + 4 * r;
-    if (c[3] != epoch) { h->err = "gndt_xchg_send: strip " + std::to_string(r) + " never published its counts (watchdog)"; return GNDT_ERR_INTERNAL; }
+    const u32 *c = h->x_counts_host + kXCountWords * r;
+    if (c[3] != epoch) {
+      h->x_send_err = "gndt_xchg_send: strip " + std::to_string(r) + " never published its counts (watchdog)";
+      h->x_send_rc = GNDT_ERR_INTERNAL;
+    }
     if (r < X.rank) for (int k = 0; k < 3; ++k) off[k] += c[k];
     total += c[0];
   }
-  if (total > L.cap_records) { h->err = "gathered map exceeds the exchange capacity: " + std::to_string(total) + " > " + std::to_string(L.cap_records) + " records"; return GNDT_ERR_CAPACITY; }
-  const u32 *own = h->x_counts_host + 4 * X.rank;
+  if (h->x_send_rc == GNDT_OK && total > L.cap_records) {
+    h->x_send_err = "gathered map exceeds the exchange capacity: " + std::to_string(total) + " > " + std::to_string(L.cap_records) + " records";
+    h->x_send_rc = GNDT_ERR_CAPACITY;
+  }
+  if (h->x_send_rc != GNDT_OK) {  // nothing was sent: gndt_xchg_view_get reports the same verdict
+    h->err = h->x_send_err;
+    return h->x_send_rc;
+  }
+  const u32 *own = h->x_counts_host + kXCountWords * X.rank;
   struct { int bit; size_t base, rec; uint64_t first, n; } tab[3] = {
       {GNDT_X_VOXELS, L.voxels, sizeof(gndt_voxel), off[0], own[0]},
       {GNDT_X_SLOPES, L.slopes, sizeof(gndt_slope), off[2], own[2]},
@@ -1274,8 +1313,10 @@ int gndt_xchg_send(gndt_handle *h, void *stream) {
 int gndt_xchg_view_get(gndt_handle *h, gndt_xchg_view *out) {
   if (!h || !out) return GNDT_ERR_INVALID_ARG;
   if (!h->x_connected || h->x_epoch == 0) { h->err = "gndt_xchg_view_get: no exchange has run"; return GNDT_ERR_STATE; }
+  h->x_peer_failed = false;
   int rc = sync_counts(h);  // synchronises the stream, surfaces watchdog / capacity errors
   if (rc != GNDT_OK) return rc;
+  if (h->x_send_rc != GNDT_OK) { h->err = h->x_send_err; return h->x_send_rc; }
   XMail mail;
   GNDT_CUDA(h, cudaMemcpy(&mail, h->xp.buf[h->xp.rank] + h->xl.mail, sizeof(XMail), cudaMemcpyDeviceToHost));
   memset(out, 0, sizeof(*out));
@@ -1288,6 +1329,11 @@ int gndt_xchg_view_get(gndt_handle *h, gndt_xchg_view *out) {
   for (int r = 0; r < h->xp.world; ++r) {
     const u32 *c = mail.counts[par][r];
     if (c[3] != h->x_epoch || mail.done[par][r] != h->x_epoch) { h->err = "exchange incomplete (epoch mismatch)"; return GNDT_ERR_INTERNAL; }
+    if (c[4]) {  // its records are missing from the gathered tables
+      h->err = "strip " + std::to_string(r) + " failed its build / update and sent no records; the gathered map is incomplete";
+      h->x_peer_failed = true;
+      return GNDT_ERR_STATE;
+    }
     out->strip_voxels[r] = c[0];
     out->strip_columns[r] = c[1];
     out->strip_slopes[r] = c[2];
@@ -1416,14 +1462,16 @@ int gndt_multi_update(gndt_multi *m, const void *xyz, size_t n, size_t stride_by
 
 int gndt_multi_view(gndt_multi *m, int index, gndt_xchg_view *out) {
   if (!m || !out || index < 0 || index >= (int)m->h.size()) return GNDT_ERR_INVALID_ARG;
-  // a failure on one strip shows up as a watchdog on the others: report the first real error
+  // a strip that failed makes the others fail too (they name it): report the failing strip's own error
+  int first = -1, first_rc = GNDT_OK;
   for (size_t i = 0; i < m->h.size(); ++i) {
     cudaSetDevice(m->dev[i]);
     gndt_xchg_view v;
     const int rc = gndt_xchg_view_get(m->h[i], (int)i == index ? out : &v);
-    if (rc != GNDT_OK) return multi_fail(m, (int)i, rc, "exchange");
+    if (rc == GNDT_OK || (first >= 0 && !m->h[first]->x_peer_failed)) continue;
+    if (first < 0 || !m->h[i]->x_peer_failed) { first = (int)i; first_rc = rc; }
   }
-  return GNDT_OK;
+  return first < 0 ? GNDT_OK : multi_fail(m, first, first_rc, "exchange");
 }
 
 int gndt_multi_cuts(gndt_multi *m, int32_t *cuts, int cap) {

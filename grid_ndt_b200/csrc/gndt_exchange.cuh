@@ -89,14 +89,17 @@ __device__ __forceinline__ bool halo_reachable(const gndt_voxel *halo, u32 n_hal
 // halo rows: `from_prev` = last row of the strip below in x, `from_next` = first row of the
 // strip above.  A row is ignored when its pointer is NULL (an end of the map) or when
 // have[0] / have[1] is 0 (no neighbour sent it); have = NULL means the rows given are present.
+// A strip with an error pending (e.g. an update that failed: its tables were not rewritten and
+// Ctl does not describe them until the verdict restores it) is left alone.
 __global__ void __launch_bounds__(256)
 halo_edges_kernel(Ctl *ctl, gndt_voxel *table, gndt_slope *slopes, const gndt_voxel *from_prev, const gndt_voxel *from_next,
                   const int *have, DevParams P) {
+  if (ctl->err) return;
   const u32 S = ctl->n_slopes;
   const int cx_lo = ctl->cx_min, cx_hi = ctl->cx_max;
   const HaloHeader *hp = (!have || have[0]) ? reinterpret_cast<const HaloHeader *>(from_prev) : nullptr;
   const HaloHeader *hn = (!have || have[1]) ? reinterpret_cast<const HaloHeader *>(from_next) : nullptr;
-  if ((hp && hp->overflow) || (hn && hn->overflow)) { if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(&ctl->err, kErrCapacity); return; }
+  if ((hp && hp->overflow) || (hn && hn->overflow)) { if (blockIdx.x == 0 && threadIdx.x == 0) atomicOr(&ctl->err, kErrHaloCapacity); return; }
   const bool use_prev = hp && hp->count && hp->cx == cx_lo - 1;  // adjacent x rows only
   const bool use_next = hn && hn->count && hn->cx == cx_hi + 1;
   if (!use_prev && !use_next) return;
@@ -141,8 +144,10 @@ constexpr u32 kXWaitLimitNs = 4000000000u;  // a peer that never shows up trips 
 // the parity of the epoch: a peer may already be one build ahead on this buffer (it publishes the
 // counts of epoch e + 1 as soon as ITS build is done) while the owner's host still reads epoch e;
 // it cannot be two ahead, because epoch e + 1 completes only after the owner has joined it.
+constexpr int kXCountWords = 8;  // {n_voxels, n_columns, n_slopes, epoch, failed, unused x 3}
 struct XMail {
-  u32 counts[2][kMaxRanks][4];  // {n_voxels, n_columns, n_slopes, epoch} of every strip
+  u32 counts[2][kMaxRanks][kXCountWords];  // of every strip; failed = 1: it published zero counts because its
+                                           // build / update failed (its records are missing everywhere)
   u32 halo_epoch[2][2];         // [.][0] row from the lower neighbour arrived, [.][1] from the upper
   u32 done[2][kMaxRanks];       // strip r has been pushed into this rank's gathered tables
 };
@@ -189,6 +194,7 @@ __global__ void xchg_publish_kernel(const Ctl *ctl, XPeers X, XLayout L, u32 epo
   st_sys(c + 0, bad ? 0u : ctl->n_voxels);
   st_sys(c + 1, bad ? 0u : ctl->n_columns);
   st_sys(c + 2, bad ? 0u : ctl->n_slopes);
+  st_sys(c + 4, bad ? 1u : 0u);
   __threadfence_system();
   st_sys(c + 3, epoch);
 }
@@ -297,7 +303,7 @@ xchg_push_kernel(Ctl *ctl, const gndt_voxel *table, const gndt_slope *slopes, co
   const u32 *own = mine->counts[epoch & 1][X.rank];
   const u32 nv = ld_sys(own + 0), nc = ld_sys(own + 1), ns = ld_sys(own + 2);
   const bool fits = total[0] <= L.cap_records;
-  if (!fits && blockIdx.x == 0 && threadIdx.x == 0) atomicOr(&ctl->err, kErrCapacity);
+  if (!fits && blockIdx.x == 0 && threadIdx.x == 0) atomicOr(&ctl->err, kErrGatherCapacity);
   // local_only: this strip goes (indices made global) into the OWN gathered tables only; the copy engines
   // carry it to the peers from there (gndt_xchg_send) and a separate kernel raises the `done` flags
   const int p_lo = local_only ? X.rank : 0, p_hi = local_only ? X.rank + 1 : X.world;

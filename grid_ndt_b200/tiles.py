@@ -87,7 +87,7 @@ class TiledTwoDmap:
                  capacity: int = 8_000_000, transport: Optional[str] = None):
         """exchange: "native" (peer-mapped memory inside libgndt.so) or "nccl" (point-to-point).
         transport (native only): "ce" = the records travel by copy engine (gndt_xchg_stage / gndt_xchg_send: one
-        256-byte host round trip per build, hidden behind the builds already queued; does not slow the build
+        512-byte host round trip per build, hidden behind the builds already queued; does not slow the build
         running beside it), "sm" = pushed by an SM kernel (gndt_xchg_run: no host round trip, but the build
         beside it on the sending GPU slows down by about the duration of the push).  Default: "ce"
         (GNDT_XCHG_TRANSPORT overrides).
@@ -128,6 +128,7 @@ class TiledTwoDmap:
         self._next = 0
         self._inflight = deque()
         self._last = self.slots[0]
+        self._cuts = None  # strip boundaries of the resident build (update() keeps them)
 
     @property
     def depth(self) -> int:
@@ -176,6 +177,7 @@ class TiledTwoDmap:
         if not update:
             if origin is not None:
                 m.setCloudFirst(origin)
+            self._cuts = np.asarray(cuts, np.int64) if cuts is not None and filter_points else None
             if cuts is not None and filter_points:
                 lo, hi = int(cuts[self.rank]), int(cuts[self.rank + 1])
                 # an empty strip (equal cuts: one x row holds more than its share of the points)
@@ -208,18 +210,19 @@ class TiledTwoDmap:
             slot_b = (self.halo_records + 1) * REC
             send_first, send_last, recv_prev, recv_next = (s.halo[i * slot_b:(i + 1) * slot_b] for i in range(4))
             _check(m._h, L.gndt_halo_pack(m._h, send_first.data_ptr(), send_last.data_ptr(), self.halo_records, st))
+            prev, nxt = halo_peers(self._cuts, self.rank, self.world)
             ops = []
-            if self.rank > 0:
-                ops += [dist.P2POp(dist.isend, send_first, self.rank - 1, group=self.group),
-                        dist.P2POp(dist.irecv, recv_prev, self.rank - 1, group=self.group)]
-            if self.rank + 1 < self.world:
-                ops += [dist.P2POp(dist.isend, send_last, self.rank + 1, group=self.group),
-                        dist.P2POp(dist.irecv, recv_next, self.rank + 1, group=self.group)]
+            if prev is not None:
+                ops += [dist.P2POp(dist.isend, send_first, prev, group=self.group),
+                        dist.P2POp(dist.irecv, recv_prev, prev, group=self.group)]
+            if nxt is not None:
+                ops += [dist.P2POp(dist.isend, send_last, nxt, group=self.group),
+                        dist.P2POp(dist.irecv, recv_next, nxt, group=self.group)]
             if ops:
                 for req in dist.batch_isend_irecv(ops):
                     req.wait()
-            _check(m._h, L.gndt_halo_edges(m._h, recv_prev.data_ptr() if self.rank > 0 else None,
-                                           recv_next.data_ptr() if self.rank + 1 < self.world else None, st))
+            _check(m._h, L.gndt_halo_edges(m._h, recv_prev.data_ptr() if prev is not None else None,
+                                           recv_next.data_ptr() if nxt is not None else None, st))
             p_cnt = C.c_void_p()
             _check(m._h, L.gndt_device_count_ptr(m._h, C.byref(p_cnt)))
             mine = _as_tensor(p_cnt.value, 16, s.device).view(torch.int32)
@@ -417,6 +420,21 @@ class TiledTwoDmap:
     def close(self):
         for s in self.slots:
             s.map.close()
+
+
+def halo_peers(cuts, rank: int, world: int):
+    """(lower, upper) halo peer of `rank`, None at an end of the map: the nearest ranks whose strip
+    [cuts[r], cuts[r+1]) is not empty.  An empty strip (equal cuts) keeps nothing and swaps no rows,
+    and the strips on either side of it swap theirs with each other, since their x rows may touch.
+    Every rank derives the same pairs from the same cuts, so each send has its matching receive.
+    cuts = None (no strip filter): the ranks either side."""
+    if cuts is None:
+        return (rank - 1 if rank > 0 else None), (rank + 1 if rank + 1 < world else None)
+    full = [r for r in range(world) if cuts[r] < cuts[r + 1]]
+    if rank not in full:
+        return None, None
+    i = full.index(rank)
+    return (full[i - 1] if i > 0 else None), (full[i + 1] if i + 1 < len(full) else None)
 
 
 def _as_tensor(ptr: int, nbytes: int, device) -> torch.Tensor:

@@ -233,6 +233,12 @@ int gndt_update(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, 
  *     moments, labels under GNDT_DEMAND_TRUE) equals the batch build without that scan.
  * Every point of the scan must have been fused before: otherwise the call fails with
  * GNDT_ERR_STATE at the next result query and the map is left unchanged.
+ *
+ * Verdict of gndt_update / gndt_remove: the next result query decides it from the call's own
+ * device work, whatever was enqueued behind it since.  A halo or strip exchange that runs before
+ * that query (gndt_halo_edges, gndt_xchg_*) and fails (a halo row over cap_halo_records, a map
+ * over cap_records, a watchdog) does not undo the update: the update stands, and the exchange's
+ * status is reported at every query from then on, as after a build, until the next build.
  */
 int gndt_remove(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem,
                 void *stream);
@@ -344,7 +350,7 @@ int gndt_xchg_run(gndt_handle *h, void *stream);
  * build that runs beside an SM push on the sending GPU loses about as much time as the push takes;
  * copy-engine traffic does not disturb it: profiles/xchg_overlap_r2.md).  gndt_xchg_stage enqueues, on
  * `stream`, everything up to this strip sitting in the rank's own gathered tables (indices global)
- * and a 256-byte read-back of all strips' counts.  gndt_xchg_send blocks the HOST until that
+ * and a 512-byte read-back of all strips' counts.  gndt_xchg_send blocks the HOST until that
  * read-back has landed (one round trip; enqueue the next builds first), then enqueues the peer
  * copies, the completion flags and the final wait, and makes `stream` wait for them.
  * gndt_xchg_counts_ready: 1 if gndt_xchg_send would not block, 0 if it would, < 0 on error.
@@ -354,7 +360,10 @@ int gndt_xchg_stage(gndt_handle *h, void *stream);
 int gndt_xchg_counts_ready(gndt_handle *h);
 int gndt_xchg_send(gndt_handle *h, void *stream);
 /* Synchronises the exchange stream; fails with GNDT_ERR_CAPACITY if the map outgrew
- * cap_records / a row outgrew cap_halo_records, GNDT_ERR_INTERNAL if a peer never showed up. */
+ * cap_records / a row outgrew cap_halo_records (both transports; with gndt_xchg_send the status
+ * it returned), GNDT_ERR_INTERNAL if a peer never showed up, and GNDT_ERR_STATE, naming the strip,
+ * if another strip's build / update failed: that strip sends no records, so the gathered map is
+ * incomplete.  A rank whose own build / update failed reports that failure instead. */
 int gndt_xchg_view_get(gndt_handle *h, gndt_xchg_view *out);
 
 /*

@@ -115,6 +115,12 @@ def main():
     same_table("empty strip: gathered columns vs untiled build", tm.gathered_numpy("columns"), ref_c)
     if rank == 0:
         print("multi-gpu empty-strip ok:", tm.strip_counts[:, 0].tolist(), flush=True)
+    if world >= 3:  # the NCCL halo must pair strips 0 and 2 across the empty strip 1 as well
+        tn = results["nccl"][0]
+        tn.build(dev_cloud, "slope", origin=origin, cuts=cuts_e, filter_points=True)
+        same_table("empty strip, nccl: gathered voxels vs untiled build", tn.gathered_numpy(), ref_v)
+        if rank == 0:
+            print("multi-gpu empty-strip nccl ok:", tn.strip_counts[:, 0].tolist(), flush=True)
 
     # two builds in flight (depth 2: the gather of the first overlaps the build of the second)
     # must give the same bytes as one-at-a-time builds
