@@ -993,8 +993,8 @@ int gndt_build_edges(gndt_handle *h, const gndt_slope *slopes, size_t n_slopes, 
     GNDT_CUDA(h, cudaMemcpyAsync(&ends[0], columns, sizeof(gndt_column), cudaMemcpyDeviceToHost, st));
     GNDT_CUDA(h, cudaMemcpyAsync(&ends[1], columns + n_columns - 1, sizeof(gndt_column), cudaMemcpyDeviceToHost, st));
     GNDT_CUDA(h, cudaStreamSynchronize(st));
-    cx_lo = ends[0].sx > 0 ? ends[0].sx - 1 : ends[0].sx;
-    cx_hi = ends[1].sx > 0 ? ends[1].sx - 1 : ends[1].sx;
+    cx_lo = contiguous_index(ends[0].sx);
+    cx_hi = contiguous_index(ends[1].sx);
   }
   const int n_rows = cx_hi - cx_lo + 1;
   const u32 S = (u32)n_slopes, C = (u32)n_columns;
@@ -1488,7 +1488,9 @@ __global__ void cx_hist_kernel(u32 *hist, const float *in, size_t stride_f, size
   for (size_t i = start + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_in; i += (size_t)gridDim.x * blockDim.x) {
     float4 p = load_point(in, stride_f, i, vec);
     int cx, cy, cz;
-    if (point_indices(p.x, p.y, p.z, o, P, cx, cy, cz)) atomicAdd(&hist[cx + kIdxBias], 1u);
+    const bool ok = P.fast_div ? point_indices<true>(p.x, p.y, p.z, o, P.grid_len, P.z_len, P.rinv[0], P.rinv[1], cx, cy, cz)
+                               : point_indices<false>(p.x, p.y, p.z, o, P.grid_len, P.z_len, P.rinv[0], P.rinv[1], cx, cy, cz);
+    if (ok) atomicAdd(&hist[cx + kIdxBias], 1u);
   }
 }
 

@@ -27,24 +27,8 @@ __global__ void graph_prepare_kernel(const gndt_column *columns, u32 C, int cx_b
   for (u32 c = blockIdx.x * blockDim.x + threadIdx.x; c < C; c += gridDim.x * blockDim.x) {
     const gndt_column col = columns[c];
     for (u32 s = col.slope_begin; s < col.slope_begin + col.slope_count; ++s) slope_col[s] = c;
-    const int cx = contiguous_index(col.sx);
-    if (c == 0 || contiguous_index(columns[c - 1].sx) != cx) row_start[cx - cx_base] = c;
-    if (c + 1 == C || contiguous_index(columns[c + 1].sx) != cx) row_end[cx - cx_base] = c + 1;
+    mark_row(columns, C, c, contiguous_index(col.sx), cx_base, row_start, row_end);
   }
-}
-
-// Column index of cell (ncx, cy) given the x-row directory, or C if the cell is empty.
-__device__ __forceinline__ u32 find_in_row(const gndt_column *columns, u32 C, const u32 *row_start, const u32 *row_end, int cx_base,
-                                           int n_rows, int ncx, int cy) {
-  const int r = ncx - cx_base;
-  if (r < 0 || r >= n_rows) return C;
-  u32 lo = row_start[r], hi = row_end[r];
-  const u32 end = hi;
-  while (lo < hi) {
-    const u32 mid = (lo + hi) >> 1;
-    if (contiguous_index(columns[mid].sy) < cy) lo = mid + 1; else hi = mid;
-  }
-  return (lo < end && contiguous_index(columns[lo].sy) == cy) ? lo : C;
 }
 
 // G2 (FILL = false): number of reachable Slopes per Slope; G4 (FILL = true): the lists.
@@ -54,15 +38,11 @@ graph_edges_kernel(const gndt_slope *slopes, u32 S, const gndt_column *columns, 
                    const u32 *row_end, int cx_base, int n_rows, u32 *deg, const u32 *offsets, u32 *targets, DevParams P) {
   for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < S; i += gridDim.x * blockDim.x) {
     const gndt_slope me = slopes[i];
-    const int cx = contiguous_index(me.sx), cy = contiguous_index(me.sy);
-    const u32 ci = slope_col[i];
     const float n[3] = {me.normal[0], me.normal[1], me.normal[2]};
     const double n_len = normal_length(n);
-    u32 nb[4] = {C, C, C, C};  // left (cy-1), right (cy+1), forward (cx+1), back (cx-1): countLRFB in contiguous indices
-    if (ci > 0 && contiguous_index(columns[ci - 1].sx) == cx && contiguous_index(columns[ci - 1].sy) == cy - 1) nb[0] = ci - 1;
-    if (ci + 1 < C && contiguous_index(columns[ci + 1].sx) == cx && contiguous_index(columns[ci + 1].sy) == cy + 1) nb[1] = ci + 1;
-    nb[2] = find_in_row(columns, C, row_start, row_end, cx_base, n_rows, cx + 1, cy);
-    nb[3] = find_in_row(columns, C, row_start, row_end, cx_base, n_rows, cx - 1, cy);
+    u32 nb[4] = {C, C, C, C};
+    neighbour_columns(columns, C, slope_col[i], contiguous_index(me.sx), contiguous_index(me.sy), row_start, row_end, cx_base, n_rows,
+                      [&](int d, u32 c, const gndt_column &) { nb[d] = c; });
     u32 k = 0;
     const u32 base = FILL ? offsets[i] : 0u;
 #pragma unroll

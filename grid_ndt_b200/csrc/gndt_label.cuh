@@ -16,8 +16,6 @@ namespace gndt {
 
 constexpr int kLabelThreads = 256;
 
-__device__ __forceinline__ int contiguous_index(int s) { return s > 0 ? s - 1 : s; }
-
 // isSlope restated in closed form (SURVEY Q8): processing order inside a column is
 // ascending first_index; a neighbour u contributes its centroid z only if it was fitted
 // BEFORE v (count >= min_points and first(u) < first(v)), else the constructor's 0.
@@ -216,6 +214,76 @@ finalize_label_kernel(Ctl *ctl, const VoxMoments *mom, gndt_voxel *table, gndt_s
   }
 }
 
+// The x-row directory of a sorted column table: row_start[cx - cx_base] = the first column of
+// x row cx, row_end[cx - cx_base] = one past its last.  Column c (of x row cx) writes the
+// entries it delimits and returns which: bit 0 the row's first column, bit 1 its last.
+__device__ __forceinline__ int mark_row(const gndt_column *columns, u32 C, u32 c, int cx, int cx_base, u32 *row_start,
+                                        u32 *row_end) {
+  int ends = 0;
+  if (c == 0 || contiguous_index(columns[c - 1].sx) != cx) { row_start[cx - cx_base] = c; ends |= 1; }
+  if (c + 1 == C || contiguous_index(columns[c + 1].sx) != cx) { row_end[cx - cx_base] = c + 1; ends |= 2; }
+  return ends;
+}
+
+// The columns of the cells left (cy - 1), right (cy + 1), forward (cx + 1) and back (cx - 1) of
+// column ci = (cx, cy): countLRFB (map2D.h:197-263) in contiguous indices, which is its quadrant
+// crossing (x==1 / y==1 cases, :219-253) without the special cases.  Left and right are the
+// adjacent columns of the same x row.  Forward and back are a search for cy in the neighbouring
+// x row of the directory (mark_row) of rows [cx_base, cx_base + n_rows).
+// visit(d, index, column) is called for each non-empty neighbour cell, d = 0..3 in that order,
+// with the record already loaded: returning indices instead makes the caller reload the record
+// behind a select, which costs edges_kernel a dependent load per direction.
+template <class Visit>
+__device__ __forceinline__ void neighbour_columns(const gndt_column *columns, u32 C, u32 ci, int cx, int cy, const u32 *row_start,
+                                                  const u32 *row_end, int cx_base, int n_rows, Visit visit) {
+  if (ci > 0) {
+    const gndt_column c = columns[ci - 1];
+    if (contiguous_index(c.sx) == cx && contiguous_index(c.sy) == cy - 1) visit(0, ci - 1, c);
+  }
+  if (ci + 1 < C) {
+    const gndt_column c = columns[ci + 1];
+    if (contiguous_index(c.sx) == cx && contiguous_index(c.sy) == cy + 1) visit(1, ci + 1, c);
+  }
+#pragma unroll
+  for (int dir = 0; dir < 2; ++dir) {
+    const int r = cx + (dir == 0 ? 1 : -1) - cx_base;
+    if (r < 0 || r >= n_rows) continue;
+    // first column of the neighbour row with cy' >= cy.  Neighbouring rows of a map are
+    // populated alike, so the same offset as in the own row is a good first guess; gallop
+    // from it to bracket cy, then bisect the bracket (1-3 probes instead of log2(row)).
+    const u32 r_lo = row_start[r], r_hi = row_end[r];
+    u32 lo = r_lo, hi = r_hi;
+    if (r_lo < r_hi) {
+      const u32 g = r_lo + min(ci - row_start[cx - cx_base], r_hi - r_lo - 1u);
+      if (contiguous_index(columns[g].sy) < cy) {
+        lo = g + 1;
+        for (u32 step = 1;; step <<= 1) {
+          const u32 probe = lo + step - 1;
+          if (probe >= r_hi) { hi = r_hi; break; }
+          if (contiguous_index(columns[probe].sy) >= cy) { hi = probe; break; }
+          lo = probe + 1;
+        }
+      } else {
+        hi = g;
+        for (u32 step = 1;; step <<= 1) {
+          if (hi < r_lo + step) { lo = r_lo; break; }
+          const u32 probe = hi - step;
+          if (contiguous_index(columns[probe].sy) < cy) { lo = probe + 1; break; }
+          hi = probe;
+        }
+      }
+    }
+    while (lo < hi) {
+      const u32 mid = (lo + hi) >> 1;
+      if (contiguous_index(columns[mid].sy) < cy) lo = mid + 1; else hi = mid;
+    }
+    if (lo < r_hi) {
+      const gndt_column c = columns[lo];
+      if (contiguous_index(c.sy) == cy) visit(2 + dir, lo, c);
+    }
+  }
+}
+
 // K4b: one thread per column: extents, first-seen index (position in the reference's
 // morton_list, src/receiver.cpp:70), the x-row directory used by the edge search, and the
 // voxel ranges of the first and last x row (Ctl::first_row_end / last_row_begin) for the halo.
@@ -234,14 +302,9 @@ __global__ void column_finish_kernel(Ctl *ctl, const u32 *vfirst, gndt_column *c
     columns[c].voxel_count = v_end - col.voxel_begin;
     columns[c].slope_count = s_end - col.slope_begin;
     const int cx = contiguous_index(col.sx);
-    if (c == 0 || contiguous_index(columns[c - 1].sx) != cx) {
-      row_start[cx - cx_min] = c;
-      if (cx == cx_max) ctl->last_row_begin = col.voxel_begin;
-    }
-    if (c + 1 == C || contiguous_index(columns[c + 1].sx) != cx) {
-      row_end[cx - cx_min] = c + 1;
-      if (cx == cx_min) ctl->first_row_end = v_end;
-    }
+    const int ends = mark_row(columns, C, c, cx, cx_min, row_start, row_end);
+    if ((ends & 1) && cx == cx_max) ctl->last_row_begin = col.voxel_begin;
+    if ((ends & 2) && cx == cx_min) ctl->first_row_end = v_end;
   }
 }
 
@@ -286,73 +349,23 @@ __device__ __forceinline__ bool cell_reachable(const gndt_column &c, const gndt_
   return false;
 }
 
-// K5: one thread per Slope in [begin, begin+count): left/right = adjacent columns of the
-// same x row, forward/back = binary search for the same cy in the neighbouring x rows.
-// Index arithmetic is in contiguous space, which is countLRFB's quadrant crossing
-// (x==1 / y==1 cases, map2D.h:219-253) without the special cases.
+// K5: one thread per Slope in [begin, begin+count): one reach bit per neighbour cell that holds
+// a Slope reachable from it.
 __global__ void __launch_bounds__(256)
 edges_kernel(Ctl *ctl, gndt_voxel *table, gndt_slope *slopes, const gndt_column *columns, const u32 *slope_col,
              const u32 *row_start, const u32 *row_end, DevParams P) {
   pdl_wait();
   pdl_trigger();
   const u32 S = ctl->n_slopes, C = ctl->n_columns;
-  const int cx_base = ctl->cx_min, cx_max = ctl->cx_max;
+  const int cx_base = ctl->cx_min, n_rows = ctl->cx_max - cx_base + 1;
+  constexpr u32 kReach[4] = {GNDT_F_REACH_L, GNDT_F_REACH_R, GNDT_F_REACH_F, GNDT_F_REACH_B};
   for (u32 i = blockIdx.x * blockDim.x + threadIdx.x; i < S; i += gridDim.x * blockDim.x) {
     gndt_slope me = slopes[i];
-    const int cx = contiguous_index(me.sx), cy = contiguous_index(me.sy);
-    const u32 ci = slope_col[i];
     const float n[3] = {me.normal[0], me.normal[1], me.normal[2]};
     const double n_len = normal_length(n);
     u32 bits = 0;
-    if (ci > 0) {  // left: cy-1
-      const gndt_column c = columns[ci - 1];
-      if (contiguous_index(c.sx) == cx && contiguous_index(c.sy) == cy - 1 && cell_reachable(c, slopes, n, n_len, me.mean[2], P))
-        bits |= GNDT_F_REACH_L;
-    }
-    if (ci + 1 < C) {  // right: cy+1
-      const gndt_column c = columns[ci + 1];
-      if (contiguous_index(c.sx) == cx && contiguous_index(c.sy) == cy + 1 && cell_reachable(c, slopes, n, n_len, me.mean[2], P))
-        bits |= GNDT_F_REACH_R;
-    }
-#pragma unroll
-    for (int dir = 0; dir < 2; ++dir) {  // forward: cx+1, back: cx-1
-      const int ncx = cx + (dir == 0 ? 1 : -1);
-      if (ncx < cx_base || ncx > cx_max) continue;
-      // first column of the neighbour row with cy' >= cy.  Neighbouring rows of a map are
-      // populated alike, so the same offset as in the own row is a good first guess; gallop
-      // from it to bracket cy, then bisect the bracket (1-3 probes instead of log2(row)).
-      const u32 r_lo = row_start[ncx - cx_base], r_hi = row_end[ncx - cx_base];
-      u32 lo = r_lo, hi = r_hi;
-      if (r_lo < r_hi) {
-        const u32 g = r_lo + min(ci - row_start[cx - cx_base], r_hi - r_lo - 1u);
-        if (contiguous_index(columns[g].sy) < cy) {
-          lo = g + 1;
-          for (u32 step = 1;; step <<= 1) {
-            const u32 probe = lo + step - 1;
-            if (probe >= r_hi) { hi = r_hi; break; }
-            if (contiguous_index(columns[probe].sy) >= cy) { hi = probe; break; }
-            lo = probe + 1;
-          }
-        } else {
-          hi = g;
-          for (u32 step = 1;; step <<= 1) {
-            if (hi < r_lo + step) { lo = r_lo; break; }
-            const u32 probe = hi - step;
-            if (contiguous_index(columns[probe].sy) < cy) { lo = probe + 1; break; }
-            hi = probe;
-          }
-        }
-      }
-      while (lo < hi) {
-        const u32 mid = (lo + hi) >> 1;
-        if (contiguous_index(columns[mid].sy) < cy) lo = mid + 1; else hi = mid;
-      }
-      if (lo < row_end[ncx - cx_base]) {
-        const gndt_column c = columns[lo];
-        if (contiguous_index(c.sy) == cy && cell_reachable(c, slopes, n, n_len, me.mean[2], P))
-          bits |= (dir == 0 ? GNDT_F_REACH_F : GNDT_F_REACH_B);
-      }
-    }
+    neighbour_columns(columns, C, slope_col[i], contiguous_index(me.sx), contiguous_index(me.sy), row_start, row_end, cx_base, n_rows,
+                      [&](int d, u32, const gndt_column &c) { if (cell_reachable(c, slopes, n, n_len, me.mean[2], P)) bits |= kReach[d]; });
     if (bits) {
       slopes[i].flags = me.flags | bits;
       table[me.voxel].flags |= bits;

@@ -211,7 +211,8 @@ __global__ void __launch_bounds__(kNdtThreads) ndt_pass_kernel(const float *in, 
     for (int r = 0; r < 3; ++r)
       x[r] = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(P.r[3 * r], p[0]), __dmul_rn(P.r[3 * r + 1], p[1])), __dmul_rn(P.r[3 * r + 2], p[2])), P.t[r]);
     int cx, cy, cz;
-    if (!point_indices(__double2float_rn(x[0]), __double2float_rn(x[1]), __double2float_rn(x[2]), P.origin, P.grid_len, P.z_len, cx, cy, cz))
+    if (!point_indices<false>(__double2float_rn(x[0]), __double2float_rn(x[1]), __double2float_rn(x[2]), P.origin, P.grid_len, P.z_len,
+                              0.f, 0.f, cx, cy, cz))
       continue;
     const double y[3] = {x[0] - P.c[0], x[1] - P.c[1], x[2] - P.c[2]};
     const u32 before = A.pairs;

@@ -184,7 +184,7 @@ struct __align__(128) RedSmem {
 template <bool FAST>
 __device__ __forceinline__ u64 point_key(const float4 &p, const float o[3], const DevParams &P) {
   int cx, cy, cz;
-  point_indices_masked_t<FAST>(p.x, p.y, p.z, o, P, 7, cx, cy, cz);  // partitioned points are all valid
+  point_indices_masked<FAST>(p.x, p.y, p.z, o, P, 7, cx, cy, cz);  // partitioned points are all valid
   return voxel_key(cx, cy, cz);
 }
 

@@ -110,7 +110,7 @@ __global__ void __launch_bounds__(256) bounds_kernel(Ctl *ctl, u32 *zhist, const
     n_drop += (live && !ok) ? 1u : 0u;
     if (tiled && ok) {
       int cx;
-      axis_idx_t<FAST>(p.x, o[0], false, P, cx);
+      axis_index<FAST>(p.x, o[0], P.grid_len, P.rinv[0], cx);
       if (cx < P.tile_lo || cx >= P.tile_hi) { n_out++; ok = false; }
     }
     u32 d = kInvalidDigit;
@@ -118,11 +118,7 @@ __global__ void __launch_bounds__(256) bounds_kernel(Ctl *ctl, u32 *zhist, const
       n_ok++;
       lo_x = fminf(lo_x, p.x); lo_y = fminf(lo_y, p.y); lo_z = fminf(lo_z, p.z);
       hi_x = fmaxf(hi_x, p.x); hi_y = fmaxf(hi_y, p.y); hi_z = fmaxf(hi_z, p.z);
-      float cf = 1.f;  // valid points never exceed the index range: no range test here
-      if (FAST) { if (!(az < P.z_len)) cf = hoisted_div_ceil(az, P.z_len, P.rinv[1]); }
-      else cf = fmaxf(ceilf(__fdiv_rn(az, P.z_len)), 1.f);
-      const int n = (int)cf;
-      const int cz = (p.z > o[2]) ? n - 1 : -n;
+      const int cz = axis_index_valid<FAST>(p.z, o[2], P.z_len, P.rinv[1]);
       d = (u32)(cz + kIdxBias) & (u32)(kZHistBins - 1);
     }
     const u32 peers = __match_any_sync(0xffffffffu, d);  // flat scenes: most lanes share a z bin
@@ -167,7 +163,7 @@ __global__ void __launch_bounds__(256) bounds_kernel(Ctl *ctl, u32 *zhist, const
     for (int w = 1; w < 8; ++w) m = (tid < 3) ? fmaxf(m, red[tid][w]) : fminf(m, red[tid][w]);
     const int ax = tid % 3;
     int c;
-    axis_idx(m, o[ax], ax == 2, P, c);  // index of the extreme coordinate
+    axis_index<FAST>(m, o[ax], ax == 2 ? P.z_len : P.grid_len, ax == 2 ? P.rinv[1] : P.rinv[0], c);  // index of the extreme coordinate
     atomicMax(&ctl->max_cx_b + tid, (u32)((tid < 3 ? c : -c) + kIdxBias));
   }
   if (tid == 0) {
@@ -370,7 +366,7 @@ sort_pass_kernel(Ctl *ctl, int pass, const float *in_raw, size_t stride_f, size_
         const float4 e = S.in[i];
         int cx, cy, cz;
         if (FIRST) {
-          bool ok = point_indices_t<FAST>(e.x, e.y, e.z, o, P, cx, cy, cz);
+          bool ok = point_indices<FAST>(e.x, e.y, e.z, o, P.grid_len, P.z_len, P.rinv[0], P.rinv[1], cx, cy, cz);
           if (ok && tiled && (cx < P.tile_lo || cx >= P.tile_hi)) ok = false;
           if (ok) {
             const u64 key = compact_key(cx, cy, cz, L);
@@ -383,7 +379,7 @@ sort_pass_kernel(Ctl *ctl, int pass, const float *in_raw, size_t stride_f, size_
               }
           }
         } else {
-          point_indices_masked_t<FAST>(e.x, e.y, e.z, o, P, need, cx, cy, cz);
+          point_indices_masked<FAST>(e.x, e.y, e.z, o, P, need, cx, cy, cz);
           u64 key = 0;
           if (need_col) key = (u64)column_id(cx, cy, L) << L.bz;
           if (need_z) key |= (u64)(u32)(cz - L.cz_min);
