@@ -621,6 +621,7 @@ static int build_device(gndt_handle *h, const float *d_in, size_t n, size_t stri
   const size_t start = h->params.origin_is_first_point ? 1 : 0;
   const DevParams dp = make_dev(h, h->params, h->cap_voxels);
   h->ndt_ready = false;
+  h->g_valid = false;  // the graph indexes the slope table this build replaces
   GNDT_CUDA(h, cudaEventRecord(h->ev[EV_START], st));
   int rc = front_end(h, st, d_in, n, stride_bytes / 4, start, dp, (VoxMoments *)h->mom.p);
   if (rc != GNDT_OK) return rc;
@@ -761,6 +762,7 @@ static int fuse_scan(gndt_handle *h, const void *xyz, size_t n, size_t stride_by
   h->launches = 0;
   h->n_changed_valid = false;
   h->ndt_ready = false;  // recomputed by the next gndt_register whatever the verdict
+  h->g_valid = false;    // rebuilt by the next gndt_build_edges whatever the verdict
 
   // capacity: every scan point could open a new voxel
   size_t cap_vox = h->cap_voxels;
@@ -988,19 +990,25 @@ int gndt_build_edges(gndt_handle *h, const gndt_slope *slopes, size_t n_slopes, 
     if (!st) st = h->last_stream;
   }
   if (n_slopes > 0xFFFFFFFEull || n_columns > 0xFFFFFFFEull) return GNDT_ERR_CAPACITY;
+  if (n_slopes && !n_columns) { h->err = "gndt_build_edges: Slopes without a column table"; return GNDT_ERR_INVALID_ARG; }
   if (n_columns) {  // x range of the (sorted) column table
     gndt_column ends[2];
     GNDT_CUDA(h, cudaMemcpyAsync(&ends[0], columns, sizeof(gndt_column), cudaMemcpyDeviceToHost, st));
     GNDT_CUDA(h, cudaMemcpyAsync(&ends[1], columns + n_columns - 1, sizeof(gndt_column), cudaMemcpyDeviceToHost, st));
     GNDT_CUDA(h, cudaStreamSynchronize(st));
+    if (!valid_signed_index(ends[0].sx) || !valid_signed_index(ends[1].sx) || contiguous_index(ends[0].sx) > contiguous_index(ends[1].sx)) {
+      h->err = "gndt_build_edges: the first and last columns are not an x range of valid indices";
+      return GNDT_ERR_INVALID_ARG;
+    }
     cx_lo = contiguous_index(ends[0].sx);
     cx_hi = contiguous_index(ends[1].sx);
   }
   const int n_rows = cx_hi - cx_lo + 1;
   const u32 S = (u32)n_slopes, C = (u32)n_columns;
-  // work buffer: scan scratch | rows start/end (zeroed) | slope_col | deg
+  // work buffer: scan scratch | table check word | rows start/end (zeroed) | slope_col | deg
   Layout W;
   const ScanScratch sc(W, n_slopes);
+  const size_t o_bad = W.take(4);
   const size_t o_rs = W.take((size_t)n_rows * 4), o_re = W.take((size_t)n_rows * 4);
   const size_t zero_bytes = W.bytes;
   const size_t o_sc = W.take((n_slopes + 1) * 4), o_dg = W.take((n_slopes + 1) * 4);
@@ -1008,7 +1016,7 @@ int gndt_build_edges(gndt_handle *h, const gndt_slope *slopes, size_t n_slopes, 
   if ((rc = ensure(h, h->g_off, (n_slopes + 1) * 4)) != GNDT_OK) return rc;
   const Buffer &w = h->g_work;
   ScanCtl *g = at<ScanCtl>(w, sc.ctl);
-  u32 *rs = at<u32>(w, o_rs), *re = at<u32>(w, o_re), *slope_col = at<u32>(w, o_sc), *deg = at<u32>(w, o_dg);
+  u32 *rs = at<u32>(w, o_rs), *re = at<u32>(w, o_re), *slope_col = at<u32>(w, o_sc), *deg = at<u32>(w, o_dg), *bad = at<u32>(w, o_bad);
   GNDT_CUDA(h, cudaMemsetAsync(w.p, 0, zero_bytes, st));
   GNDT_CUDA(h, cudaMemsetAsync(h->g_off.p, 0, (n_slopes + 1) * 4, st));
   h->g_slopes = n_slopes;
@@ -1016,19 +1024,28 @@ int gndt_build_edges(gndt_handle *h, const gndt_slope *slopes, size_t n_slopes, 
   if (S && C) {
     const DevParams dp = make_dev(h, h->params, 0);
     const int grid_c = grid_for(h, C, 256, 8), grid_s = grid_for(h, S, 256, 8);
-    launch(h, false, graph_prepare_kernel, grid_c, 256, 0, st, columns, C, cx_lo, slope_col, rs, re);
+    launch(h, false, graph_prepare_kernel, grid_c, 256, 0, st, slopes, S, columns, C, cx_lo, cx_hi, slope_col, rs, re, bad);
     launch(h, false, graph_edges_kernel<false>, grid_s, 256, 0, st, slopes, S, columns, C, slope_col, rs, re, cx_lo, n_rows, deg, nullptr,
-           nullptr, dp);
+           nullptr, (const u32 *)bad, dp);
     launch(h, false, exclusive_scan_kernel, grid_for(h, (n_slopes + kScanTile - 1) / kScanTile, 1, 4), 256, 0, st, g, deg, S, nullptr,
            (u32 *)h->g_off.p, at<u64>(w, sc.state), at<GroupState>(w, sc.groups));
     ScanCtl hg;
+    u32 hbad = 0;
     GNDT_CUDA(h, cudaMemcpyAsync(&hg, g, sizeof(hg), cudaMemcpyDeviceToHost, st));
+    GNDT_CUDA(h, cudaMemcpyAsync(&hbad, bad, sizeof(hbad), cudaMemcpyDeviceToHost, st));
     GNDT_CUDA(h, cudaStreamSynchronize(st));
+    if (hbad) {
+      h->err = (hbad & kGraphBadIndex)   ? "gndt_build_edges: a column index is 0, beyond +-GNDT_MAX_INDEX or outside the table's x range"
+               : (hbad & kGraphBadOrder) ? "gndt_build_edges: the columns are not sorted strictly by (x, y)"
+               : (hbad & kGraphBadRange) ? "gndt_build_edges: the columns' slope ranges do not tile [0, n_slopes) in order"
+                                         : "gndt_build_edges: a Slope's (sx, sy) differs from its column's";
+      return GNDT_ERR_INVALID_ARG;
+    }
     if (hg.err) { h->err = "graph scan watchdog"; return GNDT_ERR_INTERNAL; }
     h->g_targets = hg.total;
     if ((rc = ensure(h, h->g_tgt, std::max<size_t>(hg.total, 1) * 4)) != GNDT_OK) return rc;
     launch(h, false, graph_edges_kernel<true>, grid_s, 256, 0, st, slopes, S, columns, C, slope_col, rs, re, cx_lo, n_rows, nullptr,
-           (const u32 *)h->g_off.p, (u32 *)h->g_tgt.p, dp);
+           (const u32 *)h->g_off.p, (u32 *)h->g_tgt.p, (const u32 *)bad, dp);
     GNDT_CUDA(h, cudaStreamSynchronize(st));
   }
   GNDT_CUDA(h, cudaGetLastError());

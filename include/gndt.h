@@ -299,10 +299,22 @@ int gndt_device_table_ptr(gndt_handle *h, const gndt_voxel **dptr, size_t *capac
  * neighbour cell.  slopes / columns: device tables to build from (e.g. the gathered tables of a
  * multi-GPU map), or both NULL for this handle's own map.  Synchronises the stream.
  * adapter/gndt_twodmap_adapter.h (SlopeGraph) serves the planner from it.
+ * Caller tables must have the layout of this library's own tables; the call checks it on the device
+ * and returns GNDT_ERR_INVALID_ARG, naming the broken rule, when
+ *   - a column's sx / sy is 0 or outside [-GNDT_MAX_INDEX, GNDT_MAX_INDEX],
+ *   - the columns are not sorted strictly by (x, y) in contiguous index order,
+ *   - the slope ranges [slope_begin, slope_begin + slope_count) do not follow each other from 0
+ *     and end at n_slopes (n_slopes > 0 with n_columns == 0 included),
+ *   - a Slope's (sx, sy) is not its column's.
+ * A rejected call leaves no graph (gndt_copy_edges then returns GNDT_ERR_STATE).
+ * A gndt_build / gndt_build_msg / gndt_update / gndt_remove on the handle invalidates the graph it
+ * holds, whatever its verdict: the targets index the slope table that call replaces.
  */
 int gndt_build_edges(gndt_handle *h, const gndt_slope *slopes, size_t n_slopes, const gndt_column *columns,
                      size_t n_columns, void *stream);
-/* offsets: n_slopes + 1 entries, targets: n_targets entries.  offsets == targets == NULL: size query only. */
+/* offsets: n_slopes + 1 entries, targets: n_targets entries.  offsets == targets == NULL: size query only.
+ * GNDT_ERR_STATE when the handle holds no valid graph (no gndt_build_edges since the last build,
+ * update or remove, or the last one failed); GNDT_ERR_CAPACITY when a destination is too small. */
 int gndt_copy_edges(gndt_handle *h, uint32_t *offsets, size_t cap_offsets, uint32_t *targets, size_t cap_targets,
                     int dst_mem, size_t *n_slopes, size_t *n_targets);
 

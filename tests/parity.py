@@ -191,6 +191,14 @@ def compare(gpu_vox, gpu_cols, gpu_slopes, gpu_counts, o32, o64, params, check_r
         if rb.size != rep["reach_mismatch_threshold_adjacent"]:
             fail(f"reach bits: {rb.size - rep['reach_mismatch_threshold_adjacent']} mismatches are NOT threshold-adjacent")
 
+    # ---- reach bits of the GPU's own tables against the exact rule (tests/graph_reference.py): the
+    # oracle comparison above allows threshold-adjacent differences because the normals differ
+    # legitimately; on its own Slopes, edges_kernel must decide every decided edge exactly
+    from tests import graph_reference
+    errs, rep["reach_undecided_own"] = graph_reference.reach_bit_errors(gpu_slopes, params, gpu_cols)
+    for e in errs:
+        fail(f"reach bits against the GPU's own tables: {e}")
+
     # column slope_begin / slope_count follow from the labels: with identical labels they must be identical
     if rep["label_mismatch"] == 0 and (rep.get("col_slope_begin_mismatch", 0) or rep.get("col_slope_count_mismatch", 0)):
         fail(f"column slope_begin/slope_count differ ({rep['col_slope_begin_mismatch']}/{rep['col_slope_count_mismatch']}) although all labels agree")

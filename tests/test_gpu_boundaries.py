@@ -612,7 +612,7 @@ def test_reach_params(kw, demand):
     _gpu()
     from oracle import oracle as O
     from tests import parity
-    from tests.test_gpu_graph import _rows
+    from tests import graph_reference as G
     cloud = _param_cloud()
     p = default_params(GL, ZL, SI, demand, **kw)
     _parity(cloud, p, demand)
@@ -622,11 +622,12 @@ def test_reach_params(kw, demand):
     o = O.oracle_build(cloud, p)
     ooff, otgt = O.oracle_edges(o, p)
     assert np.array_equal(m.voxels["flags"] & parity.LABEL_BITS, o.voxels["flags"] & parity.LABEL_BITS)
-    got, want = _rows(off, tgt), _rows(ooff, otgt)
+    got, want = G.rows(off, tgt), G.rows(ooff, otgt)
     assert len(got) == len(want)
     bad = [i for i in range(len(got)) if got[i] != want[i]]
     if bad:  # a differing list must come from an edge within 1e-5 of a threshold
         assert parity._reach_adjacent(m.slopes["voxel"][bad], o.voxels, o.columns, p) == len(bad)
+    G.assert_graph(off, tgt, m.slopes, m.columns, p, f"{kw} {demand}: ")  # exact on the GPU's own tables
     m.close()
 
 

@@ -742,8 +742,7 @@ def test_multi_front_door_on_one_gpu():
 
 @pytest.mark.gpu
 def test_graph_from_gathered_tables():
-    from oracle import oracle as O
-    from tests import parity
+    from tests import graph_reference as G
     _gpu()
     from grid_ndt_b200 import TwoDmap
     cloud = _plan_cloud()
@@ -762,15 +761,7 @@ def test_graph_from_gathered_tables():
     uoff, utgt = m.edges()
     m.close()
     assert np.array_equal(off, uoff) and np.array_equal(tgt, utgt), "graph of the gathered tables differs from the untiled graph"
-    o = _oracle(cloud)
-    ooff, otgt = O.oracle_edges(o, _params())
-    rows = lambda a, b: [tuple(b[a[i]:a[i + 1]]) for i in range(len(a) - 1)]
-    got, want = rows(off, tgt), rows(ooff, otgt)
-    assert len(got) == len(want)
-    bad = [i for i in range(len(got)) if got[i] != want[i]]
-    if bad:
-        adj = parity._reach_adjacent(t["slopes"]["voxel"][bad], o.voxels, o.columns, _params())
-        assert adj == len(bad), f"{len(bad)} neighbour lists differ, only {adj} are threshold-adjacent"
+    G.assert_graph(off, tgt, t["slopes"], t["columns"], _params(), "gathered: ")
     sl = t["slopes"]
     cx = _contig(sl["sx"]).astype(np.int64)
     src = np.repeat(np.arange(len(sl)), np.diff(off.astype(np.int64)))

@@ -1,7 +1,8 @@
-"""The traversability graph built on the GPU (gndt_build_edges, csrc/gndt_graph.cuh) against the
-oracle's restatement of TwoDmap::AccessibleNeighbors (oracle/gndt_oracle.c, itself pinned against
-the reference's own code in tests/test_adapter.py): same lists, same order, for every Slope; the
-4 reach bits are exactly "the list has a Slope in that direction"."""
+"""The traversability graph built on the GPU (gndt_build_edges, csrc/gndt_graph.cuh) on synthetic
+clouds, held to the exact rule of tests/graph_reference.py on the GPU's own tables: same lists, same
+order, for every Slope, up to edges whose angle test acosf's 2-ulp freedom leaves undecided.  The
+reference itself is pinned to the oracle's AccessibleNeighbors in test_gpu_graph_boundaries.py.
+The 4 reach bits are exactly "the list has a Slope in that direction"."""
 import numpy as np
 import pytest
 
@@ -9,10 +10,6 @@ from grid_ndt_b200 import _abi, synthetic
 from grid_ndt_b200._abi import default_params
 
 pytestmark = pytest.mark.gpu
-
-
-def _rows(off, tgt):
-    return [tuple(tgt[off[i]:off[i + 1]]) for i in range(len(off) - 1)]
 
 
 @pytest.mark.parametrize("name,n,gl,kw,demand", [
@@ -26,25 +23,16 @@ def test_graph_equals_oracle(name, n, gl, kw, demand):
     if not torch.cuda.is_available():
         pytest.fail("gpu-marked test on a box without CUDA (no fallback exists)")
     from grid_ndt_b200 import TwoDmap
-    from oracle import oracle as O
-    from tests import parity
+    from tests import graph_reference as G
     cloud = synthetic.make(name, n, **kw)
     p = default_params(gl, 0.1, 0.08, demand)
     m = TwoDmap(gl, 0.1)
     m.setInterval(0.08)
     m.chatterCallback(cloud, demand)
     off, tgt = m.edges()
-    vox, sl = m.voxels, m.slopes
-    o = O.oracle_build(cloud, p)
-    ooff, otgt = O.oracle_edges(o, p)
-    assert np.array_equal(vox["flags"] & parity.LABEL_BITS, o.voxels["flags"] & parity.LABEL_BITS), "labels differ: pick another cloud"
-    assert len(off) == len(ooff) == len(sl) + 1
-    got, want = _rows(off, tgt), _rows(ooff, otgt)
-    bad = [i for i in range(len(got)) if got[i] != want[i]]
-    # a differing list must come from an edge within 1e-5 of a threshold (same rule as the reach bits)
-    if bad:
-        adj = parity._reach_adjacent(sl["voxel"][bad], o.voxels, o.columns, p)
-        assert adj == len(bad), f"{len(bad)} neighbour lists differ, only {adj} are threshold-adjacent"
+    sl, cols = m.slopes, m.columns
+    assert len(off) == len(sl) + 1
+    G.assert_graph(off, tgt, sl, cols, p, f"{name} {demand}: ")
     # reach bits <=> a target in that direction's cell
     cont = lambda s: np.where(s > 0, s - 1, s)
     cx, cy = cont(sl["sx"]).astype(np.int64), cont(sl["sy"]).astype(np.int64)
@@ -57,5 +45,4 @@ def test_graph_equals_oracle(name, n, gl, kw, demand):
         np.bitwise_or.at(bits, src[sel], np.uint32(mask))
     assert np.all((np.abs(dx) + np.abs(dy)) == 1), "a target outside the 4-neighbourhood"
     assert np.array_equal(bits, sl["flags"] & _abi.F_REACH_ALL), "reach bits disagree with the graph"
-    print(f"\n{name} {demand}: {len(sl)} slopes, {len(tgt)} edges, {len(bad)} threshold-adjacent list differences")
     m.close()

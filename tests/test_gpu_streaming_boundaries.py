@@ -101,10 +101,10 @@ def _tables(m):
 
 def _check_edges(m, o, p):
     from oracle import oracle as O
-    from tests.test_gpu_graph import _rows
+    from tests.graph_reference import rows
     off, tgt = m.edges()
     ooff, otgt = O.oracle_edges(o, p)
-    assert _rows(off, tgt) == _rows(ooff, otgt)
+    assert rows(off, tgt) == rows(ooff, otgt)
 
 
 # ---- 1. U1 match / U3 new keys --------------------------------------------------------------
