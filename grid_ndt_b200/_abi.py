@@ -162,6 +162,26 @@ def default_ndt_params(**kw) -> NdtParams:
     return p
 
 
+NDT_MAX_LEVELS = 8
+
+
+class NdtLevel(C.Structure):
+    """gndt_ndt_level (include/gndt.h): one coarse level of gndt_register_levels."""
+
+    _fields_ = [("factor", C.c_int32), ("max_iterations", C.c_int32), ("translation_epsilon", C.c_double),
+                ("rotation_epsilon", C.c_double)]
+
+
+def default_ndt_level(factor, **kw) -> NdtLevel:
+    """gndt_default_ndt_level(factor) with any field overridden by keyword."""
+    lv = NdtLevel(int(factor), 50, 1e-3, 1e-3)
+    for k, v in kw.items():
+        if k == "factor" or k not in dict(NdtLevel._fields_):
+            raise TypeError(f"unknown NDT level field {k!r}")
+        setattr(lv, k, v)
+    return lv
+
+
 class Registration(C.Structure):
     """gndt_registration (include/gndt.h): result of gndt_register."""
 

@@ -5,7 +5,7 @@ import os
 import subprocess
 import sys
 
-from ._abi import Counts, NdtParams, Params, PointCloud2, Registration, XchgInfo, XchgView
+from ._abi import Counts, NdtLevel, NdtParams, Params, PointCloud2, Registration, XchgInfo, XchgView
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(HERE)
@@ -98,6 +98,9 @@ SYMBOLS = {
     "gndt_origin": (_i, [_vp, C.POINTER(C.c_float)]),
     "gndt_default_ndt_params": (None, [C.POINTER(NdtParams)]),
     "gndt_register": (_i, [_vp, _vp, _sz, _sz, _i, C.POINTER(C.c_double), C.POINTER(NdtParams), C.POINTER(Registration), _vp]),
+    "gndt_default_ndt_level": (None, [C.POINTER(NdtLevel), C.c_int32]),
+    "gndt_register_levels": (_i, [_vp, _vp, _sz, _sz, _i, C.POINTER(C.c_double), C.POINTER(NdtParams), C.POINTER(NdtLevel), _i,
+                                  C.POINTER(Registration), C.POINTER(Registration), _vp]),
     "gndt_key_layout": (_i, [_vp, C.POINTER(C.c_int)]),
     "gndt_find_column": (C.c_int64, [_vp, _sz, C.c_int32, C.c_int32]),
     "gndt_find_slope": (C.c_int64, [_vp, _sz, _vp, C.c_int32, C.c_int32, C.c_int32]),

@@ -204,12 +204,17 @@ class TwoDmap:
         self._views.clear()
         return True
 
-    def register(self, scan, guess=None, stream: Optional[int] = None, **ndt) -> dict:
+    def register(self, scan, guess=None, stream: Optional[int] = None, levels=None, **ndt) -> dict:
         """NDT registration of a scan against the resident map (gndt_register): the pose
         map <- scan that best fits it, from `guess` (4x4, identity when None).  Keywords set
         gndt_ndt_params fields (outlier_ratio, min_voxel_points, max_iterations,
         translation_epsilon, rotation_epsilon).  Returns the gndt_registration fields as a dict;
-        pose is a 4x4 float64 array, termination one of _abi.NDT_*.  The map is not changed."""
+        pose is a 4x4 float64 array, termination one of _abi.NDT_*.  The map is not changed.
+
+        levels: coarse-to-fine registration (gndt_register_levels) when not None: a sequence of
+        factors, coarsest first, or of dicts with "factor" and any gndt_ndt_level field
+        (max_iterations, translation_epsilon, rotation_epsilon); the other fields keep their
+        defaults.  The result then has "levels": one dict per level, in the same shape."""
         ptr, n, stride, mem, st, keep = self._marshal(scan)
         if stream is not None:
             st = stream
@@ -218,9 +223,17 @@ class TwoDmap:
             raise GndtError(-1, "guess must be a 4x4 matrix")
         np_ = _abi.default_ndt_params(**ndt)
         out = _abi.Registration()
-        _check(self._h, lib().gndt_register(self._h, ptr, n, stride, mem, T.ctypes.data_as(C.POINTER(C.c_double)),
-                                            C.byref(np_), C.byref(out), st))
-        return out.as_dict()
+        Tp = T.ctypes.data_as(C.POINTER(C.c_double))
+        if levels is None:
+            _check(self._h, lib().gndt_register(self._h, ptr, n, stride, mem, Tp, C.byref(np_), C.byref(out), st))
+            return out.as_dict()
+        lv = [_abi.default_ndt_level(**l) if isinstance(l, dict) else _abi.default_ndt_level(l) for l in levels]
+        arr = (_abi.NdtLevel * max(len(lv), 1))(*lv)
+        per = (_abi.Registration * max(len(lv), 1))()
+        _check(self._h, lib().gndt_register_levels(self._h, ptr, n, stride, mem, Tp, C.byref(np_), arr, len(lv), C.byref(out), per, st))
+        res = out.as_dict()
+        res["levels"] = [per[i].as_dict() for i in range(len(lv))]
+        return res
 
     @property
     def changed_columns(self) -> np.ndarray:

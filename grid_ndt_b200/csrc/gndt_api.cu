@@ -111,6 +111,10 @@ struct gndt_handle {
   Buffer ndt_vox, ndt_pts, ndt_part;
   double *ndt_host = nullptr;  // pinned read-back of one pass
   bool ndt_ready = false;      // ndt_vox describes the resident map (cleared by build / update / remove)
+  // coarse levels of gndt_register_levels, by factor: Gaussians, coarse column table, its length
+  struct NdtLevel { Buffer vox, cols; u32 n_cols = 0; } ndt_lv[kNdtMaxFactor + 1];
+  uint64_t ndt_lv_ready = 0;   // bit k: ndt_lv[k] describes the resident map (cleared with ndt_ready)
+  Buffer ndt_lv_work;          // scratch of a level build
   // peer-mapped strip exchange (gndt_xchg_*)
   Buffer xbuf;
   XLayout xl = {};
@@ -600,8 +604,9 @@ int gndt_destroy(gndt_handle *h) {
   if (h->ring) { cudaFreeHost(h->ring); for (int i = 0; i < 4; ++i) if (h->ring_ev[i]) cudaEventDestroy(h->ring_ev[i]); }
   Buffer *bufs[] = {&h->in_stage, &h->buf_a, &h->buf_b, &h->zero, &h->mom, &h->mom_alt, &h->table, &h->slopes,
                     &h->columns, &h->vfirst, &h->slope_col, &h->mom_scan, &h->upd_work, &h->msg_points, &h->small, &h->lookback, &h->f_zero, &h->xbuf, &h->g_work, &h->g_off, &h->g_tgt,
-                    &h->ndt_vox, &h->ndt_pts, &h->ndt_part};
+                    &h->ndt_vox, &h->ndt_pts, &h->ndt_part, &h->ndt_lv_work};
   for (Buffer *b : bufs) if (b->p) cudaFree(b->p);
+  for (auto &l : h->ndt_lv) { if (l.vox.p) cudaFree(l.vox.p); if (l.cols.p) cudaFree(l.cols.p); }
   for (int i = 0; i < EV_COUNT; ++i) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
   delete h;
   return GNDT_OK;
@@ -621,6 +626,7 @@ static int build_device(gndt_handle *h, const float *d_in, size_t n, size_t stri
   const size_t start = h->params.origin_is_first_point ? 1 : 0;
   const DevParams dp = make_dev(h, h->params, h->cap_voxels);
   h->ndt_ready = false;
+  h->ndt_lv_ready = 0;
   h->g_valid = false;  // the graph indexes the slope table this build replaces
   GNDT_CUDA(h, cudaEventRecord(h->ev[EV_START], st));
   int rc = front_end(h, st, d_in, n, stride_bytes / 4, start, dp, (VoxMoments *)h->mom.p);
@@ -762,6 +768,7 @@ static int fuse_scan(gndt_handle *h, const void *xyz, size_t n, size_t stride_by
   h->launches = 0;
   h->n_changed_valid = false;
   h->ndt_ready = false;  // recomputed by the next gndt_register whatever the verdict
+  h->ndt_lv_ready = 0;
   h->g_valid = false;    // rebuilt by the next gndt_build_edges whatever the verdict
 
   // capacity: every scan point could open a new voxel
@@ -1739,15 +1746,96 @@ int ndt_check_args(gndt_handle *h, const double *T, const gndt_ndt_params *np) {
   return GNDT_OK;
 }
 
-}  // namespace
+// The tables of the level of factor k (gndt.h, gndt_register_levels), once per map state and factor:
+// coarse columns by slab (count, scan, emit), then coarse voxels by coarse column (count, scan,
+// emit).  Two read-backs: the map's first and last column (the slab range) and the coarse column
+// count.
+int ndt_build_level(gndt_handle *h, int k, cudaStream_t st) {
+  gndt_handle::NdtLevel &L = h->ndt_lv[k];
+  const u32 n_vox = h->host_ctl.n_voxels, n_cols = h->host_ctl.n_columns;
+  int rc;
+  if ((rc = ensure(h, L.vox, std::max<size_t>(n_vox, 1) * sizeof(NdtVoxel))) != GNDT_OK) return rc;
+  if ((rc = ensure(h, L.cols, std::max<size_t>(n_cols, 1) * sizeof(gndt_column))) != GNDT_OK) return rc;
+  L.n_cols = 0;
+  if (n_cols) {
+    const gndt_column *cols = (const gndt_column *)h->columns.p;
+    gndt_column ends[2];
+    GNDT_CUDA(h, cudaMemcpyAsync(&ends[0], cols, sizeof(gndt_column), cudaMemcpyDeviceToHost, st));
+    GNDT_CUDA(h, cudaMemcpyAsync(&ends[1], cols + n_cols - 1, sizeof(gndt_column), cudaMemcpyDeviceToHost, st));
+    GNDT_CUDA(h, cudaStreamSynchronize(st));
+    const int X0 = floor_div(contiguous_index(ends[0].sx), k), X1 = floor_div(contiguous_index(ends[1].sx), k);
+    const u32 n_slabs = (u32)(X1 - X0 + 1);
+    // work: scan scratch of the slabs | of the coarse columns (zeroed) | slab counts, offsets | members | voxel counts, offsets
+    Layout W;
+    const ScanScratch s1(W, n_slabs), s2(W, n_cols);
+    const size_t zero_bytes = W.bytes;
+    const size_t o_sc = W.take((size_t)n_slabs * 4), o_sb = W.take(((size_t)n_slabs + 1) * 4), o_m = W.take((size_t)n_cols * 4);
+    const size_t o_vc = W.take((size_t)n_cols * 4), o_vb = W.take(((size_t)n_cols + 1) * 4);
+    if ((rc = ensure(h, h->ndt_lv_work, W.bytes)) != GNDT_OK) return rc;
+    const Buffer &w = h->ndt_lv_work;
+    u32 *slab_count = at<u32>(w, o_sc), *slab_begin = at<u32>(w, o_sb), *members = at<u32>(w, o_m);
+    u32 *vcount = at<u32>(w, o_vc), *vbegin = at<u32>(w, o_vb);
+    gndt_column *ccols = (gndt_column *)L.cols.p;
+    GNDT_CUDA(h, cudaMemsetAsync(w.p, 0, zero_bytes, st));
+    const int g_slab = (int)(((size_t)n_slabs * 32 + 255) / 256);
+    launch(h, false, ndt_level_columns_kernel<false>, g_slab, 256, 0, st, cols, n_cols, k, X0, n_slabs, slab_count, (const u32 *)nullptr,
+           ccols, members);
+    launch(h, false, exclusive_scan_kernel, grid_for(h, (n_slabs + kScanTile - 1) / kScanTile, 1, 4), 256, 0, st, at<ScanCtl>(w, s1.ctl),
+           (const u32 *)slab_count, n_slabs, (const u32 *)nullptr, slab_begin, at<u64>(w, s1.state), at<GroupState>(w, s1.groups));
+    launch(h, false, ndt_level_columns_kernel<true>, g_slab, 256, 0, st, cols, n_cols, k, X0, n_slabs, (u32 *)nullptr,
+           (const u32 *)slab_begin, ccols, members);
+    ScanCtl hs;
+    GNDT_CUDA(h, cudaGetLastError());
+    GNDT_CUDA(h, cudaMemcpyAsync(&hs, at<ScanCtl>(w, s1.ctl), sizeof(hs), cudaMemcpyDeviceToHost, st));
+    GNDT_CUDA(h, cudaStreamSynchronize(st));
+    if (hs.err) { h->err = "level column scan watchdog"; return GNDT_ERR_INTERNAL; }
+    const u32 nc = hs.total;
+    const int g_col = grid_for(h, nc, 256, 8);
+    const gndt_voxel *table = (const gndt_voxel *)h->table.p;
+    launch(h, false, ndt_level_voxels_kernel<false>, g_col, 256, 0, st, table, cols, (const u32 *)members, k, h->res_params.normalize_cov,
+           ccols, nc, vcount, (const u32 *)nullptr, (NdtVoxel *)nullptr);
+    launch(h, false, exclusive_scan_kernel, grid_for(h, (nc + kScanTile - 1) / kScanTile, 1, 4), 256, 0, st, at<ScanCtl>(w, s2.ctl),
+           (const u32 *)vcount, nc, (const u32 *)nullptr, vbegin, at<u64>(w, s2.state), at<GroupState>(w, s2.groups));
+    launch(h, false, ndt_level_voxels_kernel<true>, g_col, 256, 0, st, table, cols, (const u32 *)members, k, h->res_params.normalize_cov,
+           ccols, nc, (u32 *)nullptr, (const u32 *)vbegin, (NdtVoxel *)L.vox.p);
+    GNDT_CUDA(h, cudaGetLastError());
+    GNDT_CUDA(h, cudaMemcpyAsync(&hs, at<ScanCtl>(w, s2.ctl), sizeof(hs), cudaMemcpyDeviceToHost, st));
+    GNDT_CUDA(h, cudaStreamSynchronize(st));
+    if (hs.err) { h->err = "level voxel scan watchdog"; return GNDT_ERR_INTERNAL; }
+    L.n_cols = nc;
+  }
+  h->ndt_lv_ready |= 1ull << k;
+  return GNDT_OK;
+}
 
-int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, const double guess[16],
-                  const gndt_ndt_params *np, gndt_registration *out, void *stream) {
+int ndt_check_levels(gndt_handle *h, const gndt_ndt_level *levels, int n_levels) {
+  if (n_levels < 0 || n_levels > GNDT_NDT_MAX_LEVELS || (n_levels > 0 && !levels)) {
+    h->err = "gndt_register_levels: n_levels outside [0, GNDT_NDT_MAX_LEVELS] or levels is NULL";
+    return GNDT_ERR_INVALID_ARG;
+  }
+  for (int i = 0; i < n_levels; ++i) {
+    const gndt_ndt_level &l = levels[i];
+    if (l.factor < 2 || l.factor > kNdtMaxFactor || (i > 0 && l.factor >= levels[i - 1].factor) || l.max_iterations < 0 ||
+        !(l.translation_epsilon >= 0.0) || !(l.rotation_epsilon >= 0.0) || !std::isfinite(l.translation_epsilon) ||
+        !std::isfinite(l.rotation_epsilon)) {
+      h->err = "gndt_register_levels: level " + std::to_string(i) + " out of range (factor in [2, 32] and strictly decreasing, "
+               "max_iterations >= 0, epsilons finite and >= 0)";
+      return GNDT_ERR_INVALID_ARG;
+    }
+  }
+  return GNDT_OK;
+}
+
+int register_levels(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, const double guess[16],
+                    const gndt_ndt_params *np, const gndt_ndt_level *levels, int n_levels, gndt_registration *out,
+                    gndt_registration *level_out, void *stream) {
+  const char *who = levels ? "gndt_register_levels" : "gndt_register";
   if (!h) return GNDT_ERR_INVALID_ARG;
-  if (!guess || !np || !out) { h->err = "gndt_register: guess, np and out must not be NULL"; return GNDT_ERR_INVALID_ARG; }
-  int rc = check_cloud_args(h, xyz, n, stride_bytes, mem, "gndt_register");
+  if (!guess || !np || !out) { h->err = std::string(who) + ": guess, np and out must not be NULL"; return GNDT_ERR_INVALID_ARG; }
+  int rc = check_cloud_args(h, xyz, n, stride_bytes, mem, who);
   if (rc != GNDT_OK) return rc;
   if ((rc = ndt_check_args(h, guess, np)) != GNDT_OK) return rc;
+  if ((rc = ndt_check_levels(h, levels, n_levels)) != GNDT_OK) return rc;
   GNDT_CUDA(h, cudaSetDevice(h->device));
   if ((rc = sync_counts(h)) != GNDT_OK) return rc;  // resolves a pending update / remove
   KeepLaunchCount keep(h);
@@ -1755,12 +1843,14 @@ int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes
   const gndt_params &rp = h->res_params;
   const u32 n_vox = h->host_ctl.n_voxels, n_cols = h->host_ctl.n_columns;
 
-  // the resident map's Gaussians, once per map state
+  // the resident map's Gaussians, once per map state; each level's, once per map state and factor
   if (!h->ndt_ready) {
     if ((rc = ensure(h, h->ndt_vox, std::max<size_t>(n_vox, 1) * sizeof(NdtVoxel))) != GNDT_OK) return rc;
     launch(h, false, ndt_prepare_kernel, grid_for(h, n_vox, 256, 8), 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p,
            (NdtVoxel *)h->ndt_vox.p, rp.normalize_cov);
   }
+  for (int i = 0; i < n_levels; ++i)
+    if (!(h->ndt_lv_ready >> levels[i].factor & 1) && (rc = ndt_build_level(h, levels[i].factor, st)) != GNDT_OK) return rc;
   const float *d_in;
   if ((rc = upload(h, h->ndt_pts, xyz, n * stride_bytes, mem, st, nullptr, &d_in)) != GNDT_OK) return rc;
   const int blocks = grid_for(h, n, kNdtThreads, 8);
@@ -1780,113 +1870,159 @@ int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes
   const double pbar[3] = {n_points ? h->ndt_host[0] / (double)n_points : 0.0, n_points ? h->ndt_host[1] / (double)n_points : 0.0,
                           n_points ? h->ndt_host[2] / (double)n_points : 0.0};
 
-  NdtPose P = {};
-  {
-    const double p_o = np->outlier_ratio, V = (double)rp.grid_len * (double)rp.grid_len * (double)rp.z_len;
-    const double c1 = 10.0 * (1.0 - p_o), c2 = p_o / V, d3 = -std::log(c2);
-    P.d1 = -std::log(c1 + c2) - d3;
-    P.d2 = -2.0 * std::log((-std::log(c1 * std::exp(-0.5) + c2) - d3) / P.d1);
-  }
-  for (int i = 0; i < 3; ++i) P.origin[i] = h->host_ctl.origin[i];
-  P.grid_len = rp.grid_len;
-  P.z_len = rp.z_len;
-  P.min_points = (u32)np->min_voxel_points;
-
-  auto eval = [&](const double T[16], NdtEval &e) -> int {
-    for (int i = 0; i < 3; ++i) {
-      for (int j = 0; j < 3; ++j) P.r[3 * i + j] = T[4 * i + j];
-      P.t[i] = T[4 * i + 3];
-      P.c[i] = T[4 * i] * pbar[0] + T[4 * i + 1] * pbar[1] + T[4 * i + 2] * pbar[2] + T[4 * i + 3];
+  // Levenberg-Marquardt on one level (factor 1: the map) from T_in -> *res
+  auto solve = [&](int factor, const NdtVoxel *vox, const gndt_column *cols, u32 nc, int max_iterations, double teps, double reps,
+                   const double T_in[16], gndt_registration *res) -> int {
+    NdtPose P = {};
+    {
+      const double p_o = np->outlier_ratio, kg = (double)factor * (double)rp.grid_len, kz = (double)factor * (double)rp.z_len;
+      const double V = kg * kg * kz;
+      const double c1 = 10.0 * (1.0 - p_o), c2 = p_o / V, d3 = -std::log(c2);
+      P.d1 = -std::log(c1 + c2) - d3;
+      P.d2 = -2.0 * std::log((-std::log(c1 * std::exp(-0.5) + c2) - d3) / P.d1);
     }
-    launch(h, false, ndt_pass_kernel, blocks, kNdtThreads, 0, st, d_in, stride_f, n, (const NdtVoxel *)h->ndt_vox.p,
-           (const gndt_column *)h->columns.p, n_cols, P, part);
-    launch(h, false, ndt_finish_kernel, 1, 32, 0, st, part, blocks, kNdtWidth, dres);
-    GNDT_CUDA(h, cudaGetLastError());
-    GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_host, dres, kNdtWidth * sizeof(double), cudaMemcpyDeviceToHost, st));
-    GNDT_CUDA(h, cudaStreamSynchronize(st));
-    const double *r = h->ndt_host;
-    e.score = r[0];
-    for (int k = 0; k < 6; ++k) e.g[k] = r[1 + k];
-    for (int k = 0, idx = 7; k < 6; ++k)
-      for (int l = k; l < 6; ++l, ++idx) e.H[6 * k + l] = e.H[6 * l + k] = r[idx];
-    for (int i = 0; i < 3; ++i) e.c[i] = P.c[i];
-    e.n_points = (uint64_t)r[28];
-    e.n_matched = (uint64_t)r[29];
-    e.n_pairs = (uint64_t)r[30];
+    for (int i = 0; i < 3; ++i) P.origin[i] = h->host_ctl.origin[i];
+    P.grid_len = rp.grid_len;
+    P.z_len = rp.z_len;
+    P.min_points = (u32)np->min_voxel_points;
+    P.factor = factor;
+
+    auto eval = [&](const double T[16], NdtEval &e) -> int {
+      for (int i = 0; i < 3; ++i) {
+        for (int j = 0; j < 3; ++j) P.r[3 * i + j] = T[4 * i + j];
+        P.t[i] = T[4 * i + 3];
+        P.c[i] = T[4 * i] * pbar[0] + T[4 * i + 1] * pbar[1] + T[4 * i + 2] * pbar[2] + T[4 * i + 3];
+      }
+      launch(h, false, ndt_pass_kernel, blocks, kNdtThreads, 0, st, d_in, stride_f, n, vox, cols, nc, P, part);
+      launch(h, false, ndt_finish_kernel, 1, 32, 0, st, part, blocks, kNdtWidth, dres);
+      GNDT_CUDA(h, cudaGetLastError());
+      GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_host, dres, kNdtWidth * sizeof(double), cudaMemcpyDeviceToHost, st));
+      GNDT_CUDA(h, cudaStreamSynchronize(st));
+      const double *r = h->ndt_host;
+      e.score = r[0];
+      for (int k = 0; k < 6; ++k) e.g[k] = r[1 + k];
+      for (int k = 0, idx = 7; k < 6; ++k)
+        for (int l = k; l < 6; ++l, ++idx) e.H[6 * k + l] = e.H[6 * l + k] = r[idx];
+      for (int i = 0; i < 3; ++i) e.c[i] = P.c[i];
+      e.n_points = (uint64_t)r[28];
+      e.n_matched = (uint64_t)r[29];
+      e.n_pairs = (uint64_t)r[30];
+      return GNDT_OK;
+    };
+
+    double T[16];
+    memcpy(T, T_in, sizeof(T));
+    NdtEval cur;
+    int rc = eval(T, cur);
+    if (rc != GNDT_OK) return rc;
+    int term = GNDT_NDT_MAX_ITER;
+    uint32_t iters = 0;
+    if (cur.n_pairs == 0) {
+      term = GNDT_NDT_NO_MATCH;
+      cur.score = 0.0;
+      memset(cur.g, 0, sizeof(cur.g));
+      memset(cur.H, 0, sizeof(cur.H));
+    } else {
+      // Levenberg-Marquardt on -S: (-H + lambda diag(max(-H_ii, tiny))) delta = g
+      constexpr double kLambda0 = 1e-3, kLambdaMin = 1e-12, kLambdaMax = 1e12;
+      double lambda = kLambda0;
+      while (iters < (uint32_t)max_iterations) {
+        double hmax = 0.0;
+        for (int i = 0; i < 6; ++i) hmax = std::max(hmax, std::fabs(cur.H[7 * i]));
+        const double tiny = std::max(1e-6 * hmax, 1e-300);
+        double A[36], delta[6];
+        for (int i = 0; i < 36; ++i) A[i] = -cur.H[i];
+        for (int i = 0; i < 6; ++i) A[7 * i] += lambda * std::max(-cur.H[7 * i], tiny);
+        if (!chol6(A, cur.g, delta)) {
+          lambda *= 10.0;
+          if (lambda > kLambdaMax) { term = GNDT_NDT_STALLED; break; }
+          continue;
+        }
+        // converged: the (nearly undamped) step to the optimum of the local model is below both
+        // epsilons.  Tested before the pass because there S need not rise any more: candidate sets
+        // change between poses, and on the tails of thin Gaussians the Hessian is indefinite, lambda
+        // grows and steps shrink far from the optimum, so a short damped step says nothing
+        const double dr = std::sqrt(delta[0] * delta[0] + delta[1] * delta[1] + delta[2] * delta[2]);
+        const double dp = std::sqrt(delta[3] * delta[3] + delta[4] * delta[4] + delta[5] * delta[5]);
+        if (lambda < 1.0 && dr < teps && dp < reps) { term = GNDT_NDT_CONVERGED; break; }
+        // candidate: T' = (E, c + rho - E c) o T, E = Exp(phi)
+        double E[9], Tn[16];
+        so3_exp(delta + 3, E);
+        memcpy(Tn, T, sizeof(Tn));
+        for (int i = 0; i < 3; ++i) {
+          double tt = cur.c[i] + delta[i];
+          for (int j = 0; j < 3; ++j) {
+            Tn[4 * i + j] = E[3 * i] * T[j] + E[3 * i + 1] * T[4 + j] + E[3 * i + 2] * T[8 + j];
+            tt += E[3 * i + j] * (T[4 * j + 3] - cur.c[j]);
+          }
+          Tn[4 * i + 3] = tt;
+        }
+        NdtEval cand;
+        if ((rc = eval(Tn, cand)) != GNDT_OK) return rc;
+        ++iters;
+        if (cand.score > cur.score) {
+          memcpy(T, Tn, sizeof(T));
+          cur = cand;
+          lambda = std::max(lambda / 10.0, kLambdaMin);
+        } else {
+          lambda *= 10.0;
+          if (lambda > kLambdaMax) { term = GNDT_NDT_STALLED; break; }
+        }
+      }
+    }
+    memset(res, 0, sizeof(*res));
+    memcpy(res->pose, T, sizeof(T));
+    memcpy(res->center, cur.c, sizeof(cur.c));
+    res->score = cur.score;
+    memcpy(res->gradient, cur.g, sizeof(cur.g));
+    memcpy(res->hessian, cur.H, sizeof(cur.H));
+    res->n_points = n_points;
+    res->n_matched = cur.n_matched;
+    res->n_pairs = cur.n_pairs;
+    res->iterations = iters;
+    res->termination = term;
     return GNDT_OK;
   };
 
   double T[16];
   memcpy(T, guess, sizeof(T));
-  NdtEval cur;
-  if ((rc = eval(T, cur)) != GNDT_OK) return rc;
-  int term = GNDT_NDT_MAX_ITER;
-  uint32_t iters = 0;
-  if (cur.n_pairs == 0) {
-    term = GNDT_NDT_NO_MATCH;
-    cur.score = 0.0;
-    memset(cur.g, 0, sizeof(cur.g));
-    memset(cur.H, 0, sizeof(cur.H));
-  } else {
-    // Levenberg-Marquardt on -S: (-H + lambda diag(max(-H_ii, tiny))) delta = g
-    constexpr double kLambda0 = 1e-3, kLambdaMin = 1e-12, kLambdaMax = 1e12;
-    double lambda = kLambda0;
-    while (iters < (uint32_t)np->max_iterations) {
-      double hmax = 0.0;
-      for (int i = 0; i < 6; ++i) hmax = std::max(hmax, std::fabs(cur.H[7 * i]));
-      const double tiny = std::max(1e-6 * hmax, 1e-300);
-      double A[36], delta[6];
-      for (int i = 0; i < 36; ++i) A[i] = -cur.H[i];
-      for (int i = 0; i < 6; ++i) A[7 * i] += lambda * std::max(-cur.H[7 * i], tiny);
-      if (!chol6(A, cur.g, delta)) {
-        lambda *= 10.0;
-        if (lambda > kLambdaMax) { term = GNDT_NDT_STALLED; break; }
-        continue;
-      }
-      // converged: the (nearly undamped) step to the optimum of the local model is below both
-      // epsilons.  Tested before the pass because there S need not rise any more: candidate sets
-      // change between poses, and on the tails of thin Gaussians the Hessian is indefinite, lambda
-      // grows and steps shrink far from the optimum, so a short damped step says nothing
-      const double dr = std::sqrt(delta[0] * delta[0] + delta[1] * delta[1] + delta[2] * delta[2]);
-      const double dp = std::sqrt(delta[3] * delta[3] + delta[4] * delta[4] + delta[5] * delta[5]);
-      if (lambda < 1.0 && dr < np->translation_epsilon && dp < np->rotation_epsilon) { term = GNDT_NDT_CONVERGED; break; }
-      // candidate: T' = (E, c + rho - E c) o T, E = Exp(phi)
-      double E[9], Tn[16];
-      so3_exp(delta + 3, E);
-      memcpy(Tn, T, sizeof(Tn));
-      for (int i = 0; i < 3; ++i) {
-        double tt = cur.c[i] + delta[i];
-        for (int j = 0; j < 3; ++j) {
-          Tn[4 * i + j] = E[3 * i] * T[j] + E[3 * i + 1] * T[4 + j] + E[3 * i + 2] * T[8 + j];
-          tt += E[3 * i + j] * (T[4 * j + 3] - cur.c[j]);
-        }
-        Tn[4 * i + 3] = tt;
-      }
-      NdtEval cand;
-      if ((rc = eval(Tn, cand)) != GNDT_OK) return rc;
-      ++iters;
-      if (cand.score > cur.score) {
-        memcpy(T, Tn, sizeof(T));
-        cur = cand;
-        lambda = std::max(lambda / 10.0, kLambdaMin);
-      } else {
-        lambda *= 10.0;
-        if (lambda > kLambdaMax) { term = GNDT_NDT_STALLED; break; }
-      }
-    }
+  for (int i = 0; i < n_levels; ++i) {
+    const gndt_ndt_level &l = levels[i];
+    const gndt_handle::NdtLevel &L = h->ndt_lv[l.factor];
+    gndt_registration r;
+    if ((rc = solve(l.factor, (const NdtVoxel *)L.vox.p, (const gndt_column *)L.cols.p, L.n_cols, l.max_iterations, l.translation_epsilon,
+                    l.rotation_epsilon, T, &r)) != GNDT_OK)
+      return rc;
+    memcpy(T, r.pose, sizeof(T));
+    if (level_out) level_out[i] = r;
   }
-  memset(out, 0, sizeof(*out));
-  memcpy(out->pose, T, sizeof(T));
-  memcpy(out->center, cur.c, sizeof(cur.c));
-  out->score = cur.score;
-  memcpy(out->gradient, cur.g, sizeof(cur.g));
-  memcpy(out->hessian, cur.H, sizeof(cur.H));
-  out->n_points = n_points;
-  out->n_matched = cur.n_matched;
-  out->n_pairs = cur.n_pairs;
-  out->iterations = iters;
-  out->termination = term;
-  return GNDT_OK;
+  return solve(1, (const NdtVoxel *)h->ndt_vox.p, (const gndt_column *)h->columns.p, n_cols, np->max_iterations, np->translation_epsilon,
+               np->rotation_epsilon, T, out);
+}
+
+}  // namespace
+
+int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, const double guess[16],
+                  const gndt_ndt_params *np, gndt_registration *out, void *stream) {
+  return register_levels(h, xyz, n, stride_bytes, mem, guess, np, nullptr, 0, out, nullptr, stream);
+}
+
+void gndt_default_ndt_level(gndt_ndt_level *l, int32_t factor) {
+  if (!l) return;
+  memset(l, 0, sizeof(*l));
+  l->factor = factor;
+  l->max_iterations = 50;
+  l->translation_epsilon = 1e-3;
+  l->rotation_epsilon = 1e-3;
+}
+
+int gndt_register_levels(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, const double guess[16],
+                         const gndt_ndt_params *np, const gndt_ndt_level *levels, int n_levels, gndt_registration *out,
+                         gndt_registration *level_out, void *stream) {
+  if (!h) return GNDT_ERR_INVALID_ARG;
+  if (!levels && n_levels > 0) { h->err = "gndt_register_levels: levels is NULL with n_levels > 0"; return GNDT_ERR_INVALID_ARG; }
+  static const gndt_ndt_level kNone = {};
+  return register_levels(h, xyz, n, stride_bytes, mem, guess, np, levels ? levels : &kNone, n_levels, out, level_out, stream);
 }
 
 }  // extern "C"

@@ -2,6 +2,8 @@
 // resident map and one derivative pass of a scan against them.
 //
 // prepare : one thread per voxel -> {mu, C = Sigma'^-1, usable count, cz}          (once per map)
+// level   : coarse columns (warp per x slab), then coarse voxels (thread per coarse column) of the
+//           level of factor k: Chan merges of the fitted records, C as above    (once per map, k)
 // mean    : binary64 sum of the scan's finite points (the solver's centre)         (once per call)
 // pass    : one thread per point -> score, gradient, Hessian and counts per block (once per pose)
 // finish  : one warp sums the per-block partials in block order -> 32 doubles the host reads
@@ -15,6 +17,7 @@ namespace gndt {
 
 constexpr int kNdtThreads = 128;
 constexpr int kNdtWidth = 32;  // pass: S, g[6], H upper triangle[21], n_points, n_matched, n_pairs, 0
+constexpr int kNdtMaxFactor = 32;  // levels: factors 2..32, so a slab's rows fit the lanes of one warp
 
 struct NdtVoxel {  // 80 B
   double mu[3];
@@ -30,13 +33,51 @@ struct NdtPose {
   float origin[3];
   float grid_len, z_len;
   u32 min_points;
+  int factor;         // level: cell indices are floor-divided by it (1 = the map level)
 };
 
-// Sigma from the published record (so the oracle can rebuild it from gndt_copy_voxels), eigenvalues
-// raised to >= 0.01 lambda_max, C = V diag(1/lambda') V^T.  eig3_sym's eigenvectors come from cross
-// products of rows of (A - lambda I) and lose orthogonality between two close eigenvalues; the basis
-// is therefore rebuilt from the eigenvector of the most isolated eigenvalue, which is accurate, and
-// the subspace orthogonal to it (whose split does not matter when its two eigenvalues are close).
+// floor(c / k) for k >= 1: contiguous index -1 and 0 never share a coarse cell
+__host__ __device__ __forceinline__ int floor_div(int c, int k) { return c >= 0 ? c / k : -((k - 1 - c) / k); }
+
+// C = Sigma'^-1 of a symmetric Sigma (xx xy xz yy yz zz) with its eigenvalues raised to >= 0.01
+// lambda_max; false (c untouched) when lambda_max is not positive and finite.  eig3_sym's
+// eigenvectors come from cross products of rows of (A - lambda I) and lose orthogonality between
+// two close eigenvalues; the basis is therefore rebuilt from the eigenvector of the most isolated
+// eigenvalue, which is accurate, and the subspace orthogonal to it (whose split does not matter
+// when its two eigenvalues are close).  The map level and the coarse levels both use it.
+__device__ __forceinline__ bool ndt_inverse_cov(double s[6], double c[6]) {
+  double w[3], E[3][3];
+  eig3_sym(s, w, E);
+  const double lmax = fmax(fmax(w[0], w[1]), w[2]);
+  if (!(lmax > 0.0 && isfinite(lmax))) return false;
+  // a = eigenvector of the isolated end of the spectrum, b = the other end made orthogonal, m = a x b
+  const int ia = (w[1] - w[0] >= w[2] - w[1]) ? 0 : 2, ib = 2 - ia;
+  double a[3] = {E[0][ia], E[1][ia], E[2][ia]}, b[3] = {E[0][ib], E[1][ib], E[2][ib]};
+  const double an = rsqrt(a[0] * a[0] + a[1] * a[1] + a[2] * a[2]);
+  a[0] *= an; a[1] *= an; a[2] *= an;
+  const double ab = a[0] * b[0] + a[1] * b[1] + a[2] * b[2];
+  b[0] -= ab * a[0]; b[1] -= ab * a[1]; b[2] -= ab * a[2];
+  double bn = b[0] * b[0] + b[1] * b[1] + b[2] * b[2];
+  if (!(bn > 1e-20)) {  // no usable second vector: any unit vector orthogonal to a
+    const int k = (fabs(a[0]) <= fabs(a[1]) && fabs(a[0]) <= fabs(a[2])) ? 0 : (fabs(a[1]) <= fabs(a[2]) ? 1 : 2);
+    double e[3] = {0.0, 0.0, 0.0};
+    e[k] = 1.0;
+    b[0] = e[0] - a[k] * a[0]; b[1] = e[1] - a[k] * a[1]; b[2] = e[2] - a[k] * a[2];
+    bn = b[0] * b[0] + b[1] * b[1] + b[2] * b[2];
+  }
+  const double bi = rsqrt(bn);
+  b[0] *= bi; b[1] *= bi; b[2] *= bi;
+  const double m[3] = {a[1] * b[2] - a[2] * b[1], a[2] * b[0] - a[0] * b[2], a[0] * b[1] - a[1] * b[0]};
+  const double floor_l = 0.01 * lmax;
+  const double la = 1.0 / fmax(w[ia], floor_l), lb = 1.0 / fmax(w[ib], floor_l), lm = 1.0 / fmax(w[1], floor_l);
+  const int ii[6] = {0, 0, 0, 1, 1, 2}, jj[6] = {0, 1, 2, 1, 2, 2};
+#pragma unroll
+  for (int k = 0; k < 6; ++k)
+    c[k] = a[ii[k]] * a[jj[k]] * la + b[ii[k]] * b[jj[k]] * lb + m[ii[k]] * m[jj[k]] * lm;
+  return true;
+}
+
+// Sigma from the published record (so the oracle can rebuild it from gndt_copy_voxels).
 __global__ void __launch_bounds__(256) ndt_prepare_kernel(const Ctl *ctl, const gndt_voxel *table, NdtVoxel *out, int normalize_cov) {
   const u32 V = ctl->n_voxels;
   for (u32 v = blockIdx.x * blockDim.x + threadIdx.x; v < V; v += gridDim.x * blockDim.x) {
@@ -49,34 +90,7 @@ __global__ void __launch_bounds__(256) ndt_prepare_kernel(const Ctl *ctl, const 
 #pragma unroll
       for (int k = 0; k < 6; ++k)
         s[k] = normalize_cov ? __ddiv_rn(__dmul_rn((double)r.scatter[k], n), nm1) : __ddiv_rn((double)r.scatter[k], nm1);
-      double w[3], E[3][3];
-      eig3_sym(s, w, E);
-      const double lmax = fmax(fmax(w[0], w[1]), w[2]);
-      if (lmax > 0.0 && isfinite(lmax)) {
-        // a = eigenvector of the isolated end of the spectrum, b = the other end made orthogonal, m = a x b
-        const int ia = (w[1] - w[0] >= w[2] - w[1]) ? 0 : 2, ib = 2 - ia;
-        double a[3] = {E[0][ia], E[1][ia], E[2][ia]}, b[3] = {E[0][ib], E[1][ib], E[2][ib]};
-        const double an = rsqrt(a[0] * a[0] + a[1] * a[1] + a[2] * a[2]);
-        a[0] *= an; a[1] *= an; a[2] *= an;
-        const double ab = a[0] * b[0] + a[1] * b[1] + a[2] * b[2];
-        b[0] -= ab * a[0]; b[1] -= ab * a[1]; b[2] -= ab * a[2];
-        double bn = b[0] * b[0] + b[1] * b[1] + b[2] * b[2];
-        if (!(bn > 1e-20)) {  // no usable second vector: any unit vector orthogonal to a
-          const int k = (fabs(a[0]) <= fabs(a[1]) && fabs(a[0]) <= fabs(a[2])) ? 0 : (fabs(a[1]) <= fabs(a[2]) ? 1 : 2);
-          double e[3] = {0.0, 0.0, 0.0};
-          e[k] = 1.0;
-          b[0] = e[0] - a[k] * a[0]; b[1] = e[1] - a[k] * a[1]; b[2] = e[2] - a[k] * a[2];
-          bn = b[0] * b[0] + b[1] * b[1] + b[2] * b[2];
-        }
-        const double bi = rsqrt(bn);
-        b[0] *= bi; b[1] *= bi; b[2] *= bi;
-        const double m[3] = {a[1] * b[2] - a[2] * b[1], a[2] * b[0] - a[0] * b[2], a[0] * b[1] - a[1] * b[0]};
-        const double floor_l = 0.01 * lmax;
-        const double la = 1.0 / fmax(w[ia], floor_l), lb = 1.0 / fmax(w[ib], floor_l), lm = 1.0 / fmax(w[1], floor_l);
-        const int ii[6] = {0, 0, 0, 1, 1, 2}, jj[6] = {0, 1, 2, 1, 2, 2};
-#pragma unroll
-        for (int k = 0; k < 6; ++k)
-          o.c[k] = a[ii[k]] * a[jj[k]] * la + b[ii[k]] * b[jj[k]] * lb + m[ii[k]] * m[jj[k]] * lm;
+      if (ndt_inverse_cov(s, o.c)) {
         o.mu[0] = (double)r.mean[0]; o.mu[1] = (double)r.mean[1]; o.mu[2] = (double)r.mean[2];
         o.count = r.count;
       }
@@ -193,7 +207,7 @@ __device__ __forceinline__ void ndt_column(const gndt_column &col, int cz, const
   }
 }
 
-// One derivative pass: every finite point at pose P against the 5 candidate columns.
+// One derivative pass: every finite point at pose P against the 5 candidate columns of its level.
 __global__ void __launch_bounds__(kNdtThreads) ndt_pass_kernel(const float *in, size_t stride_f, size_t n, const NdtVoxel *vox,
                                                                const gndt_column *cols, u32 n_cols, NdtPose P, double *partial) {
   NdtAcc A;
@@ -214,6 +228,7 @@ __global__ void __launch_bounds__(kNdtThreads) ndt_pass_kernel(const float *in, 
     if (!point_indices<false>(__double2float_rn(x[0]), __double2float_rn(x[1]), __double2float_rn(x[2]), P.origin, P.grid_len, P.z_len,
                               0.f, 0.f, cx, cy, cz))
       continue;
+    if (P.factor > 1) { cx = floor_div(cx, P.factor); cy = floor_div(cy, P.factor); cz = floor_div(cz, P.factor); }
     const double y[3] = {x[0] - P.c[0], x[1] - P.c[1], x[2] - P.c[2]};
     const u32 before = A.pairs;
     // table order: row cx - 1, then (cx, cy - 1 .. cy + 1), then row cx + 1
@@ -235,6 +250,127 @@ __global__ void __launch_bounds__(kNdtThreads) ndt_pass_kernel(const float *in, 
   for (int k = 0; k < 28; ++k) v[k] = A.s[k];
   v[28] = (double)n_points; v[29] = (double)n_matched; v[30] = (double)A.pairs; v[31] = 0.0;
   block_partials<kNdtWidth>(v, partial);
+}
+
+// ---- levels: the Gaussians of cells of k x k x k map cells --------------------------------
+// Coarse column tables are gndt_column records whose sx, sy, voxel_begin and voxel_count the pass
+// reads; slope_begin / slope_count hold the range of their map columns in `members` instead.
+
+// Level columns, one warp per x slab [kX, kX + k) of the map (X = X0 + warp), lane r < k on map row
+// kX + r.  The slab and its rows are ranges of the (cx, cy)-sorted column table; each row is a sorted
+// run of cy, so the warp emits its coarse columns in Y order by taking the smallest head Y of the
+// rows at a time.  Count pass (EMIT = false): slab_count[warp].  Emit pass: the coarse column at
+// slab_begin[warp] + j and its map columns, row by row, at the slab's own range of `members`.
+template <bool EMIT>
+__global__ void __launch_bounds__(256) ndt_level_columns_kernel(const gndt_column *cols, u32 n_cols, int k, int X0, u32 n_slabs,
+                                                                u32 *slab_count, const u32 *slab_begin, gndt_column *ccols,
+                                                                u32 *members) {
+  const u32 warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (warp >= n_slabs) return;  // whole warps: blockDim is a multiple of 32
+  const int x0 = (X0 + (int)warp) * k;
+  const u32 lo = column_lower_bound(cols, 0, n_cols, x0, INT_MIN), hi = column_lower_bound(cols, lo, n_cols, x0 + k, INT_MIN);
+  u32 r_lo = hi, r_hi = hi;
+  if (lane < k) {
+    r_lo = column_lower_bound(cols, lo, hi, x0 + lane, INT_MIN);
+    r_hi = column_lower_bound(cols, r_lo, hi, x0 + lane + 1, INT_MIN);
+  }
+  u32 out = EMIT ? slab_begin[warp] : 0u, mpos = lo;
+  for (;;) {
+    const int y = r_lo < r_hi ? floor_div(contiguous_index(cols[r_lo].sy), k) : INT_MAX;
+    const int Y = __reduce_min_sync(0xffffffffu, y);
+    if (Y == INT_MAX) break;
+    const u32 e = y == Y ? column_lower_bound(cols, r_lo, r_hi, x0 + lane, (Y + 1) * k) : r_lo;
+    if (EMIT) {
+      const u32 cnt = e - r_lo;
+      u32 inc = cnt;  // inclusive scan over the lanes: rows in order
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const u32 t = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += t;
+      }
+      const u32 total = __shfl_sync(0xffffffffu, inc, 31);
+      for (u32 j = r_lo; j < e; ++j) members[mpos + inc - cnt + (j - r_lo)] = j;
+      if (lane == 0) {
+        gndt_column c = {};
+        c.sx = signed_index(X0 + (int)warp);
+        c.sy = signed_index(Y);
+        c.slope_begin = mpos;
+        c.slope_count = total;
+        ccols[out] = c;
+      }
+      mpos += total;
+    }
+    ++out;
+    r_lo = e;
+  }
+  if (!EMIT && lane == 0) slab_count[warp] = out;
+}
+
+// first voxel of [lo, hi) (one column, sorted by cz) with cz >= z
+__device__ __forceinline__ u32 voxel_lower_bound(const gndt_voxel *table, u32 lo, u32 hi, int z) {
+  while (lo < hi) {
+    const u32 mid = (lo + hi) >> 1;
+    if (contiguous_index(table[mid].sz) < z) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+// Level voxels, one thread per coarse column: its coarse cells bottom to top.  A cell's Gaussian is
+// the binary64 Chan merge of its GNDT_F_FITTED records in ascending table index (map columns in
+// table order, each bottom to top), scatter un-normalised (* n_i when normalize_cov); Sigma =
+// S / (n - 1) and C as at the map level, usable when n >= 3.  Count pass: vcount[c].  Emit pass:
+// the voxels at vbegin[c] and the column's voxel_begin / voxel_count.
+template <bool EMIT>
+__global__ void __launch_bounds__(256) ndt_level_voxels_kernel(const gndt_voxel *table, const gndt_column *cols, const u32 *members,
+                                                               int k, int normalize_cov, gndt_column *ccols, u32 n_ccols,
+                                                               u32 *vcount, const u32 *vbegin, NdtVoxel *out) {
+  for (u32 c = blockIdx.x * blockDim.x + threadIdx.x; c < n_ccols; c += gridDim.x * blockDim.x) {
+    const u32 mb = ccols[c].slope_begin, me = mb + ccols[c].slope_count;
+    int Z = INT_MAX;
+    for (u32 m = mb; m < me; ++m) Z = min(Z, floor_div(contiguous_index(table[cols[members[m]].voxel_begin].sz), k));
+    const u32 o0 = EMIT ? vbegin[c] : 0u;
+    u32 nv = 0;
+    while (Z != INT_MAX) {
+      int next = INT_MAX;
+      double n = 0.0, mu[3] = {0.0, 0.0, 0.0}, S[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+      for (u32 m = mb; m < me; ++m) {
+        const gndt_column mc = cols[members[m]];
+        const u32 end = mc.voxel_begin + mc.voxel_count;
+        for (u32 v = voxel_lower_bound(table, mc.voxel_begin, end, Z * k); v < end; ++v) {
+          const gndt_voxel &r = table[v];
+          const int cz = contiguous_index(r.sz);
+          if (cz >= (Z + 1) * k) { next = min(next, floor_div(cz, k)); break; }
+          if (!EMIT || !(r.flags & GNDT_F_FITTED)) continue;
+          const double nb = (double)r.count, nn = n + nb, f = nb / nn, w = n * nb / nn;
+          const double d[3] = {(double)r.mean[0] - mu[0], (double)r.mean[1] - mu[1], (double)r.mean[2] - mu[2]};
+          const int ii[6] = {0, 0, 0, 1, 1, 2}, jj[6] = {0, 1, 2, 1, 2, 2};
+#pragma unroll
+          for (int j = 0; j < 6; ++j) S[j] += (normalize_cov ? (double)r.scatter[j] * nb : (double)r.scatter[j]) + d[ii[j]] * d[jj[j]] * w;
+#pragma unroll
+          for (int i = 0; i < 3; ++i) mu[i] += d[i] * f;
+          n = nn;
+        }
+      }
+      if (EMIT) {
+        NdtVoxel o = {};
+        o.cz = Z;
+        if (n >= 3.0) {
+          double s[6];
+#pragma unroll
+          for (int j = 0; j < 6; ++j) s[j] = S[j] / (n - 1.0);
+          if (ndt_inverse_cov(s, o.c)) {
+            o.mu[0] = mu[0]; o.mu[1] = mu[1]; o.mu[2] = mu[2];
+            o.count = (u32)n;
+          }
+        }
+        out[o0 + nv] = o;
+      }
+      ++nv;
+      Z = next;
+    }
+    if (EMIT) { ccols[c].voxel_begin = o0; ccols[c].voxel_count = nv; } else vcount[c] = nv;
+  }
 }
 
 // one warp: out[k] = sum over blocks, in block order, of partial[b][k]

@@ -498,6 +498,54 @@ int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes
                   const double guess[16], const gndt_ndt_params *np, gndt_registration *out,
                   void *stream);
 
+/*
+ * Coarse-to-fine registration (Magnusson 2009, ch. 6): gndt_register first against coarser
+ * Gaussians merged on the GPU from the resident map, then against the map itself.  The coarse
+ * levels widen the basin of convergence; the map level gives the result its accuracy.
+ *
+ * The level of factor k (2 <= k <= 32) has cells of k x k x k map cells, anchored at the map's
+ * origin.  A map cell with contiguous indices (cx, cy, cz) lies in the coarse cell (floor(cx / k),
+ * floor(cy / k), floor(cz / k)), so contiguous indices -1 and 0 never share one; a scan point lies
+ * in the coarse cell of its map cell (binned as in gndt_register, then the integer division).  The
+ * Gaussian of a coarse cell is the binary64 Chan merge, in ascending voxel-table index, of the
+ * published records (count, mean, scatter) of its GNDT_F_FITTED voxels, each scatter
+ * un-normalised (scatter, or scatter * count when normalize_cov = 1); Sigma = S / (n - 1) with n
+ * the summed count, usable when n >= 3, and the eigenvalue floor and C as at the map level.
+ * Candidates are those of gndt_register on coarse indices (own column and its 4 edge neighbours,
+ * |dZ| <= 1, n >= min_voxel_points, a usable Gaussian); the score constants use
+ * V = (k grid_len)^2 (k z_len) in binary64.
+ *
+ * Contract of gndt_register_levels:
+ *   - Each level runs gndt_register's Levenberg-Marquardt loop with its own lambda (from 1e-3),
+ *     epsilons and iteration cap, from the pose the previous level returned (the guess for the
+ *     first).  A level that ends GNDT_NDT_NO_MATCH returns, and hands on, its input pose.
+ *   - *out is the map level with np's settings: it equals, byte for byte, gndt_register started
+ *     from level_out[n_levels - 1].pose; with n_levels == 0 it is gndt_register.
+ *   - level_out (n_levels records, or NULL) receives each level's result; score, gradient,
+ *     Hessian and counts are those of the level's objective at its pose.
+ *   - Argument checks, the pending update, "nothing of the map changes" (gndt_launch_count
+ *     included) and bitwise repeatability are those of gndt_register.  GNDT_ERR_INVALID_ARG also
+ *     when levels is NULL with n_levels > 0, n_levels is outside [0, GNDT_NDT_MAX_LEVELS], a
+ *     factor is outside [2, 32], the factors do not strictly decrease, a max_iterations is
+ *     negative, or an epsilon is not finite or is negative.
+ *   - A level's tables are built on the device once per map state and factor and kept in the
+ *     handle (at most the map's voxel and column counts each) until the next gndt_build,
+ *     gndt_build_msg, gndt_update or gndt_remove, whatever its verdict; gndt_destroy frees them.
+ */
+#define GNDT_NDT_MAX_LEVELS 8
+typedef struct gndt_ndt_level {
+  int32_t factor;              /* 2..32; levels strictly decreasing, coarsest first               */
+  int32_t max_iterations;      /* as gndt_ndt_params, for this level; default 50                  */
+  double translation_epsilon;  /* convergence test of this level; defaults 1e-3 m ...             */
+  double rotation_epsilon;     /* ... and 1e-3 rad                                                */
+} gndt_ndt_level;
+void gndt_default_ndt_level(gndt_ndt_level *l, int32_t factor);
+
+int gndt_register_levels(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem,
+                         const double guess[16], const gndt_ndt_params *np,
+                         const gndt_ndt_level *levels, int n_levels, gndt_registration *out,
+                         gndt_registration *level_out, void *stream);
+
 /* ---- host-side key helpers (pure C, no device) ------------------------------------- */
 
 /* TwoDmap::transMortonXYZ (include/map2D.h:950-976) for one position: signed non-zero
