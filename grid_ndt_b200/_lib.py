@@ -101,6 +101,8 @@ SYMBOLS = {
     "gndt_default_ndt_level": (None, [C.POINTER(NdtLevel), C.c_int32]),
     "gndt_register_levels": (_i, [_vp, _vp, _sz, _sz, _i, C.POINTER(C.c_double), C.POINTER(NdtParams), C.POINTER(NdtLevel), _i,
                                   C.POINTER(Registration), C.POINTER(Registration), _vp]),
+    "gndt_register_d2d": (_i, [_vp, _vp, _sz, _sz, _i, C.POINTER(C.c_double), C.POINTER(NdtParams), C.POINTER(NdtLevel), _i,
+                               C.POINTER(Registration), C.POINTER(Registration), _vp]),
     "gndt_key_layout": (_i, [_vp, C.POINTER(C.c_int)]),
     "gndt_find_column": (C.c_int64, [_vp, _sz, C.c_int32, C.c_int32]),
     "gndt_find_slope": (C.c_int64, [_vp, _sz, _vp, C.c_int32, C.c_int32, C.c_int32]),

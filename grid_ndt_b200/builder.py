@@ -204,7 +204,7 @@ class TwoDmap:
         self._views.clear()
         return True
 
-    def register(self, scan, guess=None, stream: Optional[int] = None, levels=None, **ndt) -> dict:
+    def register(self, scan, guess=None, stream: Optional[int] = None, levels=None, method: str = "p2d", **ndt) -> dict:
         """NDT registration of a scan against the resident map (gndt_register): the pose
         map <- scan that best fits it, from `guess` (4x4, identity when None).  Keywords set
         gndt_ndt_params fields (outlier_ratio, min_voxel_points, max_iterations,
@@ -214,7 +214,12 @@ class TwoDmap:
         levels: coarse-to-fine registration (gndt_register_levels) when not None: a sequence of
         factors, coarsest first, or of dicts with "factor" and any gndt_ndt_level field
         (max_iterations, translation_epsilon, rotation_epsilon); the other fields keep their
-        defaults.  The result then has "levels": one dict per level, in the same shape."""
+        defaults.  The result then has "levels": one dict per level, in the same shape.
+
+        method: "p2d" registers the scan's points; "d2d" registers the scan's own per-cell Gaussians
+        (gndt_register_d2d, with or without levels), and the result has the same shape."""
+        if method not in ("p2d", "d2d"):
+            raise GndtError(-1, f"unknown registration method {method!r} (p2d or d2d)")
         ptr, n, stride, mem, st, keep = self._marshal(scan)
         if stream is not None:
             st = stream
@@ -224,15 +229,17 @@ class TwoDmap:
         np_ = _abi.default_ndt_params(**ndt)
         out = _abi.Registration()
         Tp = T.ctypes.data_as(C.POINTER(C.c_double))
-        if levels is None:
+        if levels is None and method == "p2d":
             _check(self._h, lib().gndt_register(self._h, ptr, n, stride, mem, Tp, C.byref(np_), C.byref(out), st))
             return out.as_dict()
-        lv = [_abi.default_ndt_level(**l) if isinstance(l, dict) else _abi.default_ndt_level(l) for l in levels]
+        lv = [_abi.default_ndt_level(**l) if isinstance(l, dict) else _abi.default_ndt_level(l) for l in levels or ()]
         arr = (_abi.NdtLevel * max(len(lv), 1))(*lv)
         per = (_abi.Registration * max(len(lv), 1))()
-        _check(self._h, lib().gndt_register_levels(self._h, ptr, n, stride, mem, Tp, C.byref(np_), arr, len(lv), C.byref(out), per, st))
+        fn = lib().gndt_register_d2d if method == "d2d" else lib().gndt_register_levels
+        _check(self._h, fn(self._h, ptr, n, stride, mem, Tp, C.byref(np_), arr, len(lv), C.byref(out), per, st))
         res = out.as_dict()
-        res["levels"] = [per[i].as_dict() for i in range(len(lv))]
+        if levels is not None:
+            res["levels"] = [per[i].as_dict() for i in range(len(lv))]
         return res
 
     @property

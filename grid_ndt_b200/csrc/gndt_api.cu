@@ -111,9 +111,15 @@ struct gndt_handle {
   Buffer ndt_vox, ndt_pts, ndt_part;
   double *ndt_host = nullptr;  // pinned read-back of one pass
   bool ndt_ready = false;      // ndt_vox describes the resident map (cleared by build / update / remove)
-  // coarse levels of gndt_register_levels, by factor: Gaussians, coarse column table, its length
-  struct NdtLevel { Buffer vox, cols; u32 n_cols = 0; } ndt_lv[kNdtMaxFactor + 1];
-  uint64_t ndt_lv_ready = 0;   // bit k: ndt_lv[k] describes the resident map (cleared with ndt_ready)
+  // coarse levels of gndt_register_levels, by factor: Gaussians, coarse column table, their lengths
+  struct NdtLevel { Buffer vox, cov, cols; u32 n_cols = 0, n_vox = 0; } ndt_lv[kNdtMaxFactor + 1];
+  uint64_t ndt_lv_ready = 0;   // bit k: ndt_lv[k].vox describes the resident map (cleared with ndt_ready)
+  // gndt_register_d2d: the same Gaussians with c = Sigma' (map level, and ndt_lv[k].cov beside the C
+  // form; the coarse columns are shared), and the builder of the scan's Gaussians (first D2D call)
+  Buffer ndt_cov;
+  bool ndt_cov_ready = false;
+  uint64_t ndt_lv_cov_ready = 0;
+  gndt_handle *ndt_scan = nullptr;
   Buffer ndt_lv_work;          // scratch of a level build
   // peer-mapped strip exchange (gndt_xchg_*)
   Buffer xbuf;
@@ -604,9 +610,10 @@ int gndt_destroy(gndt_handle *h) {
   if (h->ring) { cudaFreeHost(h->ring); for (int i = 0; i < 4; ++i) if (h->ring_ev[i]) cudaEventDestroy(h->ring_ev[i]); }
   Buffer *bufs[] = {&h->in_stage, &h->buf_a, &h->buf_b, &h->zero, &h->mom, &h->mom_alt, &h->table, &h->slopes,
                     &h->columns, &h->vfirst, &h->slope_col, &h->mom_scan, &h->upd_work, &h->msg_points, &h->small, &h->lookback, &h->f_zero, &h->xbuf, &h->g_work, &h->g_off, &h->g_tgt,
-                    &h->ndt_vox, &h->ndt_pts, &h->ndt_part, &h->ndt_lv_work};
+                    &h->ndt_vox, &h->ndt_pts, &h->ndt_part, &h->ndt_lv_work, &h->ndt_cov};
   for (Buffer *b : bufs) if (b->p) cudaFree(b->p);
-  for (auto &l : h->ndt_lv) { if (l.vox.p) cudaFree(l.vox.p); if (l.cols.p) cudaFree(l.cols.p); }
+  for (auto &l : h->ndt_lv) for (Buffer *b : {&l.vox, &l.cov, &l.cols}) if (b->p) cudaFree(b->p);
+  if (h->ndt_scan) gndt_destroy(h->ndt_scan);
   for (int i = 0; i < EV_COUNT; ++i) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
   delete h;
   return GNDT_OK;
@@ -627,6 +634,8 @@ static int build_device(gndt_handle *h, const float *d_in, size_t n, size_t stri
   const DevParams dp = make_dev(h, h->params, h->cap_voxels);
   h->ndt_ready = false;
   h->ndt_lv_ready = 0;
+  h->ndt_cov_ready = false;
+  h->ndt_lv_cov_ready = 0;
   h->g_valid = false;  // the graph indexes the slope table this build replaces
   GNDT_CUDA(h, cudaEventRecord(h->ev[EV_START], st));
   int rc = front_end(h, st, d_in, n, stride_bytes / 4, start, dp, (VoxMoments *)h->mom.p);
@@ -769,6 +778,8 @@ static int fuse_scan(gndt_handle *h, const void *xyz, size_t n, size_t stride_by
   h->n_changed_valid = false;
   h->ndt_ready = false;  // recomputed by the next gndt_register whatever the verdict
   h->ndt_lv_ready = 0;
+  h->ndt_cov_ready = false;
+  h->ndt_lv_cov_ready = 0;
   h->g_valid = false;    // rebuilt by the next gndt_build_edges whatever the verdict
 
   // capacity: every scan point could open a new voxel
@@ -1749,14 +1760,15 @@ int ndt_check_args(gndt_handle *h, const double *T, const gndt_ndt_params *np) {
 // The tables of the level of factor k (gndt.h, gndt_register_levels), once per map state and factor:
 // coarse columns by slab (count, scan, emit), then coarse voxels by coarse column (count, scan,
 // emit).  Two read-backs: the map's first and last column (the slab range) and the coarse column
-// count.
-int ndt_build_level(gndt_handle *h, int k, cudaStream_t st) {
+// count.  cov: the voxels go to L.cov with c = Sigma' (D2D); the columns are the same either way.
+int ndt_build_level(gndt_handle *h, int k, cudaStream_t st, bool cov) {
   gndt_handle::NdtLevel &L = h->ndt_lv[k];
+  Buffer &vox = cov ? L.cov : L.vox;
   const u32 n_vox = h->host_ctl.n_voxels, n_cols = h->host_ctl.n_columns;
   int rc;
-  if ((rc = ensure(h, L.vox, std::max<size_t>(n_vox, 1) * sizeof(NdtVoxel))) != GNDT_OK) return rc;
+  if ((rc = ensure(h, vox, std::max<size_t>(n_vox, 1) * sizeof(NdtVoxel))) != GNDT_OK) return rc;
   if ((rc = ensure(h, L.cols, std::max<size_t>(n_cols, 1) * sizeof(gndt_column))) != GNDT_OK) return rc;
-  L.n_cols = 0;
+  L.n_cols = L.n_vox = 0;
   if (n_cols) {
     const gndt_column *cols = (const gndt_column *)h->columns.p;
     gndt_column ends[2];
@@ -1796,15 +1808,20 @@ int ndt_build_level(gndt_handle *h, int k, cudaStream_t st) {
            ccols, nc, vcount, (const u32 *)nullptr, (NdtVoxel *)nullptr);
     launch(h, false, exclusive_scan_kernel, grid_for(h, (nc + kScanTile - 1) / kScanTile, 1, 4), 256, 0, st, at<ScanCtl>(w, s2.ctl),
            (const u32 *)vcount, nc, (const u32 *)nullptr, vbegin, at<u64>(w, s2.state), at<GroupState>(w, s2.groups));
-    launch(h, false, ndt_level_voxels_kernel<true>, g_col, 256, 0, st, table, cols, (const u32 *)members, k, h->res_params.normalize_cov,
-           ccols, nc, (u32 *)nullptr, (const u32 *)vbegin, (NdtVoxel *)L.vox.p);
+    if (cov)
+      launch(h, false, ndt_level_voxels_kernel<true, true>, g_col, 256, 0, st, table, cols, (const u32 *)members, k,
+             h->res_params.normalize_cov, ccols, nc, (u32 *)nullptr, (const u32 *)vbegin, (NdtVoxel *)vox.p);
+    else
+      launch(h, false, ndt_level_voxels_kernel<true>, g_col, 256, 0, st, table, cols, (const u32 *)members, k, h->res_params.normalize_cov,
+             ccols, nc, (u32 *)nullptr, (const u32 *)vbegin, (NdtVoxel *)vox.p);
     GNDT_CUDA(h, cudaGetLastError());
     GNDT_CUDA(h, cudaMemcpyAsync(&hs, at<ScanCtl>(w, s2.ctl), sizeof(hs), cudaMemcpyDeviceToHost, st));
     GNDT_CUDA(h, cudaStreamSynchronize(st));
     if (hs.err) { h->err = "level voxel scan watchdog"; return GNDT_ERR_INTERNAL; }
     L.n_cols = nc;
+    L.n_vox = hs.total;
   }
-  h->ndt_lv_ready |= 1ull << k;
+  (cov ? h->ndt_lv_cov_ready : h->ndt_lv_ready) |= 1ull << k;
   return GNDT_OK;
 }
 
@@ -1826,10 +1843,38 @@ int ndt_check_levels(gndt_handle *h, const gndt_ndt_level *levels, int n_levels)
   return GNDT_OK;
 }
 
+// The scan's own Gaussians for gndt_register_d2d, on the builder h->ndt_scan (created here on the first
+// call): a gndt_build of the scan with the resident map's parameters and origin, every point binned,
+// then its Sigma'-form prepare and level tables.  Launches count on the builder, not on h.
+int ndt_scan_gaussians(gndt_handle *h, const float *d_in, size_t n, size_t stride_bytes, const gndt_ndt_level *levels, int n_levels,
+                       cudaStream_t st) {
+  int rc = GNDT_OK;
+  if (!h->ndt_scan && (rc = gndt_create(&h->res_params, h->device, &h->ndt_scan)) != GNDT_OK) {
+    h->err = std::string("gndt_register_d2d: scan build: ") + gndt_last_error(nullptr);
+    return rc;
+  }
+  gndt_handle *s = h->ndt_scan;
+  gndt_params p = h->res_params;
+  p.origin_is_first_point = 0;
+  for (int i = 0; i < 3; ++i) p.origin[i] = h->host_ctl.origin[i];
+  p.tile_lo = p.tile_hi = 0;
+  p.max_voxels = 0;
+  if ((rc = gndt_set_params(s, &p)) == GNDT_OK && (rc = gndt_build(s, d_in, n, stride_bytes, GNDT_MEM_DEVICE, st)) == GNDT_OK &&
+      (rc = sync_counts(s)) == GNDT_OK && (rc = ensure(s, s->ndt_cov, std::max<size_t>(s->host_ctl.n_voxels, 1) * sizeof(NdtVoxel))) == GNDT_OK) {
+    launch(s, false, ndt_prepare_kernel<true>, grid_for(s, s->host_ctl.n_voxels, 256, 8), 256, 0, st, s->ctl, (const gndt_voxel *)s->table.p,
+           (NdtVoxel *)s->ndt_cov.p, p.normalize_cov);
+    for (int i = 0; i < n_levels && rc == GNDT_OK; ++i) rc = ndt_build_level(s, levels[i].factor, st, true);
+  }
+  if (rc != GNDT_OK) h->err = "gndt_register_d2d: scan build: " + s->err;
+  return rc;
+}
+
+// gndt_register / gndt_register_levels (P2D) and gndt_register_d2d: one Levenberg-Marquardt loop per
+// level, the derivative pass differs.
 int register_levels(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, const double guess[16],
                     const gndt_ndt_params *np, const gndt_ndt_level *levels, int n_levels, gndt_registration *out,
-                    gndt_registration *level_out, void *stream) {
-  const char *who = levels ? "gndt_register_levels" : "gndt_register";
+                    gndt_registration *level_out, void *stream, bool d2d) {
+  const char *who = d2d ? "gndt_register_d2d" : levels ? "gndt_register_levels" : "gndt_register";
   if (!h) return GNDT_ERR_INVALID_ARG;
   if (!guess || !np || !out) { h->err = std::string(who) + ": guess, np and out must not be NULL"; return GNDT_ERR_INVALID_ARG; }
   int rc = check_cloud_args(h, xyz, n, stride_bytes, mem, who);
@@ -1843,14 +1888,22 @@ int register_levels(gndt_handle *h, const void *xyz, size_t n, size_t stride_byt
   const gndt_params &rp = h->res_params;
   const u32 n_vox = h->host_ctl.n_voxels, n_cols = h->host_ctl.n_columns;
 
-  // the resident map's Gaussians, once per map state; each level's, once per map state and factor
-  if (!h->ndt_ready) {
-    if ((rc = ensure(h, h->ndt_vox, std::max<size_t>(n_vox, 1) * sizeof(NdtVoxel))) != GNDT_OK) return rc;
-    launch(h, false, ndt_prepare_kernel, grid_for(h, n_vox, 256, 8), 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p,
-           (NdtVoxel *)h->ndt_vox.p, rp.normalize_cov);
+  // the resident map's Gaussians, once per map state and form (C for P2D, Sigma' for D2D); each
+  // level's, once per map state, form and factor
+  Buffer &map_vox = d2d ? h->ndt_cov : h->ndt_vox;
+  if (!(d2d ? h->ndt_cov_ready : h->ndt_ready)) {
+    if ((rc = ensure(h, map_vox, std::max<size_t>(n_vox, 1) * sizeof(NdtVoxel))) != GNDT_OK) return rc;
+    if (d2d)
+      launch(h, false, ndt_prepare_kernel<true>, grid_for(h, n_vox, 256, 8), 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p,
+             (NdtVoxel *)map_vox.p, rp.normalize_cov);
+    else
+      launch(h, false, ndt_prepare_kernel<false>, grid_for(h, n_vox, 256, 8), 256, 0, st, h->ctl, (const gndt_voxel *)h->table.p,
+             (NdtVoxel *)map_vox.p, rp.normalize_cov);
   }
   for (int i = 0; i < n_levels; ++i)
-    if (!(h->ndt_lv_ready >> levels[i].factor & 1) && (rc = ndt_build_level(h, levels[i].factor, st)) != GNDT_OK) return rc;
+    if (!((d2d ? h->ndt_lv_cov_ready : h->ndt_lv_ready) >> levels[i].factor & 1) &&
+        (rc = ndt_build_level(h, levels[i].factor, st, d2d)) != GNDT_OK)
+      return rc;
   const float *d_in;
   if ((rc = upload(h, h->ndt_pts, xyz, n * stride_bytes, mem, st, nullptr, &d_in)) != GNDT_OK) return rc;
   const int blocks = grid_for(h, n, kNdtThreads, 8);
@@ -1865,14 +1918,32 @@ int register_levels(gndt_handle *h, const void *xyz, size_t n, size_t stride_byt
   GNDT_CUDA(h, cudaGetLastError());
   GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_host, dres, 4 * sizeof(double), cudaMemcpyDeviceToHost, st));
   GNDT_CUDA(h, cudaStreamSynchronize(st));
-  h->ndt_ready = true;
+  (d2d ? h->ndt_cov_ready : h->ndt_ready) = true;
   const uint64_t n_points = (uint64_t)h->ndt_host[3];
   const double pbar[3] = {n_points ? h->ndt_host[0] / (double)n_points : 0.0, n_points ? h->ndt_host[1] / (double)n_points : 0.0,
                           n_points ? h->ndt_host[2] / (double)n_points : 0.0};
 
+  if (d2d && (rc = ndt_scan_gaussians(h, d_in, n, stride_bytes, levels, n_levels, st)) != GNDT_OK) return rc;
+
+  // the derivative passes: pass(P) launches one at pose P and returns its number of blocks
+  auto p2d = [=](const NdtVoxel *vox, const gndt_column *cols, u32 nc) {
+    return [=](const NdtPose &P) {
+      launch(h, false, ndt_pass_kernel, blocks, kNdtThreads, 0, st, d_in, stride_f, n, vox, cols, nc, P, part);
+      return blocks;
+    };
+  };
+  auto d2d_pass = [=](const Buffer &svox, u32 n_svox, const NdtVoxel *vox, const gndt_column *cols, u32 nc) {
+    const int b = grid_for(h, n_svox, kNdtThreads, 8);  // n_svox <= n: the partials fit
+    const NdtVoxel *sv = (const NdtVoxel *)svox.p;
+    return [=](const NdtPose &P) {
+      launch(h, false, ndt_d2d_pass_kernel, b, kNdtThreads, 0, st, sv, n_svox, vox, cols, nc, P, part);
+      return b;
+    };
+  };
+
   // Levenberg-Marquardt on one level (factor 1: the map) from T_in -> *res
-  auto solve = [&](int factor, const NdtVoxel *vox, const gndt_column *cols, u32 nc, int max_iterations, double teps, double reps,
-                   const double T_in[16], gndt_registration *res) -> int {
+  auto solve = [&](int factor, const auto &pass, int max_iterations, double teps, double reps, const double T_in[16],
+                   gndt_registration *res) -> int {
     NdtPose P = {};
     {
       const double p_o = np->outlier_ratio, kg = (double)factor * (double)rp.grid_len, kz = (double)factor * (double)rp.z_len;
@@ -1893,8 +1964,8 @@ int register_levels(gndt_handle *h, const void *xyz, size_t n, size_t stride_byt
         P.t[i] = T[4 * i + 3];
         P.c[i] = T[4 * i] * pbar[0] + T[4 * i + 1] * pbar[1] + T[4 * i + 2] * pbar[2] + T[4 * i + 3];
       }
-      launch(h, false, ndt_pass_kernel, blocks, kNdtThreads, 0, st, d_in, stride_f, n, vox, cols, nc, P, part);
-      launch(h, false, ndt_finish_kernel, 1, 32, 0, st, part, blocks, kNdtWidth, dres);
+      const int nb = pass(P);
+      launch(h, false, ndt_finish_kernel, 1, 32, 0, st, part, nb, kNdtWidth, dres);
       GNDT_CUDA(h, cudaGetLastError());
       GNDT_CUDA(h, cudaMemcpyAsync(h->ndt_host, dres, kNdtWidth * sizeof(double), cudaMemcpyDeviceToHost, st));
       GNDT_CUDA(h, cudaStreamSynchronize(st));
@@ -1976,7 +2047,7 @@ int register_levels(gndt_handle *h, const void *xyz, size_t n, size_t stride_byt
     res->score = cur.score;
     memcpy(res->gradient, cur.g, sizeof(cur.g));
     memcpy(res->hessian, cur.H, sizeof(cur.H));
-    res->n_points = n_points;
+    res->n_points = cur.n_points;  // P2D: the finite points, as counted by the mean; D2D: usable scan Gaussians
     res->n_matched = cur.n_matched;
     res->n_pairs = cur.n_pairs;
     res->iterations = iters;
@@ -1989,22 +2060,31 @@ int register_levels(gndt_handle *h, const void *xyz, size_t n, size_t stride_byt
   for (int i = 0; i < n_levels; ++i) {
     const gndt_ndt_level &l = levels[i];
     const gndt_handle::NdtLevel &L = h->ndt_lv[l.factor];
+    const gndt_column *lc = (const gndt_column *)L.cols.p;
     gndt_registration r;
-    if ((rc = solve(l.factor, (const NdtVoxel *)L.vox.p, (const gndt_column *)L.cols.p, L.n_cols, l.max_iterations, l.translation_epsilon,
-                    l.rotation_epsilon, T, &r)) != GNDT_OK)
-      return rc;
+    if (d2d) {
+      const gndt_handle::NdtLevel &SL = h->ndt_scan->ndt_lv[l.factor];
+      rc = solve(l.factor, d2d_pass(SL.cov, SL.n_vox, (const NdtVoxel *)L.cov.p, lc, L.n_cols), l.max_iterations, l.translation_epsilon,
+                 l.rotation_epsilon, T, &r);
+    } else {
+      rc = solve(l.factor, p2d((const NdtVoxel *)L.vox.p, lc, L.n_cols), l.max_iterations, l.translation_epsilon, l.rotation_epsilon, T, &r);
+    }
+    if (rc != GNDT_OK) return rc;
     memcpy(T, r.pose, sizeof(T));
     if (level_out) level_out[i] = r;
   }
-  return solve(1, (const NdtVoxel *)h->ndt_vox.p, (const gndt_column *)h->columns.p, n_cols, np->max_iterations, np->translation_epsilon,
-               np->rotation_epsilon, T, out);
+  const gndt_column *mc = (const gndt_column *)h->columns.p;
+  if (d2d)
+    return solve(1, d2d_pass(h->ndt_scan->ndt_cov, h->ndt_scan->host_ctl.n_voxels, (const NdtVoxel *)map_vox.p, mc, n_cols),
+                 np->max_iterations, np->translation_epsilon, np->rotation_epsilon, T, out);
+  return solve(1, p2d((const NdtVoxel *)map_vox.p, mc, n_cols), np->max_iterations, np->translation_epsilon, np->rotation_epsilon, T, out);
 }
 
 }  // namespace
 
 int gndt_register(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, const double guess[16],
                   const gndt_ndt_params *np, gndt_registration *out, void *stream) {
-  return register_levels(h, xyz, n, stride_bytes, mem, guess, np, nullptr, 0, out, nullptr, stream);
+  return register_levels(h, xyz, n, stride_bytes, mem, guess, np, nullptr, 0, out, nullptr, stream, false);
 }
 
 void gndt_default_ndt_level(gndt_ndt_level *l, int32_t factor) {
@@ -2022,7 +2102,16 @@ int gndt_register_levels(gndt_handle *h, const void *xyz, size_t n, size_t strid
   if (!h) return GNDT_ERR_INVALID_ARG;
   if (!levels && n_levels > 0) { h->err = "gndt_register_levels: levels is NULL with n_levels > 0"; return GNDT_ERR_INVALID_ARG; }
   static const gndt_ndt_level kNone = {};
-  return register_levels(h, xyz, n, stride_bytes, mem, guess, np, levels ? levels : &kNone, n_levels, out, level_out, stream);
+  return register_levels(h, xyz, n, stride_bytes, mem, guess, np, levels ? levels : &kNone, n_levels, out, level_out, stream, false);
+}
+
+int gndt_register_d2d(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem, const double guess[16],
+                      const gndt_ndt_params *np, const gndt_ndt_level *levels, int n_levels, gndt_registration *out,
+                      gndt_registration *level_out, void *stream) {
+  if (!h) return GNDT_ERR_INVALID_ARG;
+  if (!levels && n_levels > 0) { h->err = "gndt_register_d2d: levels is NULL with n_levels > 0"; return GNDT_ERR_INVALID_ARG; }
+  static const gndt_ndt_level kNone = {};
+  return register_levels(h, xyz, n, stride_bytes, mem, guess, np, levels ? levels : &kNone, n_levels, out, level_out, stream, true);
 }
 
 }  // extern "C"

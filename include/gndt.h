@@ -546,6 +546,52 @@ int gndt_register_levels(gndt_handle *h, const void *xyz, size_t n, size_t strid
                          const gndt_ndt_level *levels, int n_levels, gndt_registration *out,
                          gndt_registration *level_out, void *stream);
 
+/*
+ * Distribution-to-distribution NDT (D2D; Stoyanov, Magnusson, Andreasson & Lilienthal, IJRR 2012):
+ * the scan's own per-cell Gaussians, not its points, registered against the map's Gaussians and
+ * those of its levels.  In this block "level k" is the level of factor k, and the map level is k = 1.
+ *
+ * Scan Gaussians.  The scan is binned in its own frame by a gndt_build with the resident map's
+ * grid_len, z_len, slope_interval, demand, min_points and normalize_cov, origin_is_first_point = 0
+ * and origin = the resident origin (gndt_origin), so every point is binned, no strip filter and
+ * max_voxels = 0.  At the map level a record gives a scan Gaussian when it is GNDT_F_FITTED, has
+ * count >= min_voxel_points and its Sigma (the map's rule: scatter / (n - 1), or scatter n / (n - 1)
+ * with normalize_cov) has a positive, finite lambda_max: mu_i = mean (binary64), Sigma'_i = Sigma
+ * with its eigenvalues raised to >= 0.01 lambda_max (not inverted).  At level k the scan's records
+ * are merged as the map's are (gndt_register_levels: binary64 Chan merge in table index of the
+ * fitted records of each k x k x k cell), usable when n >= 3 and n >= min_voxel_points, floored as
+ * above.
+ *
+ * Map side.  mu_j, the usable and count rules and the candidate cells are gndt_register's (or the
+ * level's); Sigma'_j is the floored covariance whose inverse is P2D's C, from the same eigenbasis.
+ *
+ * Pairs and score.  x'_i = R mu_i + t with gndt_register's operation order and rounding; its cell is
+ * that of x'_i rounded to binary32 (floor-divided by k at a level), and its candidates are
+ * gndt_register's: own column and its 4 edge neighbours, |dcz| <= 1, count >= min_voxel_points, a
+ * usable Gaussian.  Each pair adds -d1 exp(-d2 q / 2) to S, with q = m^T B^-1 m, m = x'_i - mu_j,
+ * B = R Sigma'_i R^T + Sigma'_j and the level's d1, d2; pairs are unweighted.  Gradient and Hessian
+ * are over xi = (rho, phi) with pairs frozen: the increment maps x' to Exp(phi)(x' - c) + c + rho and
+ * R Sigma'_i R^T to Exp(phi) R Sigma'_i R^T Exp(phi)^T; c = R pbar + t with pbar the binary64 mean of
+ * the finite scan points, as in gndt_register.  With Sigma'_i = 0 a pair is gndt_register's pair.
+ *
+ * Counts: n_points = usable scan Gaussians of the level, n_matched = those with at least one pair,
+ * n_pairs = Gaussian pairs.
+ *
+ * Contract of gndt_register_d2d: everything else is gndt_register_levels' contract, unchanged: the
+ * Levenberg-Marquardt loop per level and level_out; *out equals, byte for byte, gndt_register_d2d
+ * with n_levels = 0 started from level_out[n_levels - 1].pose; a level that ends GNDT_NDT_NO_MATCH
+ * (a scan without a usable Gaussian included) returns, and hands on, its input pose; the argument
+ * checks; the pending update; nothing of the map changes (gndt_launch_count included); bitwise
+ * repeatability.  The scan's Gaussians are built on a second builder that the handle creates on its
+ * device at the first call and gndt_destroy frees; its launches are not counted on the handle, and
+ * its errors are reported as "gndt_register_d2d: scan build: ...".  The map's Sigma'-form tables
+ * are cached beside those of gndt_register / gndt_register_levels, and cleared with them.
+ */
+int gndt_register_d2d(gndt_handle *h, const void *xyz, size_t n, size_t stride_bytes, int mem,
+                      const double guess[16], const gndt_ndt_params *np,
+                      const gndt_ndt_level *levels, int n_levels, gndt_registration *out,
+                      gndt_registration *level_out, void *stream);
+
 /* ---- host-side key helpers (pure C, no device) ------------------------------------- */
 
 /* TwoDmap::transMortonXYZ (include/map2D.h:950-976) for one position: signed non-zero

@@ -71,9 +71,9 @@ def invalidate(m, scan):
 
 def pass_only(reps):
     """Device ms per map-level ndt_pass_kernel, single level, 1 M scan, 5 cm guess."""
-    if os.environ.get("GNDT_LIB"):  # another build, which may predate the level entry points
+    if os.environ.get("GNDT_LIB"):  # another build, which may predate the level or D2D entry points
         from grid_ndt_b200 import _lib
-        for s in ("gndt_default_ndt_level", "gndt_register_levels"):
+        for s in ("gndt_default_ndt_level", "gndt_register_levels", "gndt_register_d2d"):
             _lib.SYMBOLS.pop(s, None)
     spec, cloud, m = setup()
     scan, pbar = scan_of(spec, cloud, 1_000_000)
